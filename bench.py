@@ -15,11 +15,23 @@ over the workload's synthetic input.
                       of the index sequence with 1 % substitutions, half random), generated on the device slab
                       by slab; the slabs are split over the ranks by contiguous range (STRONG scaling: the job
                       is fixed), replicated index, no data-path collective.
-The `.lph` index is produced by the reference's own build-p (its only producer; PTHash construction is out of
-scope of the GPU path) as input preparation outside every timed region and cached under bench_cache/.
+The `.lph` index is input preparation outside every timed region: Parts 1-4 of build-p through this library and the
+two PTHash functions from a plain pilot search (oracle/phf.py; c=3.0, alpha=0.94), cached in a per-user directory
+under the system's temporary directory ($TMPDIR/lphash_b200_bench_<uid>), never in the tree.  Its pilots differ from
+those the reference's build-p picks, so the codes are a different (equally valid) minimal perfect hash of the same
+k-mers.
 
-Before anything is timed the codes are checked: config 2 - every one of the 1e8 codes against the unmodified
-reference's (oracle/_ref) plus the permutation property; config 5 - every code of each rank's first slab.
+Before anything is timed the codes are checked: config 2 - the permutation property, and where the reference library
+(oracle/_ref) is built, every one of the 1e8 codes against the reference's answers on the same index; config 5 - every
+code of each rank's first slab against the reference's, where it is built.
+
+--dump-outputs DIR (rank 0) writes what the last timed step returned, as float64 .npy files: the codes at a fixed seeded
+sample of about 2 M positions (low and high 32 bits in codes_lo / codes_hi, exact; the positions in codes_index), the
+code offsets and the status words.  Inputs are a pure function of the arguments, so two builds can be compared file
+by file.
+
+--steps K sets the timed steps of every throughput figure (value, config5_1gpu); the host-buffer legs (e2e) are
+separate, shorter measurements of min(K, 5) passes (config 5: 2, its one-GPU side line: 1).
 
 Printed JSON (one line, rank 0):
   value      whole-job k-mers/s, inputs resident in HBM, CUDA-event time, max over ranks
@@ -39,6 +51,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -48,7 +61,23 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 K, M, BITS = 31, 20, 64
-CACHE = os.path.join(ROOT, "bench_cache")
+INDEX_FORMAT = 1  # part of the cached index's name: bump when oracle/phf.py or the .lph writer changes what it holds
+
+
+def cache_dir() -> str:
+    """This user's directory under the system's temporary directory (the tree may be read-only); a fresh private one
+    when that name is taken by someone else or not writable."""
+    d = os.path.join(tempfile.gettempdir(), f"lphash_b200_bench_{os.getuid()}")
+    try:
+        os.makedirs(d, mode=0o700, exist_ok=True)
+        if os.stat(d).st_uid == os.getuid() and os.access(d, os.W_OK):
+            return d
+    except OSError:
+        pass
+    return tempfile.mkdtemp(prefix="lphash_b200_bench_")
+
+
+CACHE = cache_dir()
 
 
 def log(*a):
@@ -60,23 +89,22 @@ def log(*a):
 # ---------------------------------------------------------------------------------------------
 
 def make_workload(n_kmers: int):
-    """Config-2 unitigs + the reference-built index (cached).  Returns (bases, offsets, lph)."""
+    """Config-2 unitigs + their index (cached).  Returns (bases, offsets, lph)."""
     from lphash_b200 import synth
     os.makedirs(CACHE, exist_ok=True)
-    tag = f"cfg2_n{n_kmers}_k{K}_m{M}_u{BITS}"
-    lph = os.path.join(CACHE, tag + ".lph")
+    lph = index_path(n_kmers)
     t0 = time.time()
     bases, offsets = synth.unitigs(n_kmers, K, M)
     log(f"[bench] synthetic unitigs: {len(offsets) - 1} contigs, {len(bases)} bases ({time.time() - t0:.1f}s)")
     if not os.path.exists(lph):
-        from oracle import ref  # input preparation: the reference's build-p makes the index
-        fa = os.path.join(CACHE, tag + ".fa")
-        synth.write_fasta(fa, bases, offsets)
+        from oracle import phf
         t0 = time.time()
-        csv = ref.build(fa, K, M, lph + ".tmp", bits=BITS, threads=min(host_threads(), 32), tmp_dir=CACHE)
-        os.replace(lph + ".tmp", lph)
-        os.remove(fa)
-        log(f"[bench] reference build-p: {csv} ({time.time() - t0:.1f}s)")
+        image = phf.build_lph(bases, offsets, K, M, kmer_bits=BITS, device=int(os.environ.get("LOCAL_RANK", "0")))
+        tmp = f"{lph}.{os.getpid()}.tmp"
+        with open(tmp, "wb") as out:
+            out.write(image)
+        os.replace(tmp, lph)
+        log(f"[bench] index built: {len(image)} bytes ({time.time() - t0:.1f}s)")
     return bases, offsets, lph
 
 
@@ -113,7 +141,7 @@ def bind_near_gpu(index: int):
 
 
 def index_path(n_kmers: int) -> str:
-    return os.path.join(CACHE, f"cfg2_n{n_kmers}_k{K}_m{M}_u{BITS}.lph")
+    return os.path.join(CACHE, f"cfg2_n{n_kmers}_k{K}_m{M}_u{BITS}_index{INDEX_FORMAT}.lph")
 
 
 def rotate_contigs(bases, offsets, r: int):
@@ -194,6 +222,8 @@ READ_LEN = 150
 SLAB_READS = 1 << 20            # reads per slab: 157,286,400 bases, 125,829,120 k-mers (k = 31)
 CFG5_SLABS = 64                 # 64 slabs = 1.0066e10 bases (BASELINE config 5: >= 10 Gbases)
 CFG5_SEED = 0x5EED0005
+INDEX_NOTE = ("build-p Parts 1-4 through this library, PTHash functions from oracle/phf.py's pilot search "
+              "(c=3.0, alpha=0.94, seeds 42 / 1)")
 
 
 def reads_slab_device(genome_dev, slab: int, dev):
@@ -231,7 +261,7 @@ def cfg5_config(world, slabs_total, n_kmers_total, n_bases_total):
                         f"slabs split over {world} GPU(s) by contiguous range",
             "k": K, "m": M, "kmer_bits": BITS, "slabs": slabs_total, "reads_per_slab": SLAB_READS, "read_len": READ_LEN,
             "cache": "per-launch working set (157 MB bases in + 1.0 GB codes out) >> 126 MB L2; no flush needed",
-            "index": "built by the reference's build-p (c=3.0, seed 42)",
+            "index": INDEX_NOTE,
             "sharding": "replicated index, contiguous slab range per rank, no data-path collective"}
 
 
@@ -302,7 +332,7 @@ def workload_config(n_kmers_requested, n_kmers):
                         f"rank, k={K} m={M}, 64-bit kmer_t, all members, streaming query-p",
             "k": K, "m": M, "kmer_bits": BITS, "kmers_per_rank": int(n_kmers),
             "cache": "per-step working set (bases in + 8 B codes out) ~0.9 GB >> 126 MB L2; no flush needed",
-            "index": "built by the reference's build-p (c=3.0, seed 42)", "sharding": "replicated index, "
+            "index": INDEX_NOTE, "sharding": "replicated index, "
             "same-size contig-rotated shard per rank, no collective"}
 
 
@@ -335,6 +365,35 @@ def roofline(algo_bytes, kern_ms, n_kmers, kernel_name):
             "algorithmic_bytes_per_launch": int(algo_bytes), "kernel_ms": kern_ms,
             "peak_source": "MEASURED_PEAKS.json hbm_gbs (of measured)" if peaks else "fallback 6650 GB/s (of fallback)",
             "input_only_frac": (algo_bytes - 8 * n_kmers) / (kern_ms * 1e-3) / 1e9 / peak}
+
+
+DUMP_SAMPLE = 2 << 20  # positions drawn per output by --dump-outputs (3 float64 arrays of this size: <= 48 MB)
+
+
+def snapshot_outputs(torch, args, codes_list, code_off, status):
+    """What the last timed step returned, taken on the device right after the timed region: the codes of each output
+    buffer at one fixed seeded sample of positions, the code offsets and the status words.  None without
+    --dump-outputs."""
+    if not args.dump_outputs:
+        return None
+    n = codes_list[0].numel()
+    idx = np.unique(np.random.default_rng(0xD0).integers(0, n, size=min(n, DUMP_SAMPLE // len(codes_list))))
+    ti = torch.from_numpy(idx.astype(np.int64)).to(codes_list[0].device)
+    codes = torch.stack([c.index_select(0, ti) for c in codes_list]).cpu().numpy().view(np.uint64)
+    if len(codes_list) == 1:
+        codes = codes[0]
+    # codes of non-member k-mers can use all 64 bits: two exact float64 halves
+    return {"codes_lo": codes & np.uint64(0xFFFFFFFF), "codes_hi": codes >> np.uint64(32), "codes_index": idx,
+            "code_offsets": code_off.cpu().numpy(), "status": status.cpu().numpy()}
+
+
+def write_outputs(path, outputs):
+    if outputs is None:
+        return
+    os.makedirs(path, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a).astype(np.float64))
+    log(f"[bench] outputs of the last timed step written to {path}: {', '.join(sorted(outputs))}")
 
 
 class HostBatch:
@@ -442,10 +501,9 @@ def run_ours(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     workload = args.workload or ("cfg2" if world == 1 else "cfg5")
-    # Input preparation comes before any collective: if the index is not in bench_cache/ yet (build()
-    # in __graft_entry__ prepares it where the reference tree exists), rank 0 builds it with the
-    # reference's build-p while the other ranks wait on the FILE, not inside an NCCL barrier (whose
-    # watchdog would fire during a long build).
+    # Input preparation comes before any collective: if the index is not cached yet, rank 0 builds it
+    # while the other ranks wait on the FILE, not inside an NCCL barrier (whose watchdog would fire
+    # during a long build).
     if rank != 0:
         t_wait = time.time()
         while not os.path.exists(index_path(args.kmers)):
@@ -565,6 +623,7 @@ def bench_cfg2(args, torch, dist, api, L, f, dev, stream, rank, world, bases, of
     sync_all()
     ms_total = ev0.elapsed_time(ev1)
     st_timed = f.stats()
+    outputs = snapshot_outputs(torch, args, [d_codes], d_code_off, d_status) if rank == 0 else None
     if rank == 0:
         # the timed region lasts ~12 ms, a handful of NVML polls: keep the GPU under the identical load
         # (same steps, untimed) until the sampler has seen it for at least 60 ms
@@ -616,6 +675,7 @@ def bench_cfg2(args, torch, dist, api, L, f, dev, stream, rank, world, bases, of
                       "parity": "tools/bench_rows.py scan: all records equal the reference's from_string stream"}
     except Exception as e:  # the headline line stands without it
         build_scan = {"unavailable": str(e)}
+    write_outputs(args.dump_outputs, outputs)
     value = world * n_kmers * args.steps / (ms_total * 1e-3)
     algo_bytes = int(offsets[-1] - offsets[0]) + 8 * n_kmers
     parts = {"codes_kmers": world * e["codes"]["kmers"], "codes_secs": codes_s, "runs_kmers": world * e["runs"]["kmers"],
@@ -676,7 +736,7 @@ def bench_cfg5(args, torch, dist, api, L, f, dev, stream, rank, world, index_bas
             del want
         except (ImportError, OSError, RuntimeError) as e:
             checked = f"reference compare unavailable: {e}"
-    steps = args.steps if not brief else max(3, min(args.steps, 10))
+    steps = args.steps
     if sampler is not None and rank == 0:
         sampler.start()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -689,6 +749,7 @@ def bench_cfg5(args, torch, dist, api, L, f, dev, stream, rank, world, index_bas
     sync_all()
     clocks = sampler.stop() if (sampler is not None and rank == 0) else None
     ms_total = ev0.elapsed_time(ev1)
+    outputs = snapshot_outputs(torch, args, d_codes, d_code_off, d_status) if rank == 0 and not brief else None
     st_timed = f.stats()
     launches_per_step = int(st_timed.kernel_launches) * len(slabs)
     kern_ms_local = float(st_timed.kernel_ms)
@@ -709,6 +770,7 @@ def bench_cfg5(args, torch, dist, api, L, f, dev, stream, rank, world, index_bas
     ms_total, kern_ms, codes_s, runs_s, cc_s, cr_s = (float(x) for x in t.cpu())
     if rank != 0:
         return None
+    write_outputs(args.dump_outputs, outputs)
     total_kmers = S * n_kmers_slab
     value = total_kmers * steps / (ms_total * 1e-3)
     algo_bytes = R * Lr + 8 * n_kmers_slab
@@ -772,7 +834,11 @@ def main():
     ap.add_argument("--slabs", type=int, default=CFG5_SLABS, help="slabs of the config-5 read set (64 = 1.0066e10 bases)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cfg5", action="store_true", help="one GPU: skip the config-5 side measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to DIR/<name>.npy (float64, sampled, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

@@ -23,6 +23,7 @@
 #include <cstring>
 #include <stdexcept>
 #include <string>
+#include <thread>
 #include <vector>
 
 typedef uint64_t u64;
@@ -790,6 +791,90 @@ int orc_phf_positions(const unsigned char* phf, u64 nbytes, const u64* keys, u64
         g_err = e.what();
         return -1;
     }
+}
+// Pilot search of a single_phf over pre-hashed keys, for indexes made without the reference's PTHash (oracle/phf.py).
+// Same bucketer, position function and search order as pthash (buckets by size, largest first; smallest pilot whose
+// positions are all free), so the result is a valid single_phf; it is not bit-identical to pthash's own builder.
+// taken[table_size] comes back with the occupied positions set.  Returns 0, -1 when two keys share a hash, -2 when a
+// bucket holds more than 256 keys.
+int orc_phf_search(const u64* hashes, u64 n, u64 seed, u64 dense, u64 sparse, u64 table_size, u64* pilots,
+                   unsigned char* taken) {
+    orc::SinglePhf f;
+    f.dense = dense;
+    f.sparse = sparse;
+    f.M_dense = ~u128(0) / dense + 1;
+    f.M_sparse = ~u128(0) / sparse + 1;
+    const u128 M = ~u128(0) / table_size + 1;
+    const u64 nb = dense + sparse;
+    std::vector<u64> start(nb + 1, 0), bucket(n);
+    for (u64 i = 0; i < n; ++i) ++start[(bucket[i] = f.bucket(hashes[i])) + 1];
+    for (u64 b = 0; b < nb; ++b) start[b + 1] += start[b];
+    std::vector<u64> keys(n), fill(start.begin(), start.end() - 1);
+    for (u64 i = 0; i < n; ++i) keys[fill[bucket[i]]++] = hashes[i];
+    std::vector<u64> order(nb);
+    for (u64 b = 0; b < nb; ++b) order[b] = b;
+    std::stable_sort(order.begin(), order.end(),
+                     [&](u64 a, u64 b) { return start[a + 1] - start[a] > start[b + 1] - start[b]; });
+    std::vector<u64> used((table_size + 63) / 64, 0);  // a bit per slot: stays in cache where a byte map would not
+    auto is_used = [&](u64 q) { return (used[q >> 6] >> (q & 63)) & 1; };
+    // pilot p fits when every key lands on a free slot and no two keys of the bucket share one
+    auto fits = [&](const u64* k0, u64 s, u64 p) {
+        const u64 hp = orc::murmur64(p, seed);
+        u64 q[256];
+        for (u64 i = 0; i < s; ++i) {
+            q[i] = orc::fastmod_u64(k0[i] ^ hp, M, table_size);
+            if (is_used(q[i])) return false;
+            for (u64 j = 0; j < i; ++j)
+                if (q[j] == q[i]) return false;
+        }
+        return true;
+    };
+    for (u64 b = 0; b < nb; ++b) {
+        u64* k0 = keys.data() + start[b];
+        const u64 s = start[b + 1] - start[b];
+        if (s > 256) return -2;
+        std::sort(k0, k0 + s);
+        for (u64 i = 1; i < s; ++i)
+            if (k0[i] == k0[i - 1]) return -1;
+    }
+    // Buckets are searched a batch at a time on every core against the slots taken before the batch, then committed
+    // in order.  A pilot found that way is the smallest fitting a subset of the slots taken at commit time, so when
+    // it still fits it is the pilot the one-bucket-at-a-time search finds; when it does not, the search goes on
+    // from there.  The result does not depend on the number of threads.
+    const unsigned nt = std::max(1u, std::thread::hardware_concurrency());
+    const u64 batch = 1024 * nt;
+    std::vector<u64> spec(batch);
+    for (u64 b0 = 0; b0 < nb; b0 += batch) {
+        const u64 b1 = std::min(nb, b0 + batch);
+        auto work = [&](unsigned t) {
+            for (u64 i = b0 + t; i < b1; i += nt) {
+                const u64 b = order[i], s = start[b + 1] - start[b];
+                u64 p = 0;
+                while (s && !fits(keys.data() + start[b], s, p)) ++p;
+                spec[i - b0] = p;
+            }
+        };
+        std::vector<std::thread> pool;
+        for (unsigned t = 1; t < nt; ++t) pool.emplace_back(work, t);
+        work(0);
+        for (auto& th : pool) th.join();
+        for (u64 i = b0; i < b1; ++i) {
+            const u64 b = order[i], s = start[b + 1] - start[b];
+            const u64* k0 = keys.data() + start[b];
+            u64 p = spec[i - b0];
+            pilots[b] = 0;
+            if (s == 0) continue;
+            while (!fits(k0, s, p)) ++p;
+            pilots[b] = p;
+            const u64 hp = orc::murmur64(p, seed);
+            for (u64 j = 0; j < s; ++j) {
+                const u64 q = orc::fastmod_u64(k0[j] ^ hp, M, table_size);
+                used[q >> 6] |= u64(1) << (q & 63);
+            }
+        }
+    }
+    for (u64 q = 0; q < table_size; ++q) taken[q] = is_used(q);
+    return 0;
 }
 u64 orc_fallback_order(void* h, u64 lo, u64 hi) {
     return static_cast<orc::Mphf*>(h)->fallback_order((u128(hi) << 64) | lo);

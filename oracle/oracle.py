@@ -53,6 +53,8 @@ def lib() -> C.CDLL:
     L.orc_minimizer_order.argtypes = [p, u64]
     L.orc_phf_positions.restype = C.c_int
     L.orc_phf_positions.argtypes = [p, u64, p, u64, p]
+    L.orc_phf_search.restype = C.c_int
+    L.orc_phf_search.argtypes = [p, u64, u64, u64, u64, u64, p, p]
     L.orc_fallback_order.restype = u64
     L.orc_fallback_order.argtypes = [p, u64, u64]
     L.orc_rank_of.argtypes = [p, u64, C.POINTER(C.c_int), C.POINTER(u64)]

@@ -39,7 +39,8 @@ def lib(bits: int) -> C.CDLL:
         return _libs[bits]
     path = os.path.join(REF_DIR, f"libref{bits}.so")
     if not os.path.exists(path):
-        raise FileNotFoundError(f"{path} missing: run oracle/build_ref.sh where /root/reference exists")
+        raise FileNotFoundError(f"{path} missing: build it with oracle/build_ref.sh (LPHASH_REF_DIR = the reference's "
+                                "source tree)")
     L = C.CDLL(path)
     u64, p = C.c_uint64, C.c_void_p
     L.ref_last_error.restype = C.c_char_p
@@ -162,7 +163,7 @@ class RefMphf:
             raise RuntimeError("reference load failed: " + self.L.ref_last_error().decode())
 
     def close(self):
-        if self.h:
+        if getattr(self, "h", None):  # absent when the library failed to load
             self.L.ref_free(self.h)
             self.h = None
 

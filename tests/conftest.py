@@ -17,7 +17,6 @@ GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
 GOLDEN_NAMES = ["k31_m20_u64", "k31_m16_u128", "k63_m24_u128", "k47_m20_u128", "k15_m7_u64",
                 "k21_m11_u64",
                 "k25_m13_u64", "k40_m17_u128"]  # the last two run on the generic (any k, m) kernels
-REF_DATA = "/root/reference/data"
 
 
 def pytest_configure(config):
