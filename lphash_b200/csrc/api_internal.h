@@ -1,11 +1,12 @@
 // Shared by the translation units behind the C ABI (c_api.cu, build_api.cu): error slot, CUDA error
-// propagation, the exception fence every entry point runs inside, grow-only device buffers.
+// propagation, the exception fence every entry point runs inside, owners of device resources.
 #pragma once
 #include <cuda_runtime.h>
 
 #include <new>
 #include <stdexcept>
 #include <string>
+#include <utility>
 
 #include "../../include/lphash_b200.h"
 #include "lph_image.h"
@@ -29,10 +30,18 @@ struct CudaError {
         if (e__ != cudaSuccess) throw ::lphb::CudaError{e__, #expr}; \
     } while (0)
 
+// The owners below free what they hold when they go out of scope, ignoring errors; the device that owns the
+// resource must be current then.
+
 // grow-only device buffer
 struct DevBuf {
     void* p = nullptr;
     uint64_t cap = 0;
+    DevBuf() = default;
+    DevBuf(DevBuf&& o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, 0)) {}
+    ~DevBuf() {
+        if (p) cudaFree(p);
+    }
     void reserve(uint64_t bytes) {
         if (bytes <= cap) return;
         if (p) CK(cudaFree(p));
@@ -42,13 +51,56 @@ struct DevBuf {
         CK(cudaMalloc(&p, want));
         cap = want;
     }
-    void release() {
-        if (p) cudaFree(p);
+    template <class T>
+    T* as() const { return static_cast<T*>(p); }
+};
+
+// grow-only pinned host buffer
+struct HostBuf {
+    void* p = nullptr;
+    uint64_t cap = 0;
+    HostBuf() = default;
+    HostBuf(HostBuf&& o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, 0)) {}
+    ~HostBuf() {
+        if (p) cudaFreeHost(p);
+    }
+    void reserve(uint64_t bytes) {
+        if (bytes <= cap) return;
+        if (p) CK(cudaFreeHost(p));
         p = nullptr;
         cap = 0;
+        CK(cudaMallocHost(&p, bytes));
+        cap = bytes;
     }
     template <class T>
     T* as() const { return static_cast<T*>(p); }
+};
+
+// non-blocking stream, created on first use
+struct Stream {
+    cudaStream_t s = nullptr;
+    Stream() = default;
+    Stream(Stream&& o) noexcept : s(std::exchange(o.s, nullptr)) {}
+    ~Stream() {
+        if (s) cudaStreamDestroy(s);
+    }
+    void create() {
+        if (!s) CK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+    }
+    operator cudaStream_t() const { return s; }
+};
+
+struct Event {
+    cudaEvent_t e = nullptr;
+    Event() = default;
+    Event(Event&& o) noexcept : e(std::exchange(o.e, nullptr)) {}
+    ~Event() {
+        if (e) cudaEventDestroy(e);
+    }
+    void create(unsigned flags) {
+        if (!e) CK(cudaEventCreateWithFlags(&e, flags));
+    }
+    operator cudaEvent_t() const { return e; }
 };
 
 struct DeviceGuard {
