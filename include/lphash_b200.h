@@ -145,6 +145,27 @@ int lphb_query_stream_device(lphb_mphf* f, const char* d_bases, const uint64_t* 
                              uint64_t codes_capacity, uint64_t* d_code_offsets,
                              uint64_t* d_status, void* stream);
 
+/* ---- lookup of packed k-mers -----------------------------------------------------------------
+ * The code of each of n k-mers the caller already holds as integers (from a counter, an earlier GPU stage,
+ * lphb_colliding_kmers, ...): codes[i] is what the reference's NON-streaming branch
+ * (include/partitioned_mphf.hpp:185-195) returns for the window of k bases that kmers[i] encodes - the
+ * integer k-mer of string_to_integer_no_reverse (include/mphf_utils.hpp:110-116), its leftmost-minimum
+ * m-mer (compute_minimizer_triplet, include/mphf_utils.hpp:118-137) and mphf::query
+ * (src/partitioned_mphf.cpp:292-339; for the unpartitioned handle src/unpartitioned_mphf.cpp:191-206).
+ *   kmers   n k-mers in the handle's kmer_t layout, kmer_bits / 8 little-endian bytes each: 8 for a
+ *           64-bit handle, 16 ({lo, hi}) for a 128-bit one - the layout lphb_colliding_kmers writes.
+ *           The first base sits in the most significant of the 2k used bits, A=0 C=1 G=2 T=3
+ *           (include/partitioned_mphf.hpp:106-108); bits at position 2k and above are ignored.
+ *   codes   n codes in input order: in [0, nkmers) for a member; for any other k-mer the 64-bit value
+ *           mphf::query yields (mod 2^64), as every query entry point gives it.
+ * HOST buffers in and out; n == 0 does nothing.  lphb_mphf_dirty_flags reports 0 contigs afterwards.      */
+int lphb_lookup_kmers(lphb_mphf* f, const void* kmers, uint64_t n, uint64_t* codes);
+
+/* Device-resident variant: d_kmers / d_codes are device pointers on the handle's GPU, d_kmers aligned to
+ * kmer_bits / 8 bytes and d_codes to 8; `stream` is a cudaStream_t (NULL = default stream).  Asynchronous,
+ * and ordered against the handle's other calls as lphb_query_stream_device is.                             */
+int lphb_lookup_kmers_device(lphb_mphf* f, const void* d_kmers, uint64_t n, uint64_t* d_codes, void* stream);
+
 /* Diagnostic: the flat device image behind the handle (layout: lphash_b200/csrc/device_image.h), e.g. to compare
  * the GPU-side decode of a load with the host-side one (LPHB_HOST_DECODE=1).  Read it with lphb_copy_to_host.  */
 int lphb_mphf_device_image(const lphb_mphf* f, const void** d_image, uint64_t* nbytes);
@@ -280,7 +301,7 @@ int lphb_host_alloc(void** ptr, uint64_t nbytes);
 int lphb_copy_to_host(int device, void* dst, const void* d_src, uint64_t nbytes);
 int lphb_host_free(void* ptr);
 
-/* Counters for the last lphb_query_stream* call on the handle (kernel launches, device ms). */
+/* Counters for the last lphb_query_stream* or lphb_lookup_kmers* call on the handle (kernel launches, device ms). */
 typedef struct lphb_stats {
     uint64_t kernel_launches;
     uint64_t h2d_bytes, d2h_bytes;

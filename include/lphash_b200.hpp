@@ -165,6 +165,17 @@ public:
         codes.resize(n);
     }
 
+    // The codes of n packed k-mers (lphb_lookup_kmers): codes[i] is what hf(window, k, false) gives for the
+    // window of k bases kmers[i] encodes (first base in the most significant of its 2k bits, A=0 C=1 G=2 T=3;
+    // partitioned_mphf.hpp:106-108, 185-195).  kmer_t is the width the handle was loaded with.
+    std::vector<uint64_t> lookup(const kmer_t* kmers, std::size_t n) const {
+        if (!h_) throw std::runtime_error("lphash_b200::mphf: no index loaded");
+        std::vector<uint64_t> codes(n);
+        int rc = lphb_lookup_kmers(h_, kmers, n, codes.data());
+        if (rc != LPHB_OK) detail::raise("lphash_b200::mphf::lookup", rc);
+        return codes;
+    }
+
     lphb_mphf* handle() const noexcept { return h_; }
 
 private:

@@ -67,7 +67,7 @@ EXPORTS = ["lphb_last_error", "lphb_version", "lphb_device_count", "lphb_mphf_lo
            "lphb_scan_superkmers_device", "lphb_copy_to_host", "lphb_query_nonstreaming",
            "lphb_mphf_alt_load_file", "lphb_mphf_alt_load_memory", "lphb_inverted_index_bound",
            "lphb_build_inverted_index", "lphb_lph_assemble", "lphb_lph_sections", "lphb_build_inverted_index_alt",
-           "lphb_lph_assemble_alt", "lphb_mphf_device_image"]
+           "lphb_lph_assemble_alt", "lphb_mphf_device_image", "lphb_lookup_kmers", "lphb_lookup_kmers_device"]
 
 _lib = None
 
@@ -95,6 +95,8 @@ def lib() -> C.CDLL:
     L.lphb_query_stream.argtypes = [p, p, p, u64, p, u64, p, C.POINTER(u64)]
     L.lphb_query_nonstreaming.argtypes = [p, p, p, u64, p, u64, p, C.POINTER(u64)]
     L.lphb_query_stream_device.argtypes = [p, p, p, p, u64, p, u64, p, p, p]
+    L.lphb_lookup_kmers.argtypes = [p, p, u64, p]
+    L.lphb_lookup_kmers_device.argtypes = [p, p, u64, p, p]
     L.lphb_query_stream_runs.argtypes = [p, p, p, u64, p, u64, C.POINTER(u64), p, C.POINTER(u64)]
     L.lphb_expand_runs.argtypes = [p, u64, p, u64, C.POINTER(u64), i32]
     L.lphb_mphf_dirty_flags.argtypes = [p, C.POINTER(p), C.POINTER(u64)]
@@ -274,6 +276,27 @@ class Mphf:
         _check(lib().lphb_query_stream_device(self._h, d_bases, d_offsets, h_offsets.ctypes.data,
                                               len(h_offsets) - 1, d_codes, capacity, d_code_offsets,
                                               d_status, stream))
+
+    def lookup(self, kmers, out: np.ndarray | None = None) -> np.ndarray:
+        """lphb_lookup_kmers: the codes of packed k-mers (seqio.pack_kmers), in input order.  kmers is a uint64 array
+        of shape (n,) for a 64-bit handle, (n, 2) = [lo, hi] for a 128-bit one; the first base sits in the most
+        significant of the 2k used bits (A=0 C=1 G=2 T=3), higher bits are ignored.  codes[i] is what the reference's
+        non-streaming branch gives for the window kmers[i] encodes.  Returns a uint64 (n,) array (`out` if given)."""
+        kmers = np.ascontiguousarray(kmers, dtype=np.uint64)
+        shape = "(n,)" if self.kmer_bits == 64 else "(n, 2)"
+        if kmers.ndim != (1 if self.kmer_bits == 64 else 2) or (kmers.ndim == 2 and kmers.shape[1] != 2):
+            raise ValueError(f"a {self.kmer_bits}-bit handle takes k-mers of shape {shape}, got {kmers.shape}")
+        n = kmers.shape[0]
+        codes = np.empty(max(n, 1), dtype=np.uint64) if out is None else out
+        if len(codes) < n or codes.dtype != np.uint64 or not codes.flags.c_contiguous:
+            raise ValueError("out must be a contiguous uint64 array of at least n entries")
+        _check(lib().lphb_lookup_kmers(self._h, kmers.ctypes.data, n, codes.ctypes.data))
+        return codes[:n]
+
+    def lookup_device(self, d_kmers: int, n: int, d_codes: int, stream: int = 0) -> None:
+        """lphb_lookup_kmers_device: asynchronous on `stream`; raw device pointers (ints), e.g. tensor.data_ptr(),
+        d_kmers holding n k-mers of kmer_bits / 8 bytes each."""
+        _check(lib().lphb_lookup_kmers_device(self._h, d_kmers, n, d_codes, stream))
 
 
 RUN_DTYPE = np.dtype([("first", "<u8"), ("n", "<i4")])  # 12 bytes packed: lphb_query_stream_runs records

@@ -251,19 +251,28 @@ void attach_l2_window(lphb_mphf* f, cudaStream_t s) {
     f->l2_streams.push_back(s);
 }
 
-void run_kernels(lphb_mphf* f, DevBatch const& b, cudaStream_t s) {
+// `launch` enqueues the main kernel of a call on s, between the next pair of the handle's events
+template <class Launch>
+void timed_launch(lphb_mphf* f, cudaStream_t s, Launch&& launch) {
     attach_l2_window(f, s);
     const int slot = int(f->ws.ev_next % Workspace::kEvRing);
     CK(cudaEventRecord(f->ws.ev0[slot], s));
-    // A batch of a few tiles would leave one or two warps of the tiled kernel to walk its whole (cold) code alone,
-    // about 40 us whatever the size; below 256 K bases the one-thread-per-k-mer kernel answers sooner (10 us for a
-    // record of 8,000 bases; tools/ubench/call_latency.cpp).  LPHB_GENERIC_BELOW overrides (tests: 0).
-    const char* gb = getenv("LPHB_GENERIC_BELOW");
-    const uint64_t generic_below = gb ? strtoull(gb, nullptr, 10) : (uint64_t(1) << 18);
-    if (b.end_base - b.first_base < generic_below || !launch_query_tiled(f->img, b, s)) launch_query_generic(f->img, b, s);
+    launch();
     CK(cudaEventRecord(f->ws.ev1[slot], s));
     ++f->ws.ev_next;
     ++f->ws.ev_pending;
+}
+
+void run_kernels(lphb_mphf* f, DevBatch const& b, cudaStream_t s) {
+    timed_launch(f, s, [&] {
+        // A batch of a few tiles would leave one or two warps of the tiled kernel to walk its whole (cold) code
+        // alone, about 40 us whatever the size; below 256 K bases the one-thread-per-k-mer kernel answers sooner
+        // (10 us for a record of 8,000 bases; tools/ubench/call_latency.cpp).  LPHB_GENERIC_BELOW overrides (tests: 0).
+        const char* gb = getenv("LPHB_GENERIC_BELOW");
+        const uint64_t generic_below = gb ? strtoull(gb, nullptr, 10) : (uint64_t(1) << 18);
+        if (b.end_base - b.first_base < generic_below || !launch_query_tiled(f->img, b, s))
+            launch_query_generic(f->img, b, s);
+    });
     launch_count_dirty(b.dirty, b.n_contigs, b.status, s);
     f->stats.kernel_launches += 2;
 }
@@ -684,6 +693,77 @@ int query_stream_host(lphb_mphf* f, const char* bases, const uint64_t* offsets, 
         HostQuery q{f, bases, offsets, n_contigs, codes, codes_capacity, code_offsets, n_codes, sink};
         return q.run();
     });
+}
+
+// ---- lookup of packed k-mers ---------------------------------------------------------------------
+
+// the lookup kernel, bracketed by the handle's events like a query's main kernel
+void lookup_launch(lphb_mphf* f, const void* d_kmers, uint64_t n, uint64_t* d_codes, cudaStream_t s) {
+    timed_launch(f, s, [&] { launch_lookup_kmers(f->img, d_kmers, n, d_codes, s); });
+    f->stats.kernel_launches += 1;
+}
+
+// lphb_lookup_kmers, n > 0.  When the k-mers and their codes fit the small block, one copy up, the kernel and one
+// copy down.  Otherwise the k-mers flow in chunks of pipeline_chunk_bases() input bytes through two streams (as in
+// HostQuery::clean_pass), so that the upload of chunk j+1, the kernel of chunk j and the download of chunk j-1
+// overlap; one chunk runs on the handle's stream alone.
+int lookup_host(lphb_mphf* f, const void* kmers, uint64_t n, uint64_t* codes) {
+    Workspace& ws = f->ws;
+    const cudaStream_t s = ws.stream;
+    const uint64_t kb = f->img.kmer_bits / 8, in_b = n * kb, out_b = n * 8;
+    f->stats = lphb_stats{};
+    f->last_dirty_n = 0;
+    f->last_dirty = nullptr;
+    f->stats.h2d_bytes = in_b;
+    f->stats.d2h_bytes = out_b;
+    const uint64_t codes_b = (out_b + 63) & ~uint64_t(63);  // [codes | k-mers]: the k-mers 16-byte aligned
+    if (codes_b + in_b <= Workspace::Small::kBytes && !getenv("LPHB_NO_SMALL_PATH")) {
+        ws.small.d.reserve(Workspace::Small::kBytes);
+        ws.small.h.reserve(Workspace::Small::kBytes);
+        auto* h = ws.small.h.as<unsigned char>();
+        auto* d = ws.small.d.as<unsigned char>();
+        std::memcpy(h + codes_b, kmers, in_b);
+        ws.order_after_previous(s);
+        CK(cudaMemcpyAsync(d + codes_b, h + codes_b, in_b, cudaMemcpyHostToDevice, s));
+        lookup_launch(f, d + codes_b, n, reinterpret_cast<uint64_t*>(d), s);
+        ws.mark_last(s);
+        CK(cudaMemcpyAsync(h, d, out_b, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        CK(cudaGetLastError());
+        std::memcpy(codes, h, out_b);
+        return LPHB_OK;
+    }
+    const uint64_t per = std::max<uint64_t>(1, pipeline_chunk_bases() / kb);  // k-mers per chunk
+    const uint64_t n_chunks = n / per + (n % per != 0);
+    ws.bases.reserve(in_b + 64);
+    ws.codes.reserve(out_b + 64);
+    ws.order_after_previous(s);
+    const bool piped = n_chunks > 1;
+    if (piped) {
+        ws.ensure_pipeline();
+        CK(cudaEventRecord(ws.ev_ready, s));
+    }
+    const auto* src = static_cast<const unsigned char*>(kmers);
+    for (uint64_t j = 0; j < n_chunks; ++j) {
+        const cudaStream_t st = piped ? cudaStream_t(ws.cs[j & 1]) : s;
+        if (piped && j < 2) CK(cudaStreamWaitEvent(st, ws.ev_ready, 0));
+        const uint64_t i0 = j * per, c = std::min(per, n - i0);
+        unsigned char* d_in = ws.bases.as<unsigned char>() + i0 * kb;
+        uint64_t* d_out = ws.codes.as<uint64_t>() + i0;
+        CK(cudaMemcpyAsync(d_in, src + i0 * kb, c * kb, cudaMemcpyHostToDevice, st));
+        lookup_launch(f, d_in, c, d_out, st);
+        CK(cudaMemcpyAsync(codes + i0, d_out, c * 8, cudaMemcpyDeviceToHost, st));
+    }
+    if (piped) {
+        for (int i = 0; i < 2; ++i) {
+            CK(cudaEventRecord(ws.ev_done[i], ws.cs[i]));
+            CK(cudaStreamWaitEvent(s, ws.ev_done[i], 0));
+        }
+    }
+    ws.mark_last(s);
+    CK(cudaStreamSynchronize(s));
+    CK(cudaGetLastError());
+    return LPHB_OK;
 }
 
 // ---- build-side scan ---------------------------------------------------------------------------
@@ -1166,6 +1246,36 @@ int lphb_query_stream_runs(lphb_mphf* f, const char* bases, const uint64_t* offs
     sink.capacity = runs ? runs_capacity : 0;
     sink.n_runs = n_runs;
     return query_stream_host(f, bases, offsets, n_contigs, nullptr, 0, code_offsets, n_codes, sink);
+}
+
+int lphb_lookup_kmers(lphb_mphf* f, const void* kmers, uint64_t n, uint64_t* codes) {
+    if (!f) return fail(LPHB_E_ARG, "null handle");
+    if (n == 0) return LPHB_OK;
+    if (!kmers || !codes) return fail(LPHB_E_ARG, "null argument");
+    return guarded([&]() -> int {
+        DeviceGuard g(f->device);
+        return lookup_host(f, kmers, n, codes);
+    });
+}
+
+int lphb_lookup_kmers_device(lphb_mphf* f, const void* d_kmers, uint64_t n, uint64_t* d_codes, void* stream) {
+    if (!f) return fail(LPHB_E_ARG, "null handle");
+    if (n == 0) return LPHB_OK;
+    if (!d_kmers || !d_codes) return fail(LPHB_E_ARG, "null argument");
+    if (reinterpret_cast<uintptr_t>(d_kmers) % (f->img.kmer_bits / 8) || reinterpret_cast<uintptr_t>(d_codes) % 8)
+        return fail(LPHB_E_ARG, "d_kmers must be aligned to kmer_bits / 8 bytes, d_codes to 8");
+    return guarded([&]() -> int {
+        DeviceGuard g(f->device);
+        cudaStream_t s = static_cast<cudaStream_t>(stream);
+        f->stats = lphb_stats{};
+        f->last_dirty_n = 0;
+        f->last_dirty = nullptr;
+        f->ws.order_after_previous(s);
+        lookup_launch(f, d_kmers, n, d_codes, s);
+        f->ws.mark_last(s);
+        CK(cudaGetLastError());
+        return LPHB_OK;
+    });
 }
 
 // Host side of the run-length form: the uint64_t vector the reference returns, bit for bit.  Pure

@@ -117,21 +117,25 @@ struct Probe {
     int32_t slope;  // +1, -1, or 0 for a colliding minimizer
 };
 
-LPHB_DEV Probe probe_bucket(DevImage const& f, uint64_t bucket) {
+// one bucket word as loaded (a uint32_t entry zero-extended when the table is narrow)
+LPHB_DEV Probe probe_decode(DevImage const& f, uint64_t e) {
     Probe out;
     uint32_t flags;
     if (f.buckets.wide) {
-        const uint64_t e = __ldg(reinterpret_cast<const uint64_t*>(f.buckets.entries) + bucket);
         flags = uint32_t(e >> 62);
         out.base = e & 0x3FFFFFFFFFFFFFFFull;
     } else {
-        const uint32_t e = __ldg(reinterpret_cast<const uint32_t*>(f.buckets.entries) + bucket);
-        flags = e >> 30;
+        flags = uint32_t(e) >> 30;
         out.base = e & 0x3FFFFFFFu;
     }
     out.slope = (flags & 1u) ? 0 : ((flags & 2u) ? 1 : -1);
     if (flags & 1u) out.base = f.collision_base;
     return out;
+}
+
+LPHB_DEV Probe probe_bucket(DevImage const& f, uint64_t bucket) {
+    if (f.buckets.wide) return probe_decode(f, __ldg(reinterpret_cast<const uint64_t*>(f.buckets.entries) + bucket));
+    return probe_decode(f, __ldg(reinterpret_cast<const uint32_t*>(f.buckets.entries) + bucket));
 }
 
 LPHB_DEV Probe probe_minimizer(DevImage const& f, uint64_t minimizer) {
@@ -140,6 +144,28 @@ LPHB_DEV Probe probe_minimizer(DevImage const& f, uint64_t minimizer) {
 
 LPHB_DEV uint64_t probe_hval(Probe const& pr, uint32_t p) {
     return pr.slope > 0 ? pr.base + p : pr.base - p;
+}
+
+// Leftmost-minimum m-mer of the k-mer {lo, hi} (first base in the most significant of its 2k bits) and its offset
+// p in [0, k - m]: the strict '<' keeps the leftmost on ties.  ref: compute_minimizer_triplet,
+// include/mphf_utils.hpp:118-137.
+struct Minimizer {
+    uint64_t mmer;
+    uint32_t pos;
+};
+LPHB_DEV Minimizer kmer_minimizer(uint32_t k, uint32_t m, uint64_t mm_seed, uint64_t lo, uint64_t hi) {
+    const uint64_t mm_mask = (uint64_t(1) << (2 * m)) - 1;
+    const uint32_t w = k - m + 1;
+    uint64_t best_h = 0;
+    Minimizer out{0, 0};
+    for (uint32_t p = 0; p < w; ++p) {
+        uint32_t sh = 2 * (k - m - p);
+        uint64_t mm = sh == 0 ? lo : (sh < 64 ? ((lo >> sh) | (hi << (64 - sh))) : (hi >> (sh - 64)));
+        mm &= mm_mask;
+        uint64_t h = murmur64(mm, mm_seed);
+        if (p == 0 || h < best_h) { best_h = h; out.mmer = mm; out.pos = p; }
+    }
+    return out;
 }
 
 // ASCII -> 2-bit code, 4 = invalid.  ref: src/constants.cpp:5-13.

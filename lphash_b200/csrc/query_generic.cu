@@ -50,8 +50,7 @@ __device__ __forceinline__ uint64_t find_contig(const uint64_t* offsets, uint64_
 
 __global__ void __launch_bounds__(256) k_query_generic(const __grid_constant__ DevImage f,
                                                        const __grid_constant__ DevBatch b) {
-    const uint32_t k = f.k, m = f.m, w = f.w;
-    const uint64_t mm_mask = (uint64_t(1) << (2 * m)) - 1;
+    const uint32_t k = f.k;
     uint64_t span = b.end_base - b.first_base;
     for (uint64_t t = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; t < span;
          t += uint64_t(gridDim.x) * blockDim.x) {
@@ -72,18 +71,9 @@ __global__ void __launch_bounds__(256) k_query_generic(const __grid_constant__ D
             b.dirty[c] = 1;  // plain store: every writer stores the same value
             continue;
         }
-        // leftmost minimum over the w m-mers (strict '<' keeps the leftmost on ties)
-        uint64_t best_h = 0, best_mm = 0;
-        uint32_t best_p = 0;
-        for (uint32_t p = 0; p < w; ++p) {
-            uint32_t sh = 2 * (k - m - p);
-            uint64_t mm = sh == 0 ? lo : (sh < 64 ? ((lo >> sh) | (hi << (64 - sh))) : (hi >> (sh - 64)));
-            mm &= mm_mask;
-            uint64_t h = murmur64(mm, f.mm_seed);
-            if (p == 0 || h < best_h) { best_h = h; best_mm = mm; best_p = p; }
-        }
-        Probe pr = probe_minimizer(f, best_mm);
-        uint64_t hval = pr.slope == 0 ? pr.base + fallback_order(f, lo, hi) : probe_hval(pr, best_p);
+        const Minimizer mz = kmer_minimizer(k, f.m, f.mm_seed, lo, hi);
+        Probe pr = probe_minimizer(f, mz.mmer);
+        uint64_t hval = pr.slope == 0 ? pr.base + fallback_order(f, lo, hi) : probe_hval(pr, mz.pos);
         b.codes[__ldg(b.code_off + c) + (i - start)] = hval;
     }
 }

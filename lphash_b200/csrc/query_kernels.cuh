@@ -33,6 +33,10 @@ uint64_t code_offsets_tmp_bytes(uint64_t n_contigs);
 // Generic kernel: any (k, m); one thread per k-mer, everything recomputed per k-mer.
 void launch_query_generic(DevImage const& img, DevBatch const& b, cudaStream_t stream);
 
+// Packed k-mers (lookup_kernels.cu): d_codes[i] = code of the k-mer in the low 2k bits of d_kmers[i], which holds
+// img.kmer_bits / 8 little-endian bytes ({lo, hi} for 128 bits, 16-byte aligned then); any (k, m), any n.
+void launch_lookup_kmers(DevImage const& img, const void* d_kmers, uint64_t n, uint64_t* d_codes, cudaStream_t stream);
+
 // Tiled kernel for the (k, m) pairs it is instantiated for; returns false if (k, m) is not one
 // of them (the caller then uses the generic kernel).
 bool launch_query_tiled(DevImage const& img, DevBatch const& b, cudaStream_t stream);
