@@ -134,8 +134,8 @@ int lphb_expand_runs(const void* runs, uint64_t n_runs, uint64_t* codes, uint64_
  * ACGT bases, SURVEY.md S1); d_status[0] = number of codes laid out (sum of max(0, L-k+1)),
  * d_status[1] = number of contigs containing a non-ACGT byte.  For such a contig the code slot of
  * every k-mer window that contains a non-ACGT byte is UNSPECIFIED (the slots of its other k-mers hold
- * their codes); lphb_mphf_dirty_flags names those contigs, and lphb_query_stream applies the
- * reference's exact streaming behaviour to them - this call does not.
+ * their codes); lphb_mphf_dirty_flags names those contigs, and lphb_query_stream and
+ * lphb_query_stream_exact_device apply the reference's exact streaming behaviour to them - this call does not.
  * Ordering: a handle owns one device workspace, so consecutive calls on one handle are ordered on
  * the device (each call makes its stream wait for the previous call's kernels), on whatever
  * streams they are issued; they never overlap each other.  Overlap comes from several handles or
@@ -144,6 +144,31 @@ int lphb_query_stream_device(lphb_mphf* f, const char* d_bases, const uint64_t* 
                              const uint64_t* h_offsets, uint64_t n_contigs, uint64_t* d_codes,
                              uint64_t codes_capacity, uint64_t* d_code_offsets,
                              uint64_t* d_status, void* stream);
+
+/* Exact streaming branch on device buffers (include/partitioned_mphf.hpp:73-184, src/query.cpp:52): d_codes and
+ * d_code_offsets receive what lphb_query_stream gives for the same batch, the reference's spurious codes of contigs
+ * with non-ACGT bytes included (SURVEY.md Q1).  Arguments as in lphb_query_stream_device; n_codes receives the total.
+ * SYNCHRONOUS: returns once d_codes / d_code_offsets hold the result (the layout of a contig with non-ACGT bytes is
+ * known only after its repair).  The work runs on `stream` and is ordered against the handle's other calls as in
+ * lphb_query_stream_device; every copy, the status read-back included, goes on `stream`.  A clean batch costs the
+ * stateless form plus one read-back of its 32-byte status.
+ * Capacity: sum of max(0, L-m+1) over the contigs always suffices.  With less than the result needs, the call
+ * returns LPHB_E_CAPACITY with *n_codes set; it then writes nothing at or past d_codes + codes_capacity, and the
+ * contents of d_codes / d_code_offsets are unspecified.                                                            */
+int lphb_query_stream_exact_device(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets,
+                                   const uint64_t* h_offsets, uint64_t n_contigs, uint64_t* d_codes,
+                                   uint64_t codes_capacity, uint64_t* d_code_offsets,
+                                   uint64_t* n_codes, void* stream);
+
+/* Non-streaming branch on device buffers, hf(seq, len, false) (include/partitioned_mphf.hpp:185-195; a non-ACGT
+ * byte counts as 'A', include/mphf_utils.hpp:108): every window of k bytes has its code, max(0, L-k+1) per contig,
+ * equal to lphb_query_nonstreaming.  Arguments, d_status and ordering as in lphb_query_stream_device (d_status[1]
+ * is 0); asynchronous.  The caller's bases are not modified: the kernels read a sanitized copy in the handle's
+ * workspace.                                                                                                      */
+int lphb_query_nonstreaming_device(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets,
+                                   const uint64_t* h_offsets, uint64_t n_contigs, uint64_t* d_codes,
+                                   uint64_t codes_capacity, uint64_t* d_code_offsets,
+                                   uint64_t* d_status, void* stream);
 
 /* ---- lookup of packed k-mers -----------------------------------------------------------------
  * The code of each of n k-mers the caller already holds as integers (from a counter, an earlier GPU stage,
@@ -301,7 +326,7 @@ int lphb_host_alloc(void** ptr, uint64_t nbytes);
 int lphb_copy_to_host(int device, void* dst, const void* d_src, uint64_t nbytes);
 int lphb_host_free(void* ptr);
 
-/* Counters for the last lphb_query_stream* or lphb_lookup_kmers* call on the handle (kernel launches, device ms). */
+/* Counters for the last lphb_query_* or lphb_lookup_kmers* call on the handle (kernel launches, device ms). */
 typedef struct lphb_stats {
     uint64_t kernel_launches;
     uint64_t h2d_bytes, d2h_bytes;

@@ -176,6 +176,31 @@ public:
         return codes;
     }
 
+    // Batches already in device memory: d_* are device pointers on the handle's GPU, h_offsets the host copy of the
+    // offsets, stream a cudaStream_t (nullptr: the default stream).  query_batch_device is hf(contig, len, true) for
+    // every contig, the non-ACGT quirk included (lphb_query_stream_exact_device): synchronous, it returns the number
+    // of codes; codes_capacity = sum of max(0, L-m+1) always suffices.
+    uint64_t query_batch_device(const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
+                                uint64_t n_contigs, uint64_t* d_codes, uint64_t codes_capacity,
+                                uint64_t* d_code_offsets, void* stream = nullptr) const {
+        if (!h_) throw std::runtime_error("lphash_b200::mphf: no index loaded");
+        uint64_t n = 0;
+        int rc = lphb_query_stream_exact_device(h_, d_bases, d_offsets, h_offsets, n_contigs, d_codes, codes_capacity,
+                                                d_code_offsets, &n, stream);
+        if (rc != LPHB_OK) detail::raise("lphash_b200::mphf::query_batch_device", rc);
+        return n;
+    }
+    // hf(contig, len, false) for every contig (lphb_query_nonstreaming_device): max(0, L-k+1) codes per contig,
+    // asynchronous on `stream`; d_status (4 words) as lphb_query_stream_device fills it.
+    void query_batch_device_nonstreaming(const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
+                                         uint64_t n_contigs, uint64_t* d_codes, uint64_t codes_capacity,
+                                         uint64_t* d_code_offsets, uint64_t* d_status, void* stream = nullptr) const {
+        if (!h_) throw std::runtime_error("lphash_b200::mphf: no index loaded");
+        int rc = lphb_query_nonstreaming_device(h_, d_bases, d_offsets, h_offsets, n_contigs, d_codes, codes_capacity,
+                                                d_code_offsets, d_status, stream);
+        if (rc != LPHB_OK) detail::raise("lphash_b200::mphf::query_batch_device_nonstreaming", rc);
+    }
+
     lphb_mphf* handle() const noexcept { return h_; }
 
 private:

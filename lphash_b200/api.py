@@ -33,6 +33,14 @@ class LphashError(RuntimeError):
         self.code = code
 
 
+class CapacityError(LphashError):
+    """LPHB_E_CAPACITY of a call that reports the size it needed (n_codes)"""
+
+    def __init__(self, code: int, msg: str, n_codes: int):
+        super().__init__(code, msg)
+        self.n_codes = n_codes
+
+
 class Info(C.Structure):
     _fields_ = [("k", C.c_uint32), ("m", C.c_uint32), ("kmer_bits", C.c_uint32), ("device", C.c_int32),
                 ("mm_seed", C.c_uint64), ("nkmers", C.c_uint64), ("distinct_minimizers", C.c_uint64),
@@ -67,7 +75,8 @@ EXPORTS = ["lphb_last_error", "lphb_version", "lphb_device_count", "lphb_mphf_lo
            "lphb_scan_superkmers_device", "lphb_copy_to_host", "lphb_query_nonstreaming",
            "lphb_mphf_alt_load_file", "lphb_mphf_alt_load_memory", "lphb_inverted_index_bound",
            "lphb_build_inverted_index", "lphb_lph_assemble", "lphb_lph_sections", "lphb_build_inverted_index_alt",
-           "lphb_lph_assemble_alt", "lphb_mphf_device_image", "lphb_lookup_kmers", "lphb_lookup_kmers_device"]
+           "lphb_lph_assemble_alt", "lphb_mphf_device_image", "lphb_lookup_kmers", "lphb_lookup_kmers_device",
+           "lphb_query_stream_exact_device", "lphb_query_nonstreaming_device"]
 
 _lib = None
 
@@ -95,6 +104,8 @@ def lib() -> C.CDLL:
     L.lphb_query_stream.argtypes = [p, p, p, u64, p, u64, p, C.POINTER(u64)]
     L.lphb_query_nonstreaming.argtypes = [p, p, p, u64, p, u64, p, C.POINTER(u64)]
     L.lphb_query_stream_device.argtypes = [p, p, p, p, u64, p, u64, p, p, p]
+    L.lphb_query_stream_exact_device.argtypes = [p, p, p, p, u64, p, u64, p, C.POINTER(u64), p]
+    L.lphb_query_nonstreaming_device.argtypes = [p, p, p, p, u64, p, u64, p, p, p]
     L.lphb_lookup_kmers.argtypes = [p, p, u64, p]
     L.lphb_lookup_kmers_device.argtypes = [p, p, u64, p, p]
     L.lphb_query_stream_runs.argtypes = [p, p, p, u64, p, u64, C.POINTER(u64), p, C.POINTER(u64)]
@@ -276,6 +287,30 @@ class Mphf:
         _check(lib().lphb_query_stream_device(self._h, d_bases, d_offsets, h_offsets.ctypes.data,
                                               len(h_offsets) - 1, d_codes, capacity, d_code_offsets,
                                               d_status, stream))
+
+    def query_device_exact(self, d_bases: int, d_offsets: int, h_offsets: np.ndarray, d_codes: int,
+                           capacity: int, d_code_offsets: int, stream: int = 0) -> int:
+        """lphb_query_stream_exact_device: the codes lphb_query_stream gives (non-ACGT quirk included) for a batch in
+        device buffers; raw device pointers (ints) and a cudaStream_t handle as in query_device.  Synchronous: returns
+        the number of codes once d_codes / d_code_offsets hold them.  sum(max(0, L-m+1)) is always enough capacity."""
+        h_offsets = np.ascontiguousarray(h_offsets, dtype=np.uint64)
+        n = C.c_uint64(0)
+        rc = lib().lphb_query_stream_exact_device(self._h, d_bases, d_offsets, h_offsets.ctypes.data,
+                                                  len(h_offsets) - 1, d_codes, capacity, d_code_offsets,
+                                                  C.byref(n), stream)
+        if rc == E_CAPACITY:
+            raise CapacityError(rc, lib().lphb_last_error().decode(), n.value)
+        _check(rc)
+        return n.value
+
+    def query_device_nonstreaming(self, d_bases: int, d_offsets: int, h_offsets: np.ndarray, d_codes: int,
+                                  capacity: int, d_code_offsets: int, d_status: int, stream: int = 0) -> None:
+        """lphb_query_nonstreaming_device: the reference's non-streaming branch (a non-ACGT byte counts as 'A') for a
+        batch in device buffers, asynchronous like query_device; the caller's bases are left as they are."""
+        h_offsets = np.ascontiguousarray(h_offsets, dtype=np.uint64)
+        _check(lib().lphb_query_nonstreaming_device(self._h, d_bases, d_offsets, h_offsets.ctypes.data,
+                                                    len(h_offsets) - 1, d_codes, capacity, d_code_offsets,
+                                                    d_status, stream))
 
     def lookup(self, kmers, out: np.ndarray | None = None) -> np.ndarray:
         """lphb_lookup_kmers: the codes of packed k-mers (seqio.pack_kmers), in input order.  kmers is a uint64 array

@@ -62,6 +62,7 @@ struct Workspace {
         DevBuf spur, spur_count, out_off, out;           // the runs' final codes
         DevBuf out_at, counts;                           // per contig: where its codes are in `out`, how many
         DevBuf src_off, assembled;                       // the batch's codes in their final layout
+        std::vector<uint64_t> h_src_off;                 // src_off as the host computes it
     } repair;
     // chunk pipeline of lphb_query_stream: two extra streams so that the H2D copy of chunk j+1,
     // the kernels of chunk j and the D2H copy of chunk j-1 overlap (PCIe is full duplex)
@@ -297,6 +298,141 @@ ContigCounts contig_layout(const uint64_t* offsets, uint64_t n_contigs, uint32_t
     return n;
 }
 
+// ---- contigs with non-ACGT bytes (SURVEY.md Q1; quirk_kernels.cu) ----------------------------------------------
+// Their valid k-mers are ordinary work: the contigs are gathered into a compact batch, cut into maximal runs of
+// valid / invalid bytes, and the runs go through the same query kernel as contigs of their own.  Only the
+// reference's spurious codes (pushed while a run is shorter than k) need the sequential state machine, one thread
+// per episode of a few dozen bases.  Two stages: repair_layout (the dirty contigs' codes and the final layout),
+// then, once the caller has checked its capacity, repair_assemble (the batch's codes in that layout).
+
+// A batch after its clean pass, as the repair reads it.  Device pointers, but h_offsets.
+struct DirtyBatch {
+    const char* bases;            // indexed by the offsets
+    const uint64_t* offsets;      // n_contigs + 1
+    const uint64_t* h_offsets;    // the same offsets on the host
+    uint64_t n_contigs;
+    const uint8_t* dirty;         // per contig: holds a non-ACGT byte
+    const uint64_t* clean_codes;  // the clean pass's codes, clean layout (L-k+1 per contig)
+};
+
+// Leaves the dirty contigs' final codes in the handle's repair scratch and where each contig's codes come from in
+// ws.repair.h_src_off; writes the final layout to code_offsets (host, n_contigs + 1) and returns its total.
+// *d2h_bytes = what it copied to the host.  Every copy runs on s.
+uint64_t repair_layout(lphb_mphf* f, DirtyBatch const& b, uint64_t* code_offsets, cudaStream_t s, uint64_t* d2h_bytes) {
+    Workspace::Repair& R = f->ws.repair;
+    const uint32_t k = f->img.k, w_cap = f->img.w;
+    const uint64_t n_contigs = b.n_contigs;
+    const uint64_t* offsets = b.h_offsets;
+    std::vector<uint8_t> dirty(n_contigs);
+    CK(cudaMemcpyAsync(dirty.data(), b.dirty, n_contigs, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    std::vector<uint64_t> list, starts;
+    uint64_t q_bytes = 0;
+    for (uint64_t c = 0; c < n_contigs; ++c)
+        if (dirty[c]) {
+            list.push_back(c);
+            starts.push_back(q_bytes);
+            q_bytes += offsets[c + 1] - offsets[c];
+        }
+    starts.push_back(q_bytes);
+    const uint64_t n_list = list.size();
+    R.contigs.reserve(n_list * 8);
+    R.starts.reserve((n_list + 1) * 8);
+    R.out_at.reserve(n_list * 8);
+    R.counts.reserve(n_list * 8);
+    R.bases.reserve(q_bytes + 64);
+    R.flag.reserve(q_bytes + 8);
+    R.run_off.reserve((q_bytes + 2) * 8);
+    R.run_first.reserve((n_list + 2) * 4);
+    R.status.reserve(64);
+    R.tmp.reserve(std::max<uint64_t>(quirk_tmp_bytes(q_bytes + 1), code_offsets_tmp_bytes(q_bytes + 1)));
+    CK(cudaMemcpyAsync(R.contigs.p, list.data(), n_list * 8, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(R.starts.p, starts.data(), (n_list + 1) * 8, cudaMemcpyHostToDevice, s));
+    CK(cudaMemsetAsync(R.bases.as<char>() + q_bytes, 'A', 64, s));  // read-ahead of the last tile
+    launch_gather_contigs(b.bases, b.offsets, R.contigs.as<uint64_t>(), R.starts.as<uint64_t>(), n_list, q_bytes,
+                          R.bases.as<char>(), s);
+    auto* qst = R.status.as<unsigned long long>();
+    launch_find_runs(R.bases.as<char>(), q_bytes, R.starts.as<uint64_t>(), n_list, R.flag.as<uint8_t>(),
+                     R.run_off.as<uint64_t>(), qst + 4, R.run_first.as<uint32_t>(), R.tmp.p, R.tmp.cap, s);
+    unsigned long long n_v = 0;
+    CK(cudaMemcpyAsync(&n_v, qst + 4, 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    CK(cudaGetLastError());
+    f->stats.kernel_launches += 7;
+    // the runs as a batch of their own: valid k-mers of every run, clean layout per run
+    R.run_code_off.reserve((n_v + 2) * 8);
+    R.run_dirty.reserve(n_v + 8);
+    R.run_codes.reserve(q_bytes * 8 + 64);
+    R.tile.reserve(query_tiled_ws_bytes(q_bytes));
+    CK(cudaMemsetAsync(R.run_dirty.p, 0, n_v + 8, s));
+    launch_code_offsets(R.run_off.as<uint64_t>(), n_v, k, R.run_code_off.as<uint64_t>(), qst, R.tmp.p, R.tmp.cap, s);
+    DevBatch bq{};
+    bq.bases = R.bases.as<char>();
+    bq.offsets = R.run_off.as<uint64_t>();
+    bq.code_off = R.run_code_off.as<uint64_t>();
+    bq.n_contigs = n_v;
+    bq.first_base = 0;
+    bq.end_base = q_bytes;
+    bq.codes = R.run_codes.as<uint64_t>();
+    bq.dirty = R.run_dirty.as<uint8_t>();
+    bq.status = qst;
+    bq.tile_ws = R.tile.p;
+    bq.tile_ws_bytes = R.tile.cap;
+    if (!launch_query_tiled(f->img, bq, s)) launch_query_generic(f->img, bq, s);
+    f->stats.kernel_launches += 3;
+    R.spur.reserve((n_v + 1) * uint64_t(w_cap) * 8);
+    R.spur_count.reserve((n_v + 2) * 4);
+    R.out_off.reserve((n_v + 2) * 8);
+    R.out.reserve((q_bytes + n_v * uint64_t(w_cap)) * 8 + 64);
+    launch_quirk_finish(f->img, R.bases.as<char>(), R.run_off.as<uint64_t>(), n_v, qst + 4, R.run_first.as<uint32_t>(),
+                        n_list, R.run_code_off.as<uint64_t>(), R.run_codes.as<uint64_t>(), R.spur.as<uint64_t>(),
+                        R.spur_count.as<uint32_t>(), w_cap, R.out_off.as<uint64_t>(), R.out.as<uint64_t>(),
+                        R.out_at.as<uint64_t>(), R.counts.as<uint64_t>(), R.tmp.p, R.tmp.cap, s);
+    launch_quirk_emit(R.run_code_off.as<uint64_t>(), R.run_codes.as<uint64_t>(), R.spur.as<uint64_t>(),
+                      R.spur_count.as<uint32_t>(), w_cap, n_v, qst + 4, R.out_off.as<uint64_t>(), q_bytes,
+                      R.out.as<uint64_t>(), s);
+    f->stats.kernel_launches += 6;
+    std::vector<uint64_t> counts(n_list), out_at(n_list);
+    CK(cudaMemcpyAsync(out_at.data(), R.out_at.p, n_list * 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(counts.data(), R.counts.p, n_list * 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    CK(cudaGetLastError());
+    // final layout + where each contig's codes come from (clean layout or the repaired runs)
+    std::vector<uint64_t>& src_off = R.h_src_off;
+    src_off.resize(n_contigs);
+    uint64_t new_total = 0, clean_run = 0;
+    for (uint64_t c = 0, j = 0; c < n_contigs; ++c) {
+        uint64_t len = offsets[c + 1] - offsets[c];
+        uint64_t clean_cnt = len >= k ? len - k + 1 : 0;
+        uint64_t cnt = clean_cnt;
+        if (dirty[c]) {
+            src_off[c] = out_at[j];
+            cnt = counts[j++];
+        } else {
+            src_off[c] = clean_run;
+        }
+        clean_run += clean_cnt;
+        code_offsets[c] = new_total;
+        new_total += cnt;
+    }
+    code_offsets[n_contigs] = new_total;
+    *d2h_bytes = n_contigs + n_list * 8;
+    return new_total;
+}
+
+// The batch's codes in the final layout of repair_layout (code_offsets, total new_total) into dst, which must not be
+// b.clean_codes; d_code_off receives that layout.
+void repair_assemble(lphb_mphf* f, DirtyBatch const& b, const uint64_t* code_offsets, uint64_t new_total,
+                     uint64_t* d_code_off, uint64_t* dst, cudaStream_t s) {
+    Workspace::Repair& R = f->ws.repair;
+    R.src_off.reserve((b.n_contigs + 1) * 8);
+    CK(cudaMemcpyAsync(R.src_off.p, R.h_src_off.data(), b.n_contigs * 8, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(d_code_off, code_offsets, (b.n_contigs + 1) * 8, cudaMemcpyHostToDevice, s));
+    launch_assemble(dst, d_code_off, b.clean_codes, R.out.as<uint64_t>(), R.src_off.as<uint64_t>(), b.dirty, b.n_contigs,
+                    new_total, s);
+    f->stats.kernel_launches += 1;
+}
+
 // What the caller wants back: the codes themselves (8 B per k-mer) or their run-length form (12-byte
 // records, about 2 B per k-mer: runs_kernels.cu).
 struct RunSink {
@@ -310,7 +446,7 @@ struct RunSink {
 
 // One call of lphb_query_stream, lphb_query_nonstreaming or lphb_query_stream_runs with its batch on the host.
 // Stages: the layout (run), then either the small-batch block (small_call) or the clean pass (clean_pass); when
-// a contig holds a non-ACGT byte, the repair of such contigs (repair); the output (output).
+// a contig holds a non-ACGT byte, the repair of such contigs (repair_layout, repair_assemble); the output (output).
 struct HostQuery {
     lphb_mphf* f;
     const char* bases;
@@ -346,9 +482,16 @@ struct HostQuery {
         if (small_call()) return LPHB_OK;
         const uint64_t n_dirty = clean_pass();
         if (n_dirty == 0) return copied_out ? finish(total, n_chunks, 0) : output(ws.codes.as<uint64_t>(), total, 0);
-        uint64_t new_total = 0, d2h_repair = 0;
-        const int rc = repair(&new_total, &d2h_repair);
-        if (rc != LPHB_OK) return rc;
+        const DirtyBatch db{ws.bases.as<char>() - first, ws.offsets.as<uint64_t>(), offsets, n_contigs,
+                            ws.dirty.as<uint8_t>(), ws.codes.as<uint64_t>()};
+        uint64_t d2h_repair = 0;
+        const uint64_t new_total = repair_layout(f, db, code_offsets, s, &d2h_repair);
+        *n_codes = new_total;
+        if (!want_runs && new_total > codes_capacity) return fail(LPHB_E_CAPACITY, "codes buffer too small");
+        if (want_runs && new_total >= (1ull << 31)) return fail(LPHB_E_ARG, "batch holds >= 2^31 codes: split it");
+        ws.repair.assembled.reserve(new_total * 8 + 64);
+        repair_assemble(f, db, code_offsets, new_total, ws.code_off.as<uint64_t>(), ws.repair.assembled.as<uint64_t>(), s);
+        if (want_runs) reserve_runs(new_total + 16, 1, new_total, 1);
         return output(ws.repair.assembled.as<uint64_t>(), new_total, d2h_repair);
     }
 
@@ -492,122 +635,6 @@ struct HostQuery {
         return h_status[1];
     }
 
-    // ---- contigs with non-ACGT bytes (SURVEY.md Q1; quirk_kernels.cu) ----------------------------------------
-    // Their valid k-mers are ordinary work: the contigs are gathered into a compact batch, cut into maximal runs of
-    // valid / invalid bytes, and the runs go through the same query kernel as contigs of their own.  Only the
-    // reference's spurious codes (pushed while a run is shorter than k) need the sequential state machine, one
-    // thread per episode of a few dozen bases.  Leaves the batch's codes in ws.repair.assembled, their layout in
-    // code_offsets and ws.code_off; *d2h_bytes = what it copied to the host.
-    int repair(uint64_t* new_total_out, uint64_t* d2h_bytes) {
-        Workspace::Repair& R = ws.repair;
-        const uint32_t k = f->img.k, w_cap = f->img.w;
-        std::vector<uint8_t> dirty(n_contigs);
-        CK(cudaMemcpy(dirty.data(), ws.dirty.p, n_contigs, cudaMemcpyDeviceToHost));
-        std::vector<uint64_t> list, starts;
-        uint64_t q_bytes = 0;
-        for (uint64_t c = 0; c < n_contigs; ++c)
-            if (dirty[c]) {
-                list.push_back(c);
-                starts.push_back(q_bytes);
-                q_bytes += offsets[c + 1] - offsets[c];
-            }
-        starts.push_back(q_bytes);
-        const uint64_t n_list = list.size();
-        R.contigs.reserve(n_list * 8);
-        R.starts.reserve((n_list + 1) * 8);
-        R.out_at.reserve(n_list * 8);
-        R.counts.reserve(n_list * 8);
-        R.bases.reserve(q_bytes + 64);
-        R.flag.reserve(q_bytes + 8);
-        R.run_off.reserve((q_bytes + 2) * 8);
-        R.run_first.reserve((n_list + 2) * 4);
-        R.status.reserve(64);
-        R.tmp.reserve(std::max<uint64_t>(quirk_tmp_bytes(q_bytes + 1), code_offsets_tmp_bytes(q_bytes + 1)));
-        CK(cudaMemcpyAsync(R.contigs.p, list.data(), n_list * 8, cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(R.starts.p, starts.data(), (n_list + 1) * 8, cudaMemcpyHostToDevice, s));
-        CK(cudaMemsetAsync(R.bases.as<char>() + q_bytes, 'A', 64, s));  // read-ahead of the last tile
-        launch_gather_contigs(ws.bases.as<char>() - first, ws.offsets.as<uint64_t>(), R.contigs.as<uint64_t>(),
-                              R.starts.as<uint64_t>(), n_list, q_bytes, R.bases.as<char>(), s);
-        auto* qst = R.status.as<unsigned long long>();
-        launch_find_runs(R.bases.as<char>(), q_bytes, R.starts.as<uint64_t>(), n_list, R.flag.as<uint8_t>(),
-                         R.run_off.as<uint64_t>(), qst + 4, R.run_first.as<uint32_t>(), R.tmp.p, R.tmp.cap, s);
-        unsigned long long n_v = 0;
-        CK(cudaMemcpyAsync(&n_v, qst + 4, 8, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        CK(cudaGetLastError());
-        f->stats.kernel_launches += 7;
-        // the runs as a batch of their own: valid k-mers of every run, clean layout per run
-        R.run_code_off.reserve((n_v + 2) * 8);
-        R.run_dirty.reserve(n_v + 8);
-        R.run_codes.reserve(q_bytes * 8 + 64);
-        R.tile.reserve(query_tiled_ws_bytes(q_bytes));
-        CK(cudaMemsetAsync(R.run_dirty.p, 0, n_v + 8, s));
-        launch_code_offsets(R.run_off.as<uint64_t>(), n_v, k, R.run_code_off.as<uint64_t>(), qst, R.tmp.p, R.tmp.cap, s);
-        DevBatch bq{};
-        bq.bases = R.bases.as<char>();
-        bq.offsets = R.run_off.as<uint64_t>();
-        bq.code_off = R.run_code_off.as<uint64_t>();
-        bq.n_contigs = n_v;
-        bq.first_base = 0;
-        bq.end_base = q_bytes;
-        bq.codes = R.run_codes.as<uint64_t>();
-        bq.dirty = R.run_dirty.as<uint8_t>();
-        bq.status = qst;
-        bq.tile_ws = R.tile.p;
-        bq.tile_ws_bytes = R.tile.cap;
-        if (!launch_query_tiled(f->img, bq, s)) launch_query_generic(f->img, bq, s);
-        f->stats.kernel_launches += 3;
-        R.spur.reserve((n_v + 1) * uint64_t(w_cap) * 8);
-        R.spur_count.reserve((n_v + 2) * 4);
-        R.out_off.reserve((n_v + 2) * 8);
-        R.out.reserve((q_bytes + n_v * uint64_t(w_cap)) * 8 + 64);
-        launch_quirk_finish(f->img, R.bases.as<char>(), R.run_off.as<uint64_t>(), n_v, qst + 4, R.run_first.as<uint32_t>(),
-                            n_list, R.run_code_off.as<uint64_t>(), R.run_codes.as<uint64_t>(), R.spur.as<uint64_t>(),
-                            R.spur_count.as<uint32_t>(), w_cap, R.out_off.as<uint64_t>(), R.out.as<uint64_t>(),
-                            R.out_at.as<uint64_t>(), R.counts.as<uint64_t>(), R.tmp.p, R.tmp.cap, s);
-        launch_quirk_emit(R.run_code_off.as<uint64_t>(), R.run_codes.as<uint64_t>(), R.spur.as<uint64_t>(),
-                          R.spur_count.as<uint32_t>(), w_cap, n_v, qst + 4, R.out_off.as<uint64_t>(), q_bytes,
-                          R.out.as<uint64_t>(), s);
-        f->stats.kernel_launches += 6;
-        std::vector<uint64_t> counts(n_list), out_at(n_list);
-        CK(cudaMemcpyAsync(out_at.data(), R.out_at.p, n_list * 8, cudaMemcpyDeviceToHost, s));
-        CK(cudaMemcpyAsync(counts.data(), R.counts.p, n_list * 8, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        CK(cudaGetLastError());
-        // final layout + where each contig's codes come from (clean layout or the repaired runs)
-        std::vector<uint64_t> src_off(n_contigs);
-        uint64_t new_total = 0, clean_run = 0;
-        for (uint64_t c = 0, j = 0; c < n_contigs; ++c) {
-            uint64_t len = offsets[c + 1] - offsets[c];
-            uint64_t clean_cnt = len >= k ? len - k + 1 : 0;
-            uint64_t cnt = clean_cnt;
-            if (dirty[c]) {
-                src_off[c] = out_at[j];
-                cnt = counts[j++];
-            } else {
-                src_off[c] = clean_run;
-            }
-            clean_run += clean_cnt;
-            code_offsets[c] = new_total;
-            new_total += cnt;
-        }
-        code_offsets[n_contigs] = new_total;
-        *n_codes = new_total;
-        if (!want_runs && new_total > codes_capacity) return fail(LPHB_E_CAPACITY, "codes buffer too small");
-        if (want_runs && new_total >= (1ull << 31)) return fail(LPHB_E_ARG, "batch holds >= 2^31 codes: split it");
-        R.src_off.reserve((n_contigs + 1) * 8);
-        R.assembled.reserve(new_total * 8 + 64);
-        CK(cudaMemcpyAsync(R.src_off.p, src_off.data(), n_contigs * 8, cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(ws.code_off.p, code_offsets, (n_contigs + 1) * 8, cudaMemcpyHostToDevice, s));
-        launch_assemble(R.assembled.as<uint64_t>(), ws.code_off.as<uint64_t>(), ws.codes.as<uint64_t>(), R.out.as<uint64_t>(),
-                        R.src_off.as<uint64_t>(), ws.dirty.as<uint8_t>(), n_contigs, new_total, s);
-        f->stats.kernel_launches += 1;
-        if (want_runs) reserve_runs(new_total + 16, 1, new_total, 1);
-        *new_total_out = new_total;
-        *d2h_bytes = n_contigs + n_list * 8;
-        return LPHB_OK;
-    }
-
     // ---- output: the n codes d_codes of the batch, laid out as ws.code_off says, to the caller as codes or runs
     int output(const uint64_t* d_codes, uint64_t n, uint64_t d2h_before) {
         if (!want_runs && n > codes_capacity) return fail(LPHB_E_CAPACITY, "codes buffer too small");
@@ -693,6 +720,125 @@ int query_stream_host(lphb_mphf* f, const char* bases, const uint64_t* offsets, 
         HostQuery q{f, bases, offsets, n_contigs, codes, codes_capacity, code_offsets, n_codes, sink};
         return q.run();
     });
+}
+
+// ---- batches in the caller's device buffers ------------------------------------------------------
+
+// lphb_query_stream_device and lphb_query_nonstreaming_device: the stateless codes of the batch, enqueued on s.
+// non_streaming: the kernels read a copy of the batch's bytes in the workspace with every non-ACGT byte made 'A',
+// so that every window has its code and the caller's bytes stay as they are.
+int device_query(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
+                 uint64_t n_contigs, uint64_t* d_codes, uint64_t codes_capacity, uint64_t* d_code_offsets,
+                 unsigned long long* st, cudaStream_t s, bool non_streaming) {
+    f->stats = lphb_stats{};
+    const uint32_t k = f->img.k;
+    const uint64_t total = contig_layout(h_offsets, n_contigs, k).kmers;
+    if (total > codes_capacity) return fail(LPHB_E_CAPACITY, "codes buffer too small");
+    if (total && (!d_bases || !d_codes)) return fail(LPHB_E_ARG, "null data pointer");
+    const uint64_t first = h_offsets[0], span = h_offsets[n_contigs] - first;
+    if (non_streaming && span && !d_bases) return fail(LPHB_E_ARG, "null data pointer");
+    Workspace& ws = f->ws;
+    // (growing a workspace buffer frees the old one: cudaFree waits for the device, so a previous
+    // call still running never loses its buffer)
+    ws.offsets_tmp.reserve(code_offsets_tmp_bytes(n_contigs));
+    ws.dirty.reserve(n_contigs + 8);
+    ws.tile.reserve(query_tiled_ws_bytes(span));
+    if (non_streaming) ws.bases.reserve(span + 16 + kCopySanitizePad);
+    ws.order_after_previous(s);
+    CK(cudaMemsetAsync(ws.dirty.p, 0, n_contigs + 8, s));
+    launch_code_offsets(d_offsets, n_contigs, k, d_code_offsets, st, ws.offsets_tmp.p, ws.offsets_tmp.cap, s);
+    f->stats.kernel_launches += 2;
+    const char* bases = d_bases;
+    if (non_streaming && span) {
+        launch_copy_sanitize(ws.bases.as<char>(), d_bases + first, span, s);
+        bases = ws.bases.as<char>() + copy_sanitize_at(d_bases + first) - first;  // indexed by the offsets
+        f->stats.kernel_launches += 1;
+    }
+    DevBatch b{};
+    b.bases = bases;
+    b.offsets = d_offsets;
+    b.code_off = d_code_offsets;
+    b.n_contigs = n_contigs;
+    b.first_base = first;
+    b.end_base = h_offsets[n_contigs];
+    b.codes = d_codes;
+    b.dirty = ws.dirty.as<uint8_t>();
+    b.status = st;
+    b.tile_ws = ws.tile.p;
+    b.tile_ws_bytes = ws.tile.cap;
+    if (n_contigs) run_kernels(f, b, s);
+    ws.mark_last(s);
+    f->last_dirty_n = n_contigs;
+    f->last_dirty = nullptr;
+    CK(cudaGetLastError());
+    return LPHB_OK;
+}
+
+// lphb_query_stream_exact_device: the clean pass of lphb_query_stream_device over the caller's batch, one read-back
+// of its status and, when a contig holds a non-ACGT byte, the repair lphb_query_stream runs.  The clean pass writes
+// straight into d_codes when the clean layout fits there, so a clean batch costs one device call more than the
+// stateless form: the status read.  A repair then assembles from a copy of those codes in the workspace, since the
+// assemble must not read the buffer it writes.
+int exact_device_query(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
+                       uint64_t n_contigs, uint64_t* d_codes, uint64_t codes_capacity, uint64_t* d_code_offsets,
+                       uint64_t* n_codes, cudaStream_t s) {
+    f->stats = lphb_stats{};
+    Workspace& ws = f->ws;
+    const uint32_t k = f->img.k;
+    std::vector<uint64_t> code_offsets(n_contigs + 1);
+    const uint64_t total = contig_layout(h_offsets, n_contigs, k, 0, code_offsets.data()).kmers;
+    *n_codes = total;
+    const uint64_t first = h_offsets[0], span = h_offsets[n_contigs] - first;
+    // (a contig shorter than k yields no code, spurious ones included: without a clean code there is none at all)
+    if ((span && !d_bases) || (total && !d_codes)) return fail(LPHB_E_ARG, "null data pointer");
+    const bool in_place = total <= codes_capacity;
+    ws.offsets_tmp.reserve(code_offsets_tmp_bytes(n_contigs));
+    ws.dirty.reserve(n_contigs + 8);
+    ws.tile.reserve(query_tiled_ws_bytes(span));
+    if (!in_place) ws.codes.reserve(total * 8 + 64);
+    ws.order_after_previous(s);
+    CK(cudaMemsetAsync(ws.dirty.p, 0, n_contigs + 8, s));
+    auto* st = ws.status.as<unsigned long long>();
+    launch_code_offsets(d_offsets, n_contigs, k, d_code_offsets, st, ws.offsets_tmp.p, ws.offsets_tmp.cap, s);
+    f->stats.kernel_launches += 2;
+    DevBatch b{};
+    b.bases = d_bases;
+    b.offsets = d_offsets;
+    b.code_off = d_code_offsets;
+    b.n_contigs = n_contigs;
+    b.first_base = first;
+    b.end_base = h_offsets[n_contigs];
+    b.codes = in_place ? d_codes : ws.codes.as<uint64_t>();
+    b.dirty = ws.dirty.as<uint8_t>();
+    b.status = st;
+    b.tile_ws = ws.tile.p;
+    b.tile_ws_bytes = ws.tile.cap;
+    if (n_contigs) run_kernels(f, b, s);
+    ws.mark_last(s);
+    f->last_dirty_n = n_contigs;
+    f->last_dirty = nullptr;
+    auto* h_status = ws.h_status.as<unsigned long long>();
+    CK(cudaMemcpyAsync(h_status, st, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    CK(cudaGetLastError());
+    f->stats.d2h_bytes = 4 * sizeof(unsigned long long);
+    f->stats.dirty_contigs = h_status[1];
+    if (h_status[1] == 0) return in_place ? LPHB_OK : fail(LPHB_E_CAPACITY, "codes buffer too small");
+    if (in_place) {
+        ws.codes.reserve(total * 8 + 64);
+        CK(cudaMemcpyAsync(ws.codes.p, d_codes, total * 8, cudaMemcpyDeviceToDevice, s));
+    }
+    const DirtyBatch db{d_bases, d_offsets, h_offsets, n_contigs, ws.dirty.as<uint8_t>(), ws.codes.as<uint64_t>()};
+    uint64_t d2h_repair = 0;
+    const uint64_t new_total = repair_layout(f, db, code_offsets.data(), s, &d2h_repair);
+    *n_codes = new_total;
+    f->stats.d2h_bytes += d2h_repair;
+    if (new_total > codes_capacity) return fail(LPHB_E_CAPACITY, "codes buffer too small");
+    repair_assemble(f, db, code_offsets.data(), new_total, d_code_offsets, d_codes, s);
+    ws.mark_last(s);
+    CK(cudaStreamSynchronize(s));
+    CK(cudaGetLastError());
+    return LPHB_OK;
 }
 
 // ---- lookup of packed k-mers ---------------------------------------------------------------------
@@ -1185,40 +1331,34 @@ int lphb_query_stream_device(lphb_mphf* f, const char* d_bases, const uint64_t* 
         return fail(LPHB_E_ARG, "null argument");
     return guarded([&]() -> int {
         DeviceGuard g(f->device);
-        cudaStream_t s = static_cast<cudaStream_t>(stream);
-        f->stats = lphb_stats{};
-        const uint32_t k = f->img.k;
-        const uint64_t total = contig_layout(h_offsets, n_contigs, k).kmers;
-        if (total > codes_capacity) return fail(LPHB_E_CAPACITY, "codes buffer too small");
-        if (total && (!d_bases || !d_codes)) return fail(LPHB_E_ARG, "null data pointer");
-        Workspace& ws = f->ws;
-        // (growing a workspace buffer frees the old one: cudaFree waits for the device, so a previous
-        // call still running never loses its buffer)
-        ws.offsets_tmp.reserve(code_offsets_tmp_bytes(n_contigs));
-        ws.dirty.reserve(n_contigs + 8);
-        ws.tile.reserve(query_tiled_ws_bytes(h_offsets[n_contigs] - h_offsets[0]));
-        ws.order_after_previous(s);
-        CK(cudaMemsetAsync(ws.dirty.p, 0, n_contigs + 8, s));
-        auto* st = reinterpret_cast<unsigned long long*>(d_status);
-        launch_code_offsets(d_offsets, n_contigs, k, d_code_offsets, st, ws.offsets_tmp.p, ws.offsets_tmp.cap, s);
-        f->stats.kernel_launches += 2;
-        DevBatch b{};
-        b.bases = d_bases;
-        b.offsets = d_offsets;
-        b.code_off = d_code_offsets;
-        b.n_contigs = n_contigs;
-        b.first_base = h_offsets[0];
-        b.end_base = h_offsets[n_contigs];
-        b.codes = d_codes;
-        b.dirty = ws.dirty.as<uint8_t>();
-        b.status = st;
-        b.tile_ws = ws.tile.p;
-        b.tile_ws_bytes = ws.tile.cap;
-        if (n_contigs) run_kernels(f, b, s);
-        ws.mark_last(s);
-        f->last_dirty_n = n_contigs;
-        CK(cudaGetLastError());
-        return LPHB_OK;
+        return device_query(f, d_bases, d_offsets, h_offsets, n_contigs, d_codes, codes_capacity, d_code_offsets,
+                            reinterpret_cast<unsigned long long*>(d_status), static_cast<cudaStream_t>(stream), false);
+    });
+}
+
+int lphb_query_nonstreaming_device(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets,
+                                   const uint64_t* h_offsets, uint64_t n_contigs, uint64_t* d_codes,
+                                   uint64_t codes_capacity, uint64_t* d_code_offsets, uint64_t* d_status,
+                                   void* stream) {
+    if (!f || !d_offsets || !h_offsets || !d_code_offsets || !d_status)
+        return fail(LPHB_E_ARG, "null argument");
+    return guarded([&]() -> int {
+        DeviceGuard g(f->device);
+        return device_query(f, d_bases, d_offsets, h_offsets, n_contigs, d_codes, codes_capacity, d_code_offsets,
+                            reinterpret_cast<unsigned long long*>(d_status), static_cast<cudaStream_t>(stream), true);
+    });
+}
+
+int lphb_query_stream_exact_device(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets,
+                                   const uint64_t* h_offsets, uint64_t n_contigs, uint64_t* d_codes,
+                                   uint64_t codes_capacity, uint64_t* d_code_offsets, uint64_t* n_codes,
+                                   void* stream) {
+    if (!f || !d_offsets || !h_offsets || !d_code_offsets || !n_codes)
+        return fail(LPHB_E_ARG, "null argument");
+    return guarded([&]() -> int {
+        DeviceGuard g(f->device);
+        return exact_device_query(f, d_bases, d_offsets, h_offsets, n_contigs, d_codes, codes_capacity, d_code_offsets,
+                                  n_codes, static_cast<cudaStream_t>(stream));
     });
 }
 

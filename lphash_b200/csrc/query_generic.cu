@@ -85,6 +85,38 @@ __global__ void k_sanitize(char* bases, uint64_t n) {
         if (nt4(uint8_t(bases[i])) > 3) bases[i] = 'A';
 }
 
+__device__ __forceinline__ uint32_t sanitize4(uint32_t w) {
+    uint32_t out = 0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const uint32_t ch = (w >> (8 * i)) & 0xFFu;
+        out |= (nt4(ch) > 3 ? uint32_t('A') : ch) << (8 * i);
+    }
+    return out;
+}
+
+// dst[0..n) = src[0..n) with k_sanitize's mapping, then `pad` bytes of 'A' (the read-ahead of the last tile).  dst and
+// src have the same address mod 16: the bytes before the first 16-byte boundary and after the last are copied one by
+// one, everything between in 16-byte vectors, streamed (each byte is read and written once).
+__global__ void __launch_bounds__(256) k_copy_sanitize(char* dst, const char* src, uint64_t n, uint32_t pad) {
+    const uint64_t tid = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x, stride = uint64_t(gridDim.x) * blockDim.x;
+    const uint64_t head = min(n, uint64_t((16u - uint32_t(reinterpret_cast<uintptr_t>(src) & 15u)) & 15u));
+    const uint64_t n_vec = (n - head) / 16, tail = head + n_vec * 16;
+    const uint4* s4 = reinterpret_cast<const uint4*>(src + head);
+    uint4* d4 = reinterpret_cast<uint4*>(dst + head);
+    for (uint64_t i = tid; i < n_vec; i += stride) {
+        uint4 v = __ldcs(s4 + i);
+        v.x = sanitize4(v.x);
+        v.y = sanitize4(v.y);
+        v.z = sanitize4(v.z);
+        v.w = sanitize4(v.w);
+        __stcs(d4 + i, v);
+    }
+    if (tid < head) dst[tid] = nt4(uint8_t(src[tid])) > 3 ? 'A' : src[tid];
+    if (tid < n - tail) dst[tail + tid] = nt4(uint8_t(src[tail + tid])) > 3 ? 'A' : src[tail + tid];
+    if (tid < pad) dst[n + tid] = 'A';
+}
+
 __global__ void k_count_dirty(const uint8_t* dirty, uint64_t n, unsigned long long* status) {
     unsigned long long local = 0;
     for (uint64_t c = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; c < n;
@@ -131,6 +163,16 @@ void launch_sanitize(char* d_bases, uint64_t n, cudaStream_t stream) {
     uint64_t blocks = (n + 255) / 256;
     if (blocks > 148ull * 16) blocks = 148ull * 16;
     k_sanitize<<<unsigned(blocks), 256, 0, stream>>>(d_bases, n);
+}
+
+uint64_t copy_sanitize_at(const char* src) { return reinterpret_cast<uintptr_t>(src) & 15u; }
+
+void launch_copy_sanitize(char* d_dst, const char* d_src, uint64_t n, cudaStream_t stream) {
+    char* dst = d_dst + copy_sanitize_at(d_src);
+    uint64_t blocks = (n / 16 + 255) / 256;
+    if (blocks < 1) blocks = 1;
+    if (blocks > 148ull * 16) blocks = 148ull * 16;
+    k_copy_sanitize<<<unsigned(blocks), 256, 0, stream>>>(dst, d_src, n, kCopySanitizePad);
 }
 
 void launch_count_dirty(const uint8_t* dirty, uint64_t n, unsigned long long* status,

@@ -98,6 +98,13 @@ void launch_runs(const uint64_t* codes, uint64_t n, const uint64_t* code_off, ui
 // non-ACGT bytes -> 'A' in place (the reference's non-streaming branch, include/mphf_utils.hpp:108)
 void launch_sanitize(char* d_bases, uint64_t n, cudaStream_t stream);
 
+// The same into a copy: d_src[0..n) (any alignment, not modified) -> d_dst + copy_sanitize_at(d_src), which has
+// d_src's address mod 16, followed by kCopySanitizePad bytes of 'A'.  d_dst: 16-byte aligned,
+// n + 16 + kCopySanitizePad bytes.
+constexpr uint32_t kCopySanitizePad = 64;
+uint64_t copy_sanitize_at(const char* d_src);
+void launch_copy_sanitize(char* d_dst, const char* d_src, uint64_t n, cudaStream_t stream);
+
 // status[1] += number of set flags in dirty[0..n)
 void launch_count_dirty(const uint8_t* dirty, uint64_t n, unsigned long long* status,
                         cudaStream_t stream);
