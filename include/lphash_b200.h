@@ -191,6 +191,60 @@ int lphb_lookup_kmers(lphb_mphf* f, const void* kmers, uint64_t n, uint64_t* cod
  * and ordered against the handle's other calls as lphb_query_stream_device is.                             */
 int lphb_lookup_kmers_device(lphb_mphf* f, const void* d_kmers, uint64_t n, uint64_t* d_codes, void* stream);
 
+/* ---- the index self-check: build-p --check ---------------------------------------------------------------------
+ * Replaces `check` (include/mphf_utils.hpp:51-100; caller src/build.cpp:36-43), which runs three tests over the
+ * index's input, contig by contig: check_collisions (every non-streaming code is in range and was not seen before),
+ * check_streaming_correctness (the streaming codes equal the non-streaming ones) and check_perfection (every code of
+ * 0..nkmers-1 is hit).  Here one kernel does the first two for every window of k bytes of a batch, and the third
+ * runs at the end of a SESSION, which spans any number of batches: a unitig file larger than one batch is checked as
+ * a stream.  The report does not depend on how the input is split into batches, nor on host versus device form.
+ *
+ * Definitions, per window of k bytes of the session's contigs, in session order (the k-mer ORDINAL: the position of
+ * the window in the non-streaming layout, sum of max(0, L-k+1) over the contigs before it plus its offset):
+ *   - its non-streaming code is that of lphb_query_nonstreaming: a non-ACGT byte counts as 'A'
+ *     (include/mphf_utils.hpp:108);
+ *   - a contig holding a byte outside ACGT/acgt/U/u is DIRTY, whatever its length.  Its windows are checked for
+ *     range and collisions like every other, but left out of the streaming comparison: its streaming slots are
+ *     unspecified in the stateless layout (lphb_query_stream_device).  The reference compares the two branches
+ *     element by element (include/mphf_utils.hpp:83-100), which the streaming branch's spurious codes on such a
+ *     contig would fail; on ACGT-only input the verdicts agree (DESIGN.md 4.11);
+ *   - a code >= nkmers is OUT OF RANGE.  (The reference tests hash <= nkmers, include/mphf_utils.hpp:58; with a code
+ *     equal to nkmers on the key set some code of [0, nkmers) stays unhit, so its perfection test fails and the
+ *     overall verdict is the same.)
+ * The bitmap of nkmers bits (nkmers / 8 bytes of HBM, kept by the handle and grown only) lives for the session.   */
+typedef struct lphb_check_report {
+    uint64_t kmers;              /* windows checked: sum of max(0, L-k+1) over the session's contigs        */
+    uint64_t contigs, dirty_contigs;
+    uint64_t out_of_range;       /* non-streaming codes >= nkmers                                            */
+    uint64_t duplicates;         /* in-range hits on a code already hit (= hits - distinct codes hit)        */
+    uint64_t missing;            /* codes of [0, nkmers) never hit                                           */
+    uint64_t stream_mismatches;  /* windows of clean contigs whose streaming code != non-streaming code      */
+    uint64_t first_out_of_range; /* k-mer ordinal in session order; UINT64_MAX if none                       */
+    uint64_t first_mismatch;     /* likewise                                                                 */
+    uint64_t min_duplicate_code, min_missing_code; /* UINT64_MAX if none                                     */
+    int32_t ok;                  /* 1 iff out_of_range, duplicates, missing and stream_mismatches are all 0  */
+} lphb_check_report;
+
+/* (Re)starts the handle's session: clears the bitmap and the counters.  Ordered against the handle's other calls. */
+int lphb_check_begin(lphb_mphf* f);
+
+/* One batch of the session, HOST buffers (as lphb_query_stream takes them).  The bases go up in contig-aligned
+ * chunks of LPHB_CHUNK_BASES through the query path's staging; the streaming pass runs on the device and no code
+ * comes back.  Returns once the caller's buffers may be reused.  LPHB_E_ARG without an open session.              */
+int lphb_check_batch(lphb_mphf* f, const char* bases, const uint64_t* offsets, uint64_t n_contigs);
+
+/* The same for a batch in device buffers (arguments as in lphb_query_stream_device), asynchronous on `stream` and
+ * ordered against the handle's other calls: queries may run between the batches of a session.  d_stream_codes is
+ * optional: when given, it holds the caller's streaming codes of this batch in the layout lphb_query_stream_device
+ * writes, and they are compared instead of the library running the streaming pass itself (so that a pipeline can
+ * verify codes it already produced).                                                                           */
+int lphb_check_batch_device(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
+                            uint64_t n_contigs, const uint64_t* d_stream_codes, void* stream);
+
+/* Ends the session: counts the missing codes, synchronises and fills *report.  LPHB_E_ARG without an open session.
+ * After a check call lphb_mphf_stats reports that call, lphb_mphf_dirty_flags the last batch's contigs.          */
+int lphb_check_end(lphb_mphf* f, lphb_check_report* report);
+
 /* Diagnostic: the flat device image behind the handle (layout: lphash_b200/csrc/device_image.h), e.g. to compare
  * the GPU-side decode of a load with the host-side one (LPHB_HOST_DECODE=1).  Read it with lphb_copy_to_host.  */
 int lphb_mphf_device_image(const lphb_mphf* f, const void** d_image, uint64_t* nbytes);

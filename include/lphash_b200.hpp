@@ -201,6 +201,35 @@ public:
         if (rc != LPHB_OK) detail::raise("lphash_b200::mphf::query_batch_device_nonstreaming", rc);
     }
 
+    // build-p --check (include/mphf_utils.hpp:51-100) as a session over any number of batches of the index's contigs
+    // (lphb_check_*): check_begin, check_batch / check_batch_device per batch, check_end for the report.
+    // check_batch takes host buffers and returns once they may be reused; check_batch_device takes device buffers
+    // (as query_batch_device) and is asynchronous on `stream`, d_stream_codes optional (the caller's streaming codes
+    // of the batch in the layout of lphb_query_stream_device, compared instead of the library's own streaming pass).
+    void check_begin() {
+        if (!h_) throw std::runtime_error("lphash_b200::mphf: no index loaded");
+        int rc = lphb_check_begin(h_);
+        if (rc != LPHB_OK) detail::raise("lphash_b200::mphf::check_begin", rc);
+    }
+    void check_batch(const char* bases, const uint64_t* offsets, uint64_t n_contigs) {
+        if (!h_) throw std::runtime_error("lphash_b200::mphf: no index loaded");
+        int rc = lphb_check_batch(h_, bases, offsets, n_contigs);
+        if (rc != LPHB_OK) detail::raise("lphash_b200::mphf::check_batch", rc);
+    }
+    void check_batch_device(const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
+                            uint64_t n_contigs, const uint64_t* d_stream_codes = nullptr, void* stream = nullptr) {
+        if (!h_) throw std::runtime_error("lphash_b200::mphf: no index loaded");
+        int rc = lphb_check_batch_device(h_, d_bases, d_offsets, h_offsets, n_contigs, d_stream_codes, stream);
+        if (rc != LPHB_OK) detail::raise("lphash_b200::mphf::check_batch_device", rc);
+    }
+    lphb_check_report check_end() {
+        if (!h_) throw std::runtime_error("lphash_b200::mphf: no index loaded");
+        lphb_check_report r{};
+        int rc = lphb_check_end(h_, &r);
+        if (rc != LPHB_OK) detail::raise("lphash_b200::mphf::check_end", rc);
+        return r;
+    }
+
     lphb_mphf* handle() const noexcept { return h_; }
 
 private:

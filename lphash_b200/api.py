@@ -66,6 +66,18 @@ class Stats(C.Structure):
                 ("dirty_contigs", C.c_uint64), ("kernel_ms", C.c_double)]
 
 
+class CheckReport(C.Structure):
+    """lphb_check_report: the verdict of a check session (lphb_check_begin .. lphb_check_end).  first_out_of_range and
+    first_mismatch are k-mer ordinals in session order; they and the two code fields are 2^64 - 1 when there is none."""
+    _fields_ = [("kmers", C.c_uint64), ("contigs", C.c_uint64), ("dirty_contigs", C.c_uint64),
+                ("out_of_range", C.c_uint64), ("duplicates", C.c_uint64), ("missing", C.c_uint64),
+                ("stream_mismatches", C.c_uint64), ("first_out_of_range", C.c_uint64), ("first_mismatch", C.c_uint64),
+                ("min_duplicate_code", C.c_uint64), ("min_missing_code", C.c_uint64), ("ok", C.c_int32)]
+
+    def as_dict(self) -> dict:
+        return {name: getattr(self, name) for name, _ in self._fields_}
+
+
 # every symbol include/lphash_b200.h declares (tests check the library exports all of them)
 EXPORTS = ["lphb_last_error", "lphb_version", "lphb_device_count", "lphb_mphf_load_file",
            "lphb_mphf_load_memory", "lphb_mphf_free", "lphb_mphf_info", "lphb_query_stream",
@@ -76,7 +88,8 @@ EXPORTS = ["lphb_last_error", "lphb_version", "lphb_device_count", "lphb_mphf_lo
            "lphb_mphf_alt_load_file", "lphb_mphf_alt_load_memory", "lphb_inverted_index_bound",
            "lphb_build_inverted_index", "lphb_lph_assemble", "lphb_lph_sections", "lphb_build_inverted_index_alt",
            "lphb_lph_assemble_alt", "lphb_mphf_device_image", "lphb_lookup_kmers", "lphb_lookup_kmers_device",
-           "lphb_query_stream_exact_device", "lphb_query_nonstreaming_device"]
+           "lphb_query_stream_exact_device", "lphb_query_nonstreaming_device", "lphb_check_begin", "lphb_check_batch",
+           "lphb_check_batch_device", "lphb_check_end"]
 
 _lib = None
 
@@ -108,6 +121,10 @@ def lib() -> C.CDLL:
     L.lphb_query_nonstreaming_device.argtypes = [p, p, p, p, u64, p, u64, p, p, p]
     L.lphb_lookup_kmers.argtypes = [p, p, u64, p]
     L.lphb_lookup_kmers_device.argtypes = [p, p, u64, p, p]
+    L.lphb_check_begin.argtypes = [p]
+    L.lphb_check_batch.argtypes = [p, p, p, u64]
+    L.lphb_check_batch_device.argtypes = [p, p, p, p, u64, p, p]
+    L.lphb_check_end.argtypes = [p, C.POINTER(CheckReport)]
     L.lphb_query_stream_runs.argtypes = [p, p, p, u64, p, u64, C.POINTER(u64), p, C.POINTER(u64)]
     L.lphb_expand_runs.argtypes = [p, u64, p, u64, C.POINTER(u64), i32]
     L.lphb_mphf_dirty_flags.argtypes = [p, C.POINTER(p), C.POINTER(u64)]
@@ -332,6 +349,41 @@ class Mphf:
         """lphb_lookup_kmers_device: asynchronous on `stream`; raw device pointers (ints), e.g. tensor.data_ptr(),
         d_kmers holding n k-mers of kmer_bits / 8 bytes each."""
         _check(lib().lphb_lookup_kmers_device(self._h, d_kmers, n, d_codes, stream))
+
+    # -- the index self-check (build-p --check) ---------------------------------------------------------------------
+    def check_begin(self) -> None:
+        """lphb_check_begin: (re)starts the handle's check session"""
+        _check(lib().lphb_check_begin(self._h))
+
+    def check_batch(self, bases, offsets) -> None:
+        """lphb_check_batch: one batch of the session, host arrays as query_batch takes them"""
+        bases, offsets = _as_batch(bases, offsets)
+        if np.any(np.diff(offsets.astype(np.int64)) < 0):
+            raise ValueError("offsets must be non-decreasing")
+        if int(offsets[-1]) > len(bases):
+            raise ValueError("offsets index past the end of bases")
+        _check(lib().lphb_check_batch(self._h, bases.ctypes.data, offsets.ctypes.data, len(offsets) - 1))
+
+    def check_batch_device(self, d_bases: int, d_offsets: int, h_offsets: np.ndarray, d_stream_codes: int = 0,
+                           stream: int = 0) -> None:
+        """lphb_check_batch_device: raw device pointers (ints) as in query_device; d_stream_codes (0: none) holds the
+        caller's streaming codes of the batch in query_device's layout.  Asynchronous on `stream`."""
+        h_offsets = np.ascontiguousarray(h_offsets, dtype=np.uint64)
+        _check(lib().lphb_check_batch_device(self._h, d_bases, d_offsets, h_offsets.ctypes.data, len(h_offsets) - 1,
+                                             d_stream_codes or None, stream))
+
+    def check_end(self) -> CheckReport:
+        """lphb_check_end: closes the session and returns its report"""
+        r = CheckReport()
+        _check(lib().lphb_check_end(self._h, C.byref(r)))
+        return r
+
+    def check(self, bases, offsets) -> CheckReport:
+        """one-batch session: is this handle a minimal perfect hash of these contigs' k-mers, and do its streaming
+        and non-streaming codes agree on them?"""
+        self.check_begin()
+        self.check_batch(bases, offsets)
+        return self.check_end()
 
 
 RUN_DTYPE = np.dtype([("first", "<u8"), ("n", "<i4")])  # 12 bytes packed: lphb_query_stream_runs records

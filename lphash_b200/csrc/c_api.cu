@@ -18,6 +18,7 @@
 
 #include "../../include/lphash_b200.h"
 #include "api_internal.h"
+#include "check_kernels.cuh"
 #include "image_decode.cuh"
 #include "lph_image.h"
 #include "query_kernels.cuh"
@@ -68,6 +69,15 @@ struct Workspace {
     // the kernels of chunk j and the D2H copy of chunk j-1 overlap (PCIe is full duplex)
     Stream cs[2];
     Event ev_ready, ev_done[2];
+    // session of the index self-check (lphb_check_begin .. lphb_check_end)
+    struct Check {
+        bool open = false;
+        DevBuf bitmap;    // one bit per code of [0, nkmers): hit
+        DevBuf counters;  // kCheckCounters words (check_kernels.cuh)
+        HostBuf h_counters;
+        uint64_t kmers = 0, contigs = 0;  // of the batches so far: the next batch's first k-mer ordinal
+        uint64_t host_dirty = 0;          // dirty contigs the host form counted (the device form counts in `counters`)
+    } check;
     // The handle has ONE device workspace (dirty flags, tile records, scan scratch).  Calls may arrive
     // on different streams (lphb_query_stream_device takes the caller's): every call first makes its
     // stream wait for the previous call's last kernel, so that two calls never share the workspace
@@ -264,18 +274,52 @@ void timed_launch(lphb_mphf* f, cudaStream_t s, Launch&& launch) {
     ++f->ws.ev_pending;
 }
 
+// the streaming query kernel over a batch: tiled where (k, m) is instantiated, else generic
+void launch_stream_pass(lphb_mphf* f, DevBatch const& b, cudaStream_t s) {
+    // A batch of a few tiles would leave one or two warps of the tiled kernel to walk its whole (cold) code
+    // alone, about 40 us whatever the size; below 256 K bases the one-thread-per-k-mer kernel answers sooner
+    // (10 us for a record of 8,000 bases; tools/ubench/call_latency.cpp).  LPHB_GENERIC_BELOW overrides (tests: 0).
+    const char* gb = getenv("LPHB_GENERIC_BELOW");
+    const uint64_t generic_below = gb ? strtoull(gb, nullptr, 10) : (uint64_t(1) << 18);
+    if (b.end_base - b.first_base < generic_below || !launch_query_tiled(f->img, b, s))
+        launch_query_generic(f->img, b, s);
+}
+
 void run_kernels(lphb_mphf* f, DevBatch const& b, cudaStream_t s) {
-    timed_launch(f, s, [&] {
-        // A batch of a few tiles would leave one or two warps of the tiled kernel to walk its whole (cold) code
-        // alone, about 40 us whatever the size; below 256 K bases the one-thread-per-k-mer kernel answers sooner
-        // (10 us for a record of 8,000 bases; tools/ubench/call_latency.cpp).  LPHB_GENERIC_BELOW overrides (tests: 0).
-        const char* gb = getenv("LPHB_GENERIC_BELOW");
-        const uint64_t generic_below = gb ? strtoull(gb, nullptr, 10) : (uint64_t(1) << 18);
-        if (b.end_base - b.first_base < generic_below || !launch_query_tiled(f->img, b, s))
-            launch_query_generic(f->img, b, s);
-    });
+    timed_launch(f, s, [&] { launch_stream_pass(f, b, s); });
     launch_count_dirty(b.dirty, b.n_contigs, b.status, s);
     f->stats.kernel_launches += 2;
+}
+
+// ---- the index self-check (lphb_check_*) -----------------------------------------------------------------------
+// One batch or chunk b (bases, offsets, code_off from ordinal j0 of the batch on, n_contigs, dirty zeroed) through
+// the check: the contigs' dirty flags (any non-ACGT byte, whatever the contig's length) counted into
+// dirty_status[1]; unless the caller gave its own streaming codes, the streaming pass into b.codes; then the check
+// kernel, timed, over the ordinals [j0, j1) of the batch.
+void check_chunk(lphb_mphf* f, DevBatch const& b, uint64_t j0, uint64_t j1, const uint64_t* caller_codes,
+                 unsigned long long* dirty_status, cudaStream_t s) {
+    Workspace::Check& C = f->ws.check;
+    launch_flag_invalid_bytes(b.bases, b.first_base, b.end_base - b.first_base, b.offsets, b.n_contigs, b.dirty, s);
+    launch_count_dirty(b.dirty, b.n_contigs, dirty_status, s);
+    f->stats.kernel_launches += 2;
+    if (!caller_codes && j1 > j0) {
+        launch_stream_pass(f, b, s);
+        f->stats.kernel_launches += 1;
+    }
+    CheckBatch cb{};
+    cb.bases = b.bases;
+    cb.offsets = b.offsets;
+    cb.code_off = b.code_off;
+    cb.n_contigs = b.n_contigs;
+    cb.j0 = j0;
+    cb.j1 = j1;
+    cb.ordinal_base = C.kmers;
+    cb.stream_codes = caller_codes ? caller_codes : b.codes;
+    cb.dirty = b.dirty;
+    cb.bitmap = C.bitmap.as<uint32_t>();
+    cb.counters = C.counters.as<unsigned long long>();
+    timed_launch(f, s, [&] { launch_check_windows(f->img, cb, s); });
+    f->stats.kernel_launches += 1;
 }
 
 // Layout of a batch of contigs (host offsets): max(0, L-k+1) k-mers per contig and, with m, max(0, L-m+1) m-mers.
@@ -442,6 +486,8 @@ struct RunSink {
     // the reference's NON-streaming branch (include/partitioned_mphf.hpp:185-195): every window of k bytes is a
     // k-mer, a non-ACGT byte counts as 'A' (include/mphf_utils.hpp:108); no streaming state, hence no quirk
     bool non_streaming = false;
+    // the index self-check (lphb_check_batch): every chunk goes through check_chunk; no code leaves the device
+    bool check = false;
 };
 
 // One call of lphb_query_stream, lphb_query_nonstreaming or lphb_query_stream_runs with its batch on the host.
@@ -461,7 +507,7 @@ struct HostQuery {
     cudaStream_t s = ws.stream;
     const bool want_runs = sink.runs != nullptr || sink.n_runs != nullptr;
     uint64_t first = 0, span = 0, total = 0;  // bases of the batch, codes of the clean layout
-    bool copied_out = false;  // the clean pass copied every chunk's results out
+    bool copied_out = false;  // the clean pass copied every chunk's results out (a check: ran its chunks piped)
     uint64_t n_chunks = 1;
     uint64_t runs_per = 0;    // codes per scratch set of the run-length pass
     uint64_t runs_done = 0;   // run records already placed in the caller's buffer
@@ -481,6 +527,10 @@ struct HostQuery {
         f->last_dirty = nullptr;
         if (small_call()) return LPHB_OK;
         const uint64_t n_dirty = clean_pass();
+        if (sink.check) {
+            ws.check.host_dirty += n_dirty;
+            return LPHB_OK;
+        }
         if (n_dirty == 0) return copied_out ? finish(total, n_chunks, 0) : output(ws.codes.as<uint64_t>(), total, 0);
         const DirtyBatch db{ws.bases.as<char>() - first, ws.offsets.as<uint64_t>(), offsets, n_contigs,
                             ws.dirty.as<uint8_t>(), ws.codes.as<uint64_t>()};
@@ -503,7 +553,7 @@ struct HostQuery {
         const uint64_t codes_b = (total * 8 + 63) & ~uint64_t(63), dirty_b = (n_contigs + 8 + 63) & ~uint64_t(63);
         const uint64_t off_b = (n_contigs + 1) * 8;
         const uint64_t in_b = 64 + dirty_b + 2 * off_b + span + 64, all_b = codes_b + in_b;
-        if (want_runs || !codes || !total || total > codes_capacity || all_b > Workspace::Small::kBytes ||
+        if (want_runs || sink.check || !codes || !total || total > codes_capacity || all_b > Workspace::Small::kBytes ||
             getenv("LPHB_NO_SMALL_PATH"))
             return false;
         ws.small.d.reserve(Workspace::Small::kBytes);
@@ -576,7 +626,7 @@ struct HostQuery {
         for (uint64_t c = 0; c < n_contigs; ++c)
             if (offsets[c + 1] - offsets[cuts.back()] >= chunk && c + 1 < n_contigs) cuts.push_back(c + 1);
         cuts.push_back(n_contigs);
-        copied_out = cuts.size() > 2 && (want_runs ? sink.runs != nullptr : (total <= codes_capacity && codes));
+        copied_out = cuts.size() > 2 && (sink.check || (want_runs ? sink.runs != nullptr : (total <= codes_capacity && codes)));
         if (!copied_out) cuts = {0, n_contigs};
         n_chunks = cuts.size() - 1;
         std::vector<uint64_t> tile_at(n_chunks + 1, 0);
@@ -613,6 +663,10 @@ struct HostQuery {
             b.status = ws.status.as<unsigned long long>();
             b.tile_ws = static_cast<char*>(ws.tile.p) + tile_at[j];
             b.tile_ws_bytes = tile_at[j + 1] - tile_at[j];
+            if (sink.check) {
+                check_chunk(f, b, code_offsets[c0], code_offsets[c1], nullptr, b.status, st);
+                continue;
+            }
             run_kernels(f, b, st);
             if (copied_out) {
                 emit(j, j & 1, ws.codes.as<uint64_t>(), code_offsets[c0], code_offsets[c1], b.code_off, b.n_contigs, st);
@@ -909,6 +963,106 @@ int lookup_host(lphb_mphf* f, const void* kmers, uint64_t n, uint64_t* codes) {
     ws.mark_last(s);
     CK(cudaStreamSynchronize(s));
     CK(cudaGetLastError());
+    return LPHB_OK;
+}
+
+// ---- the index self-check: sessions ----------------------------------------------------------------------------
+
+// lphb_check_begin: the bitmap and the counters cleared on the handle's stream, ordered after the previous call
+void check_begin(lphb_mphf* f) {
+    Workspace& ws = f->ws;
+    Workspace::Check& C = ws.check;
+    const cudaStream_t s = ws.stream;
+    const uint64_t bitmap_bytes = (f->img.nkmers + 31) / 32 * 4;
+    C.bitmap.reserve(bitmap_bytes + 8);
+    C.counters.reserve(kCheckCounters * 8);
+    C.h_counters.reserve(kCheckCounters * 8);
+    f->stats = lphb_stats{};
+    ws.order_after_previous(s);
+    CK(cudaMemsetAsync(C.bitmap.p, 0, bitmap_bytes + 8, s));
+    CK(cudaMemsetAsync(C.counters.p, 0, kCheckFirstMin * 8, s));
+    CK(cudaMemsetAsync(C.counters.as<unsigned long long>() + kCheckFirstMin, 0xFF, (kCheckCounters - kCheckFirstMin) * 8, s));
+    ws.mark_last(s);
+    CK(cudaGetLastError());
+    C.kmers = C.contigs = C.host_dirty = 0;
+    C.open = true;
+}
+
+// lphb_check_batch_device: asynchronous on s.  The code offsets of the batch go to ws.code_off, the streaming pass
+// (without caller codes) to ws.codes.
+int check_batch_device(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
+                       uint64_t n_contigs, const uint64_t* d_stream_codes, cudaStream_t s) {
+    Workspace& ws = f->ws;
+    Workspace::Check& C = ws.check;
+    f->stats = lphb_stats{};
+    const uint64_t total = contig_layout(h_offsets, n_contigs, f->img.k).kmers;
+    const uint64_t first = h_offsets[0], span = h_offsets[n_contigs] - first;
+    if (span && !d_bases) return fail(LPHB_E_ARG, "d_bases is null");
+    f->last_dirty_n = n_contigs;
+    f->last_dirty = nullptr;
+    if (n_contigs == 0) return LPHB_OK;
+    ws.offsets_tmp.reserve(code_offsets_tmp_bytes(n_contigs));
+    ws.code_off.reserve((n_contigs + 1) * 8);
+    ws.dirty.reserve(n_contigs + 8);
+    if (!d_stream_codes) {
+        ws.codes.reserve(total * 8 + 64);
+        ws.tile.reserve(query_tiled_ws_bytes(span));
+    }
+    ws.order_after_previous(s);
+    CK(cudaMemsetAsync(ws.dirty.p, 0, n_contigs + 8, s));
+    launch_code_offsets(d_offsets, n_contigs, f->img.k, ws.code_off.as<uint64_t>(), ws.status.as<unsigned long long>(),
+                        ws.offsets_tmp.p, ws.offsets_tmp.cap, s);
+    f->stats.kernel_launches += 2;
+    DevBatch b{};
+    b.bases = d_bases;
+    b.offsets = d_offsets;
+    b.code_off = ws.code_off.as<uint64_t>();
+    b.n_contigs = n_contigs;
+    b.first_base = first;
+    b.end_base = h_offsets[n_contigs];
+    b.codes = ws.codes.as<uint64_t>();
+    b.dirty = ws.dirty.as<uint8_t>();
+    b.status = ws.status.as<unsigned long long>();
+    b.tile_ws = ws.tile.p;
+    b.tile_ws_bytes = ws.tile.cap;
+    check_chunk(f, b, 0, total, d_stream_codes, C.counters.as<unsigned long long>(), s);
+    ws.mark_last(s);
+    CK(cudaGetLastError());
+    C.kmers += total;
+    C.contigs += n_contigs;
+    return LPHB_OK;
+}
+
+// lphb_check_end: the missing codes, the counters to the host, the session closed
+int check_end(lphb_mphf* f, lphb_check_report* r) {
+    Workspace& ws = f->ws;
+    Workspace::Check& C = ws.check;
+    const cudaStream_t s = ws.stream;
+    const uint64_t nkmers = f->img.nkmers;
+    C.open = false;
+    ws.order_after_previous(s);
+    launch_check_missing(C.bitmap.as<uint32_t>(), nkmers, C.counters.as<unsigned long long>(), s);
+    auto* h = C.h_counters.as<unsigned long long>();
+    CK(cudaMemcpyAsync(h, C.counters.p, kCheckCounters * 8, cudaMemcpyDeviceToHost, s));
+    ws.mark_last(s);
+    CK(cudaStreamSynchronize(s));
+    CK(cudaGetLastError());
+    f->stats = lphb_stats{};
+    f->stats.kernel_launches = 1;
+    f->stats.d2h_bytes = kCheckCounters * 8;
+    *r = lphb_check_report{};
+    r->kmers = h[kCheckKmers];
+    r->contigs = C.contigs;
+    r->dirty_contigs = h[kCheckDirty] + C.host_dirty;
+    r->out_of_range = h[kCheckOutOfRange];
+    r->duplicates = h[kCheckDuplicates];
+    r->missing = nkmers - h[kCheckHits];
+    r->stream_mismatches = h[kCheckMismatches];
+    r->first_out_of_range = h[kCheckFirstOutOfRange];
+    r->first_mismatch = h[kCheckFirstMismatch];
+    r->min_duplicate_code = h[kCheckMinDuplicate];
+    r->min_missing_code = h[kCheckMinMissing];
+    r->ok = r->out_of_range == 0 && r->duplicates == 0 && r->missing == 0 && r->stream_mismatches == 0;
     return LPHB_OK;
 }
 
@@ -1386,6 +1540,53 @@ int lphb_query_stream_runs(lphb_mphf* f, const char* bases, const uint64_t* offs
     sink.capacity = runs ? runs_capacity : 0;
     sink.n_runs = n_runs;
     return query_stream_host(f, bases, offsets, n_contigs, nullptr, 0, code_offsets, n_codes, sink);
+}
+
+int lphb_check_begin(lphb_mphf* f) {
+    if (!f) return fail(LPHB_E_ARG, "null handle");
+    return guarded([&]() -> int {
+        DeviceGuard g(f->device);
+        check_begin(f);
+        return LPHB_OK;
+    });
+}
+
+int lphb_check_batch(lphb_mphf* f, const char* bases, const uint64_t* offsets, uint64_t n_contigs) {
+    if (!f || !offsets) return fail(LPHB_E_ARG, "null argument");
+    if (!f->ws.check.open) return fail(LPHB_E_ARG, "no check session open: call lphb_check_begin first");
+    return guarded([&]() -> int {
+        DeviceGuard g(f->device);
+        std::vector<uint64_t> code_offsets(n_contigs + 1);
+        uint64_t n_codes = 0;
+        RunSink sink;
+        sink.check = true;
+        HostQuery q{f, bases, offsets, n_contigs, nullptr, 0, code_offsets.data(), &n_codes, sink};
+        const int rc = q.run();
+        if (rc != LPHB_OK) return rc;
+        f->ws.check.kmers += n_codes;
+        f->ws.check.contigs += n_contigs;
+        return LPHB_OK;
+    });
+}
+
+int lphb_check_batch_device(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
+                            uint64_t n_contigs, const uint64_t* d_stream_codes, void* stream) {
+    if (!f || !d_offsets || !h_offsets) return fail(LPHB_E_ARG, "null argument");
+    if (!f->ws.check.open) return fail(LPHB_E_ARG, "no check session open: call lphb_check_begin first");
+    return guarded([&]() -> int {
+        DeviceGuard g(f->device);
+        return check_batch_device(f, d_bases, d_offsets, h_offsets, n_contigs, d_stream_codes,
+                                  static_cast<cudaStream_t>(stream));
+    });
+}
+
+int lphb_check_end(lphb_mphf* f, lphb_check_report* report) {
+    if (!f || !report) return fail(LPHB_E_ARG, "null argument");
+    if (!f->ws.check.open) return fail(LPHB_E_ARG, "no check session open: call lphb_check_begin first");
+    return guarded([&]() -> int {
+        DeviceGuard g(f->device);
+        return check_end(f, report);
+    });
 }
 
 int lphb_lookup_kmers(lphb_mphf* f, const void* kmers, uint64_t n, uint64_t* codes) {
