@@ -225,7 +225,9 @@ typedef struct lphb_check_report {
     int32_t ok;                  /* 1 iff out_of_range, duplicates, missing and stream_mismatches are all 0  */
 } lphb_check_report;
 
-/* (Re)starts the handle's session: clears the bitmap and the counters.  Ordered against the handle's other calls. */
+/* (Re)starts the handle's session: clears the bitmap and the counters.  Ordered against the handle's other calls.
+ * The bitmap holds nkmers bits: LPHB_E_ARG for nkmers >= 2^64 - 32, LPHB_E_NOMEM (with the size) when the device
+ * cannot hold it; either way no session is open afterwards and the handle stays usable.                          */
 int lphb_check_begin(lphb_mphf* f);
 
 /* One batch of the session, HOST buffers (as lphb_query_stream takes them).  The bases go up in contig-aligned

@@ -968,13 +968,26 @@ int lookup_host(lphb_mphf* f, const void* kmers, uint64_t n, uint64_t* codes) {
 
 // ---- the index self-check: sessions ----------------------------------------------------------------------------
 
-// lphb_check_begin: the bitmap and the counters cleared on the handle's stream, ordered after the previous call
-void check_begin(lphb_mphf* f) {
+// lphb_check_begin: the bitmap and the counters cleared on the handle's stream, ordered after the previous call.
+// nkmers comes from the file header: k_check_windows needs nkmers < 2^64 - 32 (its match keys), and the bitmap's
+// size is computed without wrap-around and refused with LPHB_E_NOMEM when the device cannot hold it.
+int check_begin(lphb_mphf* f) {
     Workspace& ws = f->ws;
     Workspace::Check& C = ws.check;
     const cudaStream_t s = ws.stream;
-    const uint64_t bitmap_bytes = (f->img.nkmers + 31) / 32 * 4;
-    C.bitmap.reserve(bitmap_bytes + 8);
+    const uint64_t nkmers = f->img.nkmers;
+    C.open = false;  // a failed begin leaves no session, not the previous one over a freed bitmap
+    if (nkmers >= ~uint64_t(0) - 31)
+        return fail(LPHB_E_ARG, "check: nkmers = " + std::to_string(nkmers) + " in the header: at most 2^64 - 33 can be checked");
+    const uint64_t bitmap_bytes = (nkmers / 32 + (nkmers % 32 != 0)) * 4;
+    try {
+        C.bitmap.reserve(bitmap_bytes + 8);
+    } catch (CudaError const& e) {
+        if (e.e != cudaErrorMemoryAllocation) throw;
+        cudaGetLastError();
+        return fail(LPHB_E_NOMEM, "check: cannot allocate the " + std::to_string(bitmap_bytes + 8) +
+                                      "-byte bitmap of nkmers = " + std::to_string(nkmers) + " on the device");
+    }
     C.counters.reserve(kCheckCounters * 8);
     C.h_counters.reserve(kCheckCounters * 8);
     f->stats = lphb_stats{};
@@ -986,6 +999,7 @@ void check_begin(lphb_mphf* f) {
     CK(cudaGetLastError());
     C.kmers = C.contigs = C.host_dirty = 0;
     C.open = true;
+    return LPHB_OK;
 }
 
 // lphb_check_batch_device: asynchronous on s.  The code offsets of the batch go to ws.code_off, the streaming pass
@@ -1546,8 +1560,7 @@ int lphb_check_begin(lphb_mphf* f) {
     if (!f) return fail(LPHB_E_ARG, "null handle");
     return guarded([&]() -> int {
         DeviceGuard g(f->device);
-        check_begin(f);
-        return LPHB_OK;
+        return check_begin(f);
     });
 }
 

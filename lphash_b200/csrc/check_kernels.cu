@@ -79,7 +79,8 @@ __global__ void __launch_bounds__(kCheckThreads) k_check_windows(const __grid_co
                 first_mm = min(first_mm, ordinal);
             }
         }
-        // lanes without an in-range code take keys no in-range code can equal (codes < nkmers < 2^64 - 32)
+        // lanes without an in-range code take keys no in-range code can equal (codes < nkmers < 2^64 - 32, which
+        // lphb_check_begin enforces on the header's nkmers)
         const unsigned word_peers = __match_any_sync(kFull, in_range ? code >> 5 : ~uint64_t(lane));
         const unsigned code_peers = __match_any_sync(kFull, in_range ? code : ~uint64_t(lane));
         if (in_range) {

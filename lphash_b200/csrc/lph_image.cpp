@@ -279,7 +279,7 @@ ImageBuilder::BucketWriter ImageBuilder::begin_buckets(uint64_t T) {
     const char* fw = getenv("LPHB_FORCE_WIDE_BUCKETS");
     const bool force_wide = fw && fw[0] && fw[0] != '0';
     BucketWriter wtr;
-    wtr.wide = force_wide || img_.nkmers + 256 >= (1ull << 30);
+    wtr.wide = force_wide || img_.nkmers >= (1ull << 30) - 256;  // not nkmers + 256: the header's nkmers is unbounded
     const uint64_t off = (arena_.size() + 255) & ~uint64_t(255);
     arena_.resize(off + (wtr.wide ? (T + 4) * 8 : (T + 8) * 4), 0);
     wtr.p = arena_.data() + off;
@@ -616,7 +616,7 @@ ImagePlan ImageBuilder::plan(const uint8_t* data, uint64_t n, int kmer_bits, boo
     place_phf(P.minimizer_order, img.minimizer_order);
     place_phf(P.fallback, img.fallback);
     const char* fw = getenv("LPHB_FORCE_WIDE_BUCKETS");
-    const bool wide = (fw && fw[0] && fw[0] != '0') || img.nkmers + 256 >= (1ull << 30);
+    const bool wide = (fw && fw[0] && fw[0] != '0') || img.nkmers >= (1ull << 30) - 256;  // as begin_buckets
     const uint64_t T = D + P.minimizer_order.n_free;
     img.buckets.n = T;
     img.buckets.wide = wide ? 1 : 0;

@@ -62,13 +62,14 @@ def _dictionary(values) -> bytes:
     return _compact(ranks) + _compact(dict_)
 
 
-def _ef(values) -> bytes:
-    """pthash ef_sequence<false>::encode(begin, n), universe = the last value: {high bits, darray1, low bits}"""
+def _ef(values, universe: int | None = None) -> bytes:
+    """pthash ef_sequence<false>::encode(begin, n), universe = the last value unless given: {high bits, darray1, low
+    bits}"""
     v = np.ascontiguousarray(values, dtype=np.uint64)
     n = len(v)
     if n == 0:
         return invindex._u64(0) + invindex._vec([]) + invindex.darray1_image([]) + _compact([], 0)
-    u = int(v[-1])
+    u = int(v[-1]) if universe is None else universe
     l = (u // n).bit_length() - 1 if u // n else 0
     ones = (v >> np.uint64(l)) + np.arange(n, dtype=np.uint64)
     high = np.zeros(n + (u >> l) + 1, dtype=np.uint8)

@@ -50,9 +50,11 @@ def restate(o, contigs, stream=None):
     codes = np.concatenate(ns + [empty]).astype(np.uint64)
     oor = codes >= np.uint64(nkmers)
     uniq, cnt = np.unique(codes[~oor], return_counts=True)
-    hit = np.zeros(nkmers, dtype=bool)
-    hit[uniq.astype(np.int64)] = True
-    missing = np.flatnonzero(~hit)
+    # the missing codes without a bitmap of nkmers entries (indexes of 2^32 k-mers and more): uniq is sorted, so the
+    # smallest code never hit is the first i with uniq[i] != i, else len(uniq)
+    gaps = np.flatnonzero(uniq != np.arange(len(uniq), dtype=np.uint64))
+    n_missing = nkmers - len(uniq)
+    min_missing = int(gaps[0]) if len(gaps) else len(uniq) if n_missing else NONE
     mism, at = [], 0
     for c, v in zip(contigs, ns):
         if len(v) and is_clean(c):
@@ -60,11 +62,11 @@ def restate(o, contigs, stream=None):
             mism.extend((at + np.flatnonzero(st != v)).tolist())
         at += len(v)
     r = dict(kmers=len(codes), contigs=len(contigs), dirty_contigs=sum(not is_clean(c) for c in contigs),
-             out_of_range=int(oor.sum()), duplicates=int(cnt.sum() - len(uniq)), missing=len(missing),
+             out_of_range=int(oor.sum()), duplicates=int(cnt.sum() - len(uniq)), missing=n_missing,
              stream_mismatches=len(mism), first_out_of_range=int(np.argmax(oor)) if oor.any() else NONE,
              first_mismatch=min(mism) if mism else NONE,
              min_duplicate_code=int(uniq[cnt > 1][0]) if (cnt > 1).any() else NONE,
-             min_missing_code=int(missing[0]) if len(missing) else NONE)
+             min_missing_code=min_missing)
     r["ok"] = int(r["out_of_range"] == r["duplicates"] == r["missing"] == r["stream_mismatches"] == 0)
     return r
 
