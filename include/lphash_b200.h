@@ -306,6 +306,52 @@ int lphb_scan_classify(int device, uint32_t k, uint32_t m, uint64_t seed, const 
                        uint64_t triplets_capacity, uint64_t* n_triplets, uint64_t* ids,
                        uint64_t ids_capacity, uint64_t* n_ids, uint64_t* n_kmers);
 
+/* ---- build-p Parts 1 + 2 over a stream of batches: the build session ----------------------------
+ * lphb_scan_classify over an input of any size, fed batch by batch, with host memory bounded by one batch.
+ *   Result   triplets and ids are exactly what lphb_scan_classify returns on the concatenation of the session's
+ *            batches started at mm_count = 0, i.e. minimizer::classify (src/minimizer.cpp:5-50) over the whole
+ *            record stream: one triplet per distinct minimizer in ascending order, the ascending ids of every
+ *            occurrence of a minimizer seen more than once.  They do not depend on how the input is cut into
+ *            batches, nor on host versus device form.  A batch holds whole contigs; the per-batch limits of
+ *            lphb_scan_superkmers hold (fewer than 2^32 k-mers and 2^32 bases each), session totals are 64-bit.
+ *            Each batch is scanned and classified on the device as it comes; the session keeps one summary entry
+ *            per distinct minimizer of the batch (18 bytes) and the batch's locally colliding ids (8 bytes each),
+ *            and lphb_build_end merges them.  The merge runs in slices of at most LPHB_BUILD_SLICE distinct-minimizer
+ *            entries (environment variable; default 2^26, about 5 GB of workspace).
+ *   Capacity lphb_build_end with a buffer too small for the result (NULL with capacity 0 asks for the sizes) returns
+ *            LPHB_E_CAPACITY with *report filled in; the session stays open and keeps the merged result on the device,
+ *            so a second call with the reported sizes only copies it out.  A successful end fills *report, frees the
+ *            session's device memory and closes the session.
+ *   Errors   a batch or an end on a closed session: LPHB_E_ARG.  An end without a batch: an empty result.  A batch
+ *            that cannot get its device memory: LPHB_E_NOMEM with the size in the message; that batch is not added
+ *            and the session is unchanged and usable (nothing spills to host memory).  A batch that fails otherwise
+ *            is not added either.
+ *   Threads  calls on one session are serialised by the caller; a batch takes its turn on the device with the
+ *            other build-side calls (lphb_scan_*), an end does not.
+ * A batch shares the per-device scan workspace of lphb_scan_superkmers (freed by lphb_scan_release).          */
+typedef struct lphb_build lphb_build;
+typedef struct lphb_build_report {
+    uint64_t batches, contigs, kmers; /* kmers: as lphb_scan_classify's n_kmers, summed                    */
+    uint64_t mm_count;                /* m-mer ordinals consumed (the running mm_count)                     */
+    uint64_t records;                 /* super-k-mers of Part 1 (the CSV's total_minimizers)                */
+    uint64_t n_triplets, n_ids, colliding_minimizers; /* set by lphb_build_end; triplets of size 0 last    */
+    uint64_t device_bytes;            /* HBM the session holds (at an end: before it frees it)              */
+} lphb_build_report;
+/* k, m, seed as for lphb_scan_superkmers.  LPHB_E_ARG for k/m out of range before any CUDA call. */
+int lphb_build_begin(int device, uint32_t k, uint32_t m, uint64_t seed, lphb_build** out);
+/* One batch in HOST buffers (as lphb_scan_superkmers takes it).  Returns once the batch is in the session. */
+int lphb_build_batch(lphb_build* b, const char* bases, const uint64_t* offsets, uint64_t n_contigs);
+/* One batch in DEVICE buffers on the session's device (arguments as lphb_scan_superkmers_device).  SYNCHRONOUS:
+ * it first waits for `stream` (a cudaStream_t, NULL = default stream), on which the caller wrote the buffers, and
+ * returns once the caller's buffers may be reused.                                                               */
+int lphb_build_batch_device(lphb_build* b, const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
+                            uint64_t n_contigs, void* stream);
+/* triplets: packed 10-byte mm_triplet_t as lphb_classify writes them; capacities count triplets and ids. */
+int lphb_build_end(lphb_build* b, void* triplets, uint64_t triplets_capacity, uint64_t* ids, uint64_t ids_capacity,
+                   lphb_build_report* report);
+/* Frees the session, open or closed (NULL: nothing to do). */
+int lphb_build_free(lphb_build* b);
+
 /* ---- build-p Part 3: the inverted index --------------------------------------------------------
  * Replaces the loop that re-keys every triplet by minimizer_order(itself) and sorts the result
  * (src/partitioned_mphf.cpp:92-106) and mphf::build_inverted_index (src/partitioned_mphf.cpp:163-268):

@@ -305,6 +305,66 @@ private:
     }
 };
 
+// Parts 1 + 2 of build-p over an input fed batch by batch (lphb_build_*): end() gives what minimizer::classify gives
+// over the whole record stream (src/minimizer.cpp:5-50), however the input was cut.  Move-only; the destructor frees
+// the session.
+class build_session {
+public:
+    build_session(uint32_t k, uint32_t m, uint64_t seed, int device = 0) {
+        const int rc = lphb_build_begin(device, k, m, seed, &b_);
+        if (rc != LPHB_OK) detail::raise("lphash_b200::build_session", rc);
+    }
+    build_session(build_session&& o) noexcept : b_(std::exchange(o.b_, nullptr)) {}
+    build_session& operator=(build_session&& o) noexcept {
+        if (this != &o) {
+            lphb_build_free(b_);
+            b_ = std::exchange(o.b_, nullptr);
+        }
+        return *this;
+    }
+    build_session(build_session const&) = delete;
+    build_session& operator=(build_session const&) = delete;
+    ~build_session() { lphb_build_free(b_); }
+
+    // one batch of whole contigs in host memory
+    void batch(const char* bases, const uint64_t* offsets, uint64_t n_contigs) {
+        const int rc = lphb_build_batch(b_, bases, offsets, n_contigs);
+        if (rc != LPHB_OK) detail::raise("lphash_b200::build_session::batch", rc);
+    }
+    // one batch in device memory, written by the caller on `stream` (a cudaStream_t)
+    void batch_device(const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets, uint64_t n_contigs,
+                      void* stream = nullptr) {
+        const int rc = lphb_build_batch_device(b_, d_bases, d_offsets, h_offsets, n_contigs, stream);
+        if (rc != LPHB_OK) detail::raise("lphash_b200::build_session::batch_device", rc);
+    }
+    // merges the batches and closes the session: triplets in ascending minimizer order, ids ascending
+    lphb_build_report end(std::vector<mm_triplet_t>& triplets, std::vector<uint64_t>& ids) {
+        lphb_build_report r{};
+        int rc = lphb_build_end(b_, nullptr, 0, nullptr, 0, &r);
+        if (rc == LPHB_E_CAPACITY) {
+            triplets.resize(r.n_triplets);
+            ids.resize(r.n_ids);
+            rc = lphb_build_end(b_, triplets.data(), triplets.size(), ids.data(), ids.size(), &r);
+        } else if (rc == LPHB_OK) {
+            triplets.clear();
+            ids.clear();
+        }
+        if (rc != LPHB_OK) detail::raise("lphash_b200::build_session::end", rc);
+        return r;
+    }
+    // the same into caller-owned buffers: LPHB_OK (session closed) or LPHB_E_CAPACITY (r holds the sizes; the session
+    // stays open for another end)
+    int end(mm_triplet_t* triplets, uint64_t triplets_capacity, uint64_t* ids, uint64_t ids_capacity,
+            lphb_build_report& r) {
+        const int rc = lphb_build_end(b_, triplets, triplets_capacity, ids, ids_capacity, &r);
+        if (rc != LPHB_OK && rc != LPHB_E_CAPACITY) detail::raise("lphash_b200::build_session::end", rc);
+        return rc;
+    }
+
+private:
+    lphb_build* b_ = nullptr;
+};
+
 namespace minimizer {
 
 // minimizer::from_string (include/minimizer.hpp:11-170): appends one mm_record_t per super-k-mer

@@ -29,12 +29,19 @@ inline bool cpu_requested() {  // LPHASH_B200_CPU_BUILD=1 forwards the whole bui
     return e && e[0] == '1';
 }
 
+// text per batch of the streamed input; LPHASH_B200_BATCH_BYTES sets it (a test forces many batches with it)
+inline size_t batch_bytes() {
+    constexpr size_t kDefault = size_t(1) << 30;  // well under a batch's 2^32 bases
+    const char* e = std::getenv("LPHASH_B200_BATCH_BYTES");
+    const size_t v = e ? size_t(std::strtoull(e, nullptr, 10)) : 0;
+    return v ? v : kDefault;
+}
+
 struct Parts {
     int device = 0;
     uint32_t k = 0, m = 0;
     pthash::build_configuration cfg;
-    lphash_b200::fastx::Batch input;
-    uint64_t n_records = 0, nkmers = 0;
+    uint64_t n_records = 0, nkmers = 0;  // contigs of the input, k-mers of Part 1
     // one triplet per distinct minimizer, ascending; ids of every occurrence of a colliding minimizer, ascending
     // (uninitialised storage: at 2.5e9 k-mers a zero-filled worst-case vector would be tens of GB)
     struct Triplets {
@@ -53,7 +60,8 @@ struct Parts {
     } coll_ids;
     std::vector<unsigned char> minimizer_order, fallback;  // the two serialized single_phf objects
 
-    // Parts 1 and 2
+    // Parts 1 and 2: the file streamed through a build session, one batch of at most batch_bytes() of text at a time,
+    // so that host memory holds one batch and the result, never the whole input
     void scan_and_order(configuration const& config) {
         k = uint32_t(config.k);
         m = uint32_t(config.m);
@@ -66,51 +74,65 @@ struct Parts {
         cfg.ram = static_cast<uint64_t>(config.max_memory) * essentials::GB;
         cfg.tmp_dir = config.tmp_dirname;
         if (config.verbose) std::cerr << "Part 1: file reading and info gathering\n";
-        lphash_b200::fastx::read_file(config.input_filename.c_str(), input);
-        n_records = input.n_records();
+        lphash_b200::build_session session(k, m, config.mm_seed, device);
         uint64_t max_kmers = 0;
-        for (uint64_t c = 0; c < n_records; ++c) {
-            const uint64_t len = input.offsets[c + 1] - input.offsets[c];
-            if (len >= k) max_kmers += len - k + 1;
-        }
+        n_records = lphash_b200::fastx::stream_file(config.input_filename, batch_bytes(), [&](lphash_b200::fastx::Batch const& b) {
+            for (uint64_t c = 0; c < b.n_records(); ++c) {
+                const uint64_t len = b.offsets[c + 1] - b.offsets[c];
+                if (len >= k) max_kmers += len - k + 1;
+            }
+            session.batch(b.bases.data(), b.offsets.data(), b.n_records());
+        });
         // super-k-mers are about 2 / (k - m + 2) of the k-mers; a third is room enough for every window of 5 or
-        // more (an input that needs more - LPHB_E_CAPACITY reports the counts - is scanned again with exactly that)
-        uint64_t cap = max_kmers / 3 + 4096, n_triplets = 0, n_ids = 0, mm_count = 0;
+        // more (an input that needs more - LPHB_E_CAPACITY reports the counts - gets exactly that on the second end)
+        uint64_t cap = max_kmers / 3 + 4096;
         if (const char* e = std::getenv("LPHASH_B200_FIRST_CAP")) cap = std::strtoull(e, nullptr, 10) + 1;  // test hook
+        lphb_build_report report{};
         for (int attempt = 0;; ++attempt) {
             triplets.p.reset(new lphash_b200::mm_triplet_t[cap]);
             coll_ids.p.reset(new uint64_t[cap]);
-            mm_count = 0;
-            const int rc = lphb_scan_classify(device, k, m, config.mm_seed, input.bases.data(), input.offsets.data(), n_records,
-                                              &mm_count, triplets.p.get(), cap, &n_triplets, coll_ids.p.get(), cap, &n_ids, &nkmers);
+            const int rc = session.end(triplets.p.get(), cap, coll_ids.p.get(), cap, report);
             if (rc == LPHB_E_CAPACITY && attempt == 0) {
-                cap = std::max(n_triplets, n_ids) + 1;
+                cap = std::max(report.n_triplets, report.n_ids) + 1;
                 continue;
             }
             check(rc);
             break;
         }
-        triplets.n = n_triplets;
-        coll_ids.n = n_ids;
+        triplets.n = report.n_triplets;
+        coll_ids.n = report.n_ids;
+        nkmers = report.kmers;
         if (config.verbose) std::cerr << "Part 2: build MPHF\n";
-        std::vector<uint64_t> keys(n_triplets);
-        for (uint64_t i = 0; i < n_triplets; ++i) keys[i] = triplets.p[i].itself;
+        std::vector<uint64_t> keys(triplets.n);
+        for (uint64_t i = 0; i < triplets.n; ++i) keys[i] = triplets.p[i].itself;
         pthash_minimizers_mphf_t f;
-        f.build_in_external_memory(keys.begin(), n_triplets, cfg);
+        f.build_in_external_memory(keys.begin(), triplets.n, cfg);
         lphash_b200::memory_saver saver;
         saver.visit(f);
         minimizer_order.swap(saver.bytes);
     }
 
-    // Part 4
+    // Part 4: a second pass over the file in the same batches; each batch gets the colliding ids of its m-mer range
     void fallback_function(configuration const& config) {
         if (config.verbose) std::cerr << "Part 4: build fallback MPHF\n";
-        uint64_t n_coll_kmers = 0, mm_again = 0;
+        uint64_t n_coll_kmers = 0, mm_count = 0;
         const uint64_t kcap = coll_ids.size() * (uint64_t(k) - m + 1) + 1;  // a super-k-mer holds at most k - m + 1 k-mers
         std::unique_ptr<kmer_t[]> kmers(new kmer_t[kcap]);
-        check(lphb_colliding_kmers(device, k, m, config.mm_seed, input.bases.data(), input.offsets.data(), n_records, &mm_again,
-                                   coll_ids.data(), coll_ids.size(), int(sizeof(kmer_t) * 8), kmers.get(), kcap,
-                                   &n_coll_kmers));
+        const uint64_t* ids_end = coll_ids.data() + coll_ids.size();
+        lphash_b200::fastx::stream_file(config.input_filename, batch_bytes(), [&](lphash_b200::fastx::Batch const& b) {
+            uint64_t mm_bound = mm_count;  // the batch's ordinals end at or before this (non-ACGT bytes only remove m-mers)
+            for (uint64_t c = 0; c < b.n_records(); ++c) {
+                const uint64_t len = b.offsets[c + 1] - b.offsets[c];
+                if (len >= m) mm_bound += len - m + 1;
+            }
+            const uint64_t* first = std::lower_bound(coll_ids.data(), ids_end, mm_count);
+            const uint64_t* last = std::lower_bound(first, ids_end, mm_bound);
+            uint64_t n = 0;
+            check(lphb_colliding_kmers(device, k, m, config.mm_seed, b.bases.data(), b.offsets.data(), b.n_records(), &mm_count,
+                                       first, uint64_t(last - first), int(sizeof(kmer_t) * 8), kmers.get() + n_coll_kmers,
+                                       kcap - n_coll_kmers, &n));
+            n_coll_kmers += n;
+        });
         pthash_fallback_mphf_t f;
         f.build_in_external_memory(kmers.get(), n_coll_kmers, cfg);
         lphash_b200::memory_saver saver;

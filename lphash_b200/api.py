@@ -78,6 +78,16 @@ class CheckReport(C.Structure):
         return {name: getattr(self, name) for name, _ in self._fields_}
 
 
+class BuildReport(C.Structure):
+    """lphb_build_report: totals of a build session (n_triplets, n_ids, colliding_minimizers are set by its end)"""
+    _fields_ = [("batches", C.c_uint64), ("contigs", C.c_uint64), ("kmers", C.c_uint64), ("mm_count", C.c_uint64),
+                ("records", C.c_uint64), ("n_triplets", C.c_uint64), ("n_ids", C.c_uint64),
+                ("colliding_minimizers", C.c_uint64), ("device_bytes", C.c_uint64)]
+
+    def as_dict(self) -> dict:
+        return {name: getattr(self, name) for name, _ in self._fields_}
+
+
 # every symbol include/lphash_b200.h declares (tests check the library exports all of them)
 EXPORTS = ["lphb_last_error", "lphb_version", "lphb_device_count", "lphb_mphf_load_file",
            "lphb_mphf_load_memory", "lphb_mphf_free", "lphb_mphf_info", "lphb_query_stream",
@@ -89,7 +99,8 @@ EXPORTS = ["lphb_last_error", "lphb_version", "lphb_device_count", "lphb_mphf_lo
            "lphb_build_inverted_index", "lphb_lph_assemble", "lphb_lph_sections", "lphb_build_inverted_index_alt",
            "lphb_lph_assemble_alt", "lphb_mphf_device_image", "lphb_lookup_kmers", "lphb_lookup_kmers_device",
            "lphb_query_stream_exact_device", "lphb_query_nonstreaming_device", "lphb_check_begin", "lphb_check_batch",
-           "lphb_check_batch_device", "lphb_check_end"]
+           "lphb_check_batch_device", "lphb_check_end", "lphb_build_begin", "lphb_build_batch",
+           "lphb_build_batch_device", "lphb_build_end", "lphb_build_free"]
 
 _lib = None
 
@@ -152,6 +163,11 @@ def lib() -> C.CDLL:
     L.lphb_lph_assemble_alt.argtypes = [C.c_uint32, C.c_uint32, u64, u64, u64, C.POINTER(InvertedIndexAlt), p, u64, p, u64,
                                         p, u64, p, u64, C.POINTER(u64)]
     L.lphb_host_free.argtypes = [p]
+    L.lphb_build_begin.argtypes = [i32, C.c_uint32, C.c_uint32, u64, C.POINTER(p)]
+    L.lphb_build_batch.argtypes = [p, p, p, u64]
+    L.lphb_build_batch_device.argtypes = [p, p, p, p, u64, p]
+    L.lphb_build_end.argtypes = [p, p, u64, p, u64, C.POINTER(BuildReport)]
+    L.lphb_build_free.argtypes = [p]
     for name in EXPORTS:
         if getattr(L, name).restype is C.c_int:
             pass
@@ -465,6 +481,67 @@ def scan_classify(bases, offsets, k: int, m: int, seed: int = 42, mm_count: int 
                                     trip.ctypes.data, cap, C.byref(nt), ids.ctypes.data, cap, C.byref(ni),
                                     C.byref(nk)))
     return trip[: nt.value].copy(), ids[: ni.value].copy(), nk.value, mm.value
+
+
+class BuildSession:
+    """lphb_build_*: Parts 1 + 2 of build-p over an input fed batch by batch.  end() returns what scan_classify returns
+    on the concatenation of the batches (mm_count = 0): (triplets, colliding ids, BuildReport).
+
+        with BuildSession(k, m, seed) as s:
+            for bases, offsets in batches:
+                s.batch(bases, offsets)
+            triplets, ids, report = s.end()
+    """
+
+    def __init__(self, k: int, m: int, seed: int = 42, device: int = 0):
+        self.k, self.m, self.seed, self.device = k, m, seed, device
+        h = C.c_void_p()
+        _check(lib().lphb_build_begin(device, k, m, seed, C.byref(h)))
+        self._h = h
+
+    def batch(self, bases, offsets) -> None:
+        """one batch of whole contigs in host arrays (as scan_classify takes them)"""
+        bases, offsets = _as_batch(bases, offsets)
+        _check(lib().lphb_build_batch(self._h, bases.ctypes.data, offsets.ctypes.data, len(offsets) - 1))
+
+    def batch_device(self, d_bases: int, d_offsets: int, h_offsets, stream: int = 0) -> None:
+        """one batch in device buffers: raw pointers (ints), e.g. tensor.data_ptr(), d_bases indexed by the offsets,
+        h_offsets their host copy; waits for `stream` (a cudaStream_t) first.  Synchronous."""
+        h_offsets = np.ascontiguousarray(h_offsets, dtype=np.uint64)
+        _check(lib().lphb_build_batch_device(self._h, d_bases, d_offsets, h_offsets.ctypes.data, len(h_offsets) - 1,
+                                             stream))
+
+    def end(self):
+        """merges the batches and closes the session: (triplets[TRIPLET_DTYPE] ascending, ids ascending, BuildReport).
+        The first call asks for the sizes, the second copies the result out."""
+        L = lib()
+        r = BuildReport()
+        rc = L.lphb_build_end(self._h, None, 0, None, 0, C.byref(r))
+        if rc == OK:
+            return np.empty(0, dtype=TRIPLET_DTYPE), np.empty(0, dtype=np.uint64), r
+        if rc != E_CAPACITY:
+            _check(rc)
+        trip = np.empty(r.n_triplets, dtype=TRIPLET_DTYPE)
+        ids = np.empty(r.n_ids, dtype=np.uint64)
+        _check(L.lphb_build_end(self._h, trip.ctypes.data, len(trip), ids.ctypes.data, len(ids), C.byref(r)))
+        return trip, ids, r
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h.value:
+            lib().lphb_build_free(self._h)
+            self._h = C.c_void_p()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 def colliding_kmers(bases, offsets, k: int, m: int, ids, seed: int = 42, kmer_bits: int = 64,

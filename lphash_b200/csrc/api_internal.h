@@ -29,6 +29,10 @@ struct CudaError {
         cudaError_t e__ = (expr);                             \
         if (e__ != cudaSuccess) throw ::lphb::CudaError{e__, #expr}; \
     } while (0)
+// a device allocation that failed for want of memory (a CudaError to every caller that does not ask for the size)
+struct DeviceOom : CudaError {
+    uint64_t bytes;
+};
 
 // The owners below free what they hold when they go out of scope, ignoring errors; the device that owns the
 // resource must be current then.
@@ -48,7 +52,12 @@ struct DevBuf {
         p = nullptr;
         cap = 0;
         uint64_t want = bytes + bytes / 8 + 256;
-        CK(cudaMalloc(&p, want));
+        const cudaError_t e = cudaMalloc(&p, want);
+        if (e == cudaErrorMemoryAllocation) {
+            p = nullptr;
+            throw DeviceOom{{e, "cudaMalloc(&p, want)"}, want};
+        }
+        CK(e);
         cap = want;
     }
     template <class T>

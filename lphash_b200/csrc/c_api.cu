@@ -18,6 +18,7 @@
 
 #include "../../include/lphash_b200.h"
 #include "api_internal.h"
+#include "build_session.h"
 #include "check_kernels.cuh"
 #include "image_decode.cuh"
 #include "lph_image.h"
@@ -1364,6 +1365,18 @@ int classify_device(const uint8_t* d_rec, uint64_t n, void* triplets, uint64_t t
     return LPHB_OK;
 }
 
+// Adds the batch the scan session holds (records still on the device) to a build session.
+int build_take_scan(lphb_build* b, ScanSession& S, uint64_t n_contigs, uint64_t mm_out) {
+    build_add_batch(b, S.records.as<uint8_t>(), S.n_records, S.s);
+    lphb_build_report& t = b->totals;
+    t.batches += 1;
+    t.contigs += n_contigs;
+    t.kmers += S.n_kmers;
+    t.records += S.n_records;
+    t.mm_count = mm_out;
+    return LPHB_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1799,6 +1812,41 @@ int lphb_scan_classify(int device, uint32_t k, uint32_t m, uint64_t seed, const 
         }
         *mm_count = mm_out;
         return LPHB_OK;
+    });
+}
+
+int lphb_build_batch(lphb_build* b, const char* bases, const uint64_t* offsets, uint64_t n_contigs) {
+    if (!b || !offsets) return fail(LPHB_E_ARG, "null argument");
+    if (!b->dev) return fail(LPHB_E_ARG, "the build session has ended");
+    return guarded_nomem([&]() -> int {
+        DeviceGuard g(b->device);
+        std::lock_guard<std::mutex> lock(device_sessions(b->device).mu);
+        ScanSession& S = scan_session(b->device);
+        uint64_t mm_out = b->totals.mm_count;
+        int rc = run_scan(S, b->k, b->m, b->seed, bases, offsets, n_contigs, b->totals.mm_count, &mm_out);
+        if (rc != LPHB_OK) return rc;
+        return build_take_scan(b, S, n_contigs, mm_out);
+    });
+}
+
+int lphb_build_batch_device(lphb_build* b, const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
+                            uint64_t n_contigs, void* stream) {
+    if (!b || !d_offsets || !h_offsets) return fail(LPHB_E_ARG, "null argument");
+    if (!b->dev) return fail(LPHB_E_ARG, "the build session has ended");
+    return guarded_nomem([&]() -> int {
+        DeviceGuard g(b->device);
+        std::lock_guard<std::mutex> lock(device_sessions(b->device).mu);
+        ScanSession& S = scan_session(b->device);
+        const ContigCounts n = begin_scan(S, b->k, b->m, h_offsets, n_contigs);
+        uint64_t mm_out = b->totals.mm_count + n.mmers;
+        if (n_contigs && n.mmers) {
+            if (!d_bases) return fail(LPHB_E_ARG, "d_bases is null");
+            CK(cudaStreamSynchronize(static_cast<cudaStream_t>(stream)));  // the caller wrote its buffers on `stream`
+            int rc = run_scan_device(S, b->k, b->m, b->seed, d_bases, d_offsets, h_offsets, n_contigs, b->totals.mm_count,
+                                     &mm_out);
+            if (rc != LPHB_OK) return rc;
+        }
+        return build_take_scan(b, S, n_contigs, mm_out);
     });
 }
 

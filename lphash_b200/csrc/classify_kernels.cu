@@ -74,6 +74,14 @@ __global__ void k_classify_emit(const uint8_t* records, const uint64_t* key, con
     }
 }
 
+__global__ void k_group_singleton_ids(const uint8_t* records, const uint32_t* idx, const uint8_t* flags,
+                                      const uint32_t* gslot, uint64_t n, uint64_t* sid) {
+    for (uint64_t i = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; i < n; i += uint64_t(gridDim.x) * blockDim.x) {
+        const uint8_t f = flags[i];
+        if (f & 1u) sid[gslot[i]] = (f & 2u) ? ~0ull : rec_u64(records + 18ull * idx[i] + 8);
+    }
+}
+
 }  // namespace
 
 uint64_t classify_tmp_bytes(uint64_t n) {
@@ -117,6 +125,11 @@ void launch_classify_emit(const uint8_t* records, const uint64_t* key_sorted, co
         size_t bytes = tmp_bytes;
         cub::DeviceRadixSort::SortKeys(d_tmp, bytes, ids_unsorted, ids_sorted, n_ids, 0, 64, stream);
     }
+}
+
+void launch_classify_singleton_ids(const uint8_t* records, const uint32_t* idx_sorted, const uint8_t* flags,
+                                   const uint32_t* gslot, uint64_t n, uint64_t* sid, cudaStream_t stream) {
+    if (n) k_group_singleton_ids<<<cgrid(n), 256, 0, stream>>>(records, idx_sorted, flags, gslot, n, sid);
 }
 
 }  // namespace lphb

@@ -67,5 +67,8 @@ void launch_classify_emit(const uint8_t* records, const uint64_t* key_sorted, co
                           const uint8_t* flags, const uint32_t* gslot, const uint32_t* cslot, uint64_t n,
                           uint8_t* triplets, uint64_t* ids_unsorted, uint64_t* ids_sorted, uint64_t n_ids,
                           void* d_tmp, uint64_t tmp_bytes, cudaStream_t stream);
+// After step 1: sid[g] = the id of group g's record when the group holds one record, UINT64_MAX otherwise.
+void launch_classify_singleton_ids(const uint8_t* records, const uint32_t* idx_sorted, const uint8_t* flags,
+                                   const uint32_t* gslot, uint64_t n, uint64_t* sid, cudaStream_t stream);
 
 }  // namespace lphb
