@@ -1,8 +1,10 @@
-// Shared by the translation units behind the C ABI (c_api.cu, build_api.cu): error slot, CUDA error
-// propagation, the exception fence every entry point runs inside, owners of device resources.
+// Shared by the translation units behind the C ABI (c_api.cu, scan_api.cu, build_session.cu, build_api.cu): error
+// slot, CUDA error propagation, the exception fence every entry point runs inside, owners of device resources, the
+// layout of a batch of contigs.
 #pragma once
 #include <cuda_runtime.h>
 
+#include <cstdint>
 #include <new>
 #include <stdexcept>
 #include <string>
@@ -123,6 +125,31 @@ struct DeviceGuard {
         if (prev >= 0) cudaSetDevice(prev);
     }
 };
+
+// Layout of a batch of contigs (host offsets): max(0, L-k+1) k-mers per contig and, with m, max(0, L-m+1) m-mers.
+// With code_offsets, writes where each contig's codes start (n_contigs + 1 entries).  Offsets that decrease are
+// an argument error (thrown; guarded() reports it as LPHB_E_ARG).
+struct ContigCounts {
+    uint64_t kmers = 0, mmers = 0;
+};
+inline ContigCounts contig_layout(const uint64_t* offsets, uint64_t n_contigs, uint32_t k, uint32_t m = 0,
+                                  uint64_t* code_offsets = nullptr) {
+    ContigCounts n;
+    for (uint64_t c = 0; c < n_contigs; ++c) {
+        if (offsets[c + 1] < offsets[c]) throw std::invalid_argument("offsets must be non-decreasing");
+        const uint64_t len = offsets[c + 1] - offsets[c];
+        if (code_offsets) code_offsets[c] = n.kmers;
+        n.kmers += len >= k ? len - k + 1 : 0;
+        if (m) n.mmers += len >= m ? len - m + 1 : 0;
+    }
+    if (code_offsets) code_offsets[n_contigs] = n.kmers;
+    return n;
+}
+
+// The (k, m) the build side takes (the scan and build sessions): the error text when (k, m) is outside, else null.
+inline const char* scan_km_error(uint32_t k, uint32_t m) {
+    return m == 0 || m > 31 || k < m || k > 63 ? "need 1 <= m <= 31, m <= k <= 63" : nullptr;
+}
 
 // nothing may cross the C boundary as an exception
 template <class F>

@@ -101,40 +101,46 @@ uint64_t slice_entries() {
     return v ? v : kSliceEntries;
 }
 
-// Step 1 of classify on n records in the session's workspace; counts[0] = groups, counts[1] = members of groups of
-// several.  Returns the workspace size step 2 takes.
-uint64_t classify_groups(BuildDevice& D, const uint8_t* rec, uint64_t n, int key_bits, cudaStream_t s,
-                         uint64_t counts[2]) {
-    D.key.reserve(n * 8);
-    D.key2.reserve(n * 8);
-    D.idx.reserve(n * 4);
-    D.idx2.reserve(n * 4);
-    D.flags.reserve(n + 8);
-    D.gslot.reserve(n * 4);
-    D.cslot.reserve(n * 4);
-    D.counts.reserve(64);
-    const uint64_t tb = classify_tmp_bytes(n);
-    D.tmp.reserve(tb);
-    launch_classify_groups(rec, n, D.key.as<uint64_t>(), D.key2.as<uint64_t>(), D.idx.as<uint32_t>(), D.idx2.as<uint32_t>(),
-                           D.flags.as<uint8_t>(), D.gslot.as<uint32_t>(), D.cslot.as<uint32_t>(),
-                           D.counts.as<unsigned long long>(), D.tmp.p, tb, key_bits, s);
-    unsigned long long h[2] = {0, 0};
-    CK(cudaMemcpyAsync(h, D.counts.p, sizeof(h), cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    CK(cudaGetLastError());
-    counts[0] = h[0];
-    counts[1] = h[1];
-    return tb;
-}
-
 }  // namespace
 
-uint64_t BuildDevice::bytes() const {
+void Classify::group(const uint8_t* rec, uint64_t n, int key_bits, cudaStream_t s) {
+    key.reserve(n * 8);
+    key2.reserve(n * 8);
+    idx.reserve(n * 4);
+    idx2.reserve(n * 4);
+    flags.reserve(n + 8);
+    gslot.reserve(n * 4);
+    cslot.reserve(n * 4);
+    counts.reserve(64);
+    tmp_bytes = classify_tmp_bytes(n);
+    tmp.reserve(tmp_bytes);
+    launch_classify_groups(rec, n, key.as<uint64_t>(), key2.as<uint64_t>(), idx.as<uint32_t>(), idx2.as<uint32_t>(),
+                           flags.as<uint8_t>(), gslot.as<uint32_t>(), cslot.as<uint32_t>(), counts.as<unsigned long long>(),
+                           tmp.p, tmp_bytes, key_bits, s);
+    unsigned long long h[2] = {0, 0};
+    CK(cudaMemcpyAsync(h, counts.p, sizeof(h), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    CK(cudaGetLastError());
+    groups = h[0];
+    members = h[1];
+}
+
+void Classify::emit(const uint8_t* rec, uint64_t n, uint8_t* triplets, uint64_t* ids, cudaStream_t s) {
+    idu.reserve(members * 8);
+    launch_classify_emit(rec, key2.as<uint64_t>(), idx2.as<uint32_t>(), flags.as<uint8_t>(), gslot.as<uint32_t>(),
+                         cslot.as<uint32_t>(), n, triplets, idu.as<uint64_t>(), ids, ids ? members : 0, tmp.p, tmp_bytes, s);
+}
+
+uint64_t Classify::bytes() const {
     uint64_t n = 0;
+    for (const DevBuf* d : {&key, &key2, &idx, &idx2, &flags, &gslot, &cslot, &counts, &tmp, &idu}) n += d->cap;
+    return n;
+}
+
+uint64_t BuildDevice::bytes() const {
+    uint64_t n = cls.bytes();
     for (auto const& b : batches) n += b.trip.cap + b.sid.cap + b.lids.cap;
-    for (const DevBuf* d : {&key, &key2, &idx, &idx2, &flags, &gslot, &cslot, &counts, &tmp, &idu, &rec, &bounds, &desc,
-                            &marks, &idw, &nsel, &res_trip, &res_ids})
-        n += d->cap;
+    for (const DevBuf* d : {&rec, &bounds, &desc, &marks, &idw, &nsel, &res_trip, &res_ids}) n += d->cap;
     return n;
 }
 
@@ -142,19 +148,15 @@ void build_add_batch(lphb_build* b, const uint8_t* rec, uint64_t n, cudaStream_t
     BuildDevice& D = *b->dev;
     BatchSummary sum;
     if (n) {
-        uint64_t c[2];
-        const uint64_t tb = classify_groups(D, rec, n, int(2 * b->m), s, c);  // a minimizer is 2m bits
-        sum.n_groups = c[0];
-        sum.n_lids = c[1];
-        sum.trip.reserve(c[0] * 10);
-        sum.sid.reserve(c[0] * 8);
-        sum.lids.reserve(c[1] * 8);
-        D.idu.reserve(c[1] * 8);
-        launch_classify_emit(rec, D.key2.as<uint64_t>(), D.idx2.as<uint32_t>(), D.flags.as<uint8_t>(), D.gslot.as<uint32_t>(),
-                             D.cslot.as<uint32_t>(), n, sum.trip.as<uint8_t>(), D.idu.as<uint64_t>(), sum.lids.as<uint64_t>(),
-                             c[1], D.tmp.p, tb, s);
-        launch_classify_singleton_ids(rec, D.idx2.as<uint32_t>(), D.flags.as<uint8_t>(), D.gslot.as<uint32_t>(), n,
-                                      sum.sid.as<uint64_t>(), s);
+        D.cls.group(rec, n, int(2 * b->m), s);  // a minimizer is 2m bits
+        sum.n_groups = D.cls.groups;
+        sum.n_lids = D.cls.members;
+        sum.trip.reserve(sum.n_groups * 10);
+        sum.sid.reserve(sum.n_groups * 8);
+        sum.lids.reserve(sum.n_lids * 8);
+        D.cls.emit(rec, n, sum.trip.as<uint8_t>(), sum.lids.as<uint64_t>(), s);
+        launch_classify_singleton_ids(rec, D.cls.idx2.as<uint32_t>(), D.cls.flags.as<uint8_t>(), D.cls.gslot.as<uint32_t>(),
+                                      n, sum.sid.as<uint64_t>(), s);
         CK(cudaStreamSynchronize(s));
         CK(cudaGetLastError());
     }
@@ -223,15 +225,11 @@ void build_merge(lphb_build* b) {
                                                    D.rec.as<uint8_t>() + 18 * at);
             at += cnt;
         }
-        uint64_t c[2];
-        const uint64_t tb = classify_groups(D, D.rec.as<uint8_t>(), n, key_bits, s, c);
-        D.idu.reserve(c[1] * 8);
-        // n_ids = 0: the origins are only marked, not sorted
-        launch_classify_emit(D.rec.as<uint8_t>(), D.key2.as<uint64_t>(), D.idx2.as<uint32_t>(), D.flags.as<uint8_t>(),
-                             D.gslot.as<uint32_t>(), D.cslot.as<uint32_t>(), n, D.res_trip.as<uint8_t>() + 10 * T,
-                             D.idu.as<uint64_t>(), nullptr, 0, D.tmp.p, tb, s);
-        if (c[1]) k_mark<<<grid(c[1]), 256, 0, s>>>(D.idu.as<uint64_t>(), c[1], D.marks.as<uint8_t>());
-        T += c[0];
+        Classify& C = D.cls;
+        C.group(D.rec.as<uint8_t>(), n, key_bits, s);
+        C.emit(D.rec.as<uint8_t>(), n, D.res_trip.as<uint8_t>() + 10 * T, nullptr, s);  // the origins are only marked
+        if (C.members) k_mark<<<grid(C.members), 256, 0, s>>>(C.idu.as<uint64_t>(), C.members, D.marks.as<uint8_t>());
+        T += C.groups;
     }
     D.nsel.reserve(64);
     auto* d_cnt = D.nsel.as<unsigned long long>();
@@ -243,7 +241,7 @@ void build_merge(lphb_build* b) {
     CK(cub::DeviceSelect::Flagged(nullptr, t_sel, (const uint64_t*)nullptr, (const uint8_t*)nullptr, (uint64_t*)nullptr,
                                   (long long*)nullptr, (int64_t)ids_batch_max));
     CK(cub::DeviceRadixSort::SortKeys(nullptr, t_sort, (const uint64_t*)nullptr, (uint64_t*)nullptr, ids_batch_max));
-    D.tmp.reserve(std::max<uint64_t>(t_sel, t_sort));
+    D.cls.tmp.reserve(std::max<uint64_t>(t_sel, t_sort));
     D.idw.reserve(ids_batch_max * 8);
     D.res_ids.reserve(ids_bound * 8);
     auto* d_sel = reinterpret_cast<long long*>(d_cnt + 1);
@@ -253,16 +251,16 @@ void build_merge(lphb_build* b) {
         if (!B.n_groups) continue;
         if (B.n_lids)
             CK(cudaMemcpyAsync(D.idw.p, B.lids.p, B.n_lids * 8, cudaMemcpyDeviceToDevice, s));
-        size_t bytes = D.tmp.cap;
-        CK(cub::DeviceSelect::Flagged(D.tmp.p, bytes, B.sid.as<uint64_t>(), D.marks.as<uint8_t>() + base[j],
+        size_t bytes = D.cls.tmp.cap;
+        CK(cub::DeviceSelect::Flagged(D.cls.tmp.p, bytes, B.sid.as<uint64_t>(), D.marks.as<uint8_t>() + base[j],
                                       D.idw.as<uint64_t>() + B.n_lids, d_sel, (int64_t)B.n_groups, s));
         long long sel = 0;
         CK(cudaMemcpyAsync(&sel, d_sel, 8, cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
         const uint64_t n = B.n_lids + uint64_t(sel);
         if (n) {
-            bytes = D.tmp.cap;
-            CK(cub::DeviceRadixSort::SortKeys(D.tmp.p, bytes, D.idw.as<uint64_t>(), D.res_ids.as<uint64_t>() + I, n, 0, 64, s));
+            bytes = D.cls.tmp.cap;
+            CK(cub::DeviceRadixSort::SortKeys(D.cls.tmp.p, bytes, D.idw.as<uint64_t>(), D.res_ids.as<uint64_t>() + I, n, 0, 64, s));
         }
         I += n;
     }
@@ -287,7 +285,7 @@ extern "C" {
 int lphb_build_begin(int device, uint32_t k, uint32_t m, uint64_t seed, lphb_build** out) {
     if (!out) return fail(LPHB_E_ARG, "null argument");
     *out = nullptr;
-    if (m == 0 || m > 31 || k < m || k > 63) return fail(LPHB_E_ARG, "need 1 <= m <= 31, m <= k <= 63");
+    if (const char* e = scan_km_error(k, m)) return fail(LPHB_E_ARG, e);
     if (device < 0 || device >= 64) return fail(LPHB_E_ARG, "device index out of range");
     return guarded([&]() -> int {
         DeviceGuard g(device);

@@ -1,6 +1,7 @@
 // The state behind lphb_build (include/lphash_b200.h, build session): the classify of each batch reduced to one
 // entry per distinct minimizer, and the merge of those summaries into the session's triplets and ids
-// (build_session.cu).  The batch entry points live in c_api.cu, next to the scan they run first.
+// (build_session.cu).  The batch entry points live in scan_api.cu, next to the scan they run first.  Also the
+// classify workspace, which lphb_classify and lphb_scan_classify use too.
 #pragma once
 #include <memory>
 #include <string>
@@ -9,6 +10,18 @@
 #include "api_internal.h"
 
 namespace lphb {
+
+// Workspace of minimizer::classify (classify_kernels.cu) over n records on the device.
+struct Classify {
+    DevBuf key, key2, idx, idx2, flags, gslot, cslot, counts, tmp, idu;
+    uint64_t tmp_bytes = 0;           // what step 2 may use of tmp
+    uint64_t groups = 0, members = 0;  // of step 1: groups (triplets), members of groups of several (ids)
+    // Step 1 (sort by minimizer, group) on stream s, its counts read back; returns after the device finished.
+    void group(const uint8_t* rec, uint64_t n, int key_bits, cudaStream_t s);
+    // Step 2 on s: the groups' triplets; the members' ids unsorted in idu and, unless ids is null, sorted into ids.
+    void emit(const uint8_t* rec, uint64_t n, uint8_t* triplets, uint64_t* ids, cudaStream_t s);
+    uint64_t bytes() const;
+};
 
 // One batch after its classify: G entries sorted by minimizer, L local collision ids.
 struct BatchSummary {
@@ -21,9 +34,9 @@ struct BatchSummary {
 // Everything the session holds on the device; dropped as a whole when the session closes.
 struct BuildDevice {
     std::vector<BatchSummary> batches;
-    DevBuf key, key2, idx, idx2, flags, gslot, cslot, counts, tmp, idu;  // classify of one batch or one slice
-    DevBuf rec, bounds, desc, marks, idw, nsel, res_trip, res_ids;      // the merge
-    Stream s;                                                            // the merge's stream
+    Classify cls;                                                   // classify of one batch or one slice
+    DevBuf rec, bounds, desc, marks, idw, nsel, res_trip, res_ids;  // the merge
+    Stream s;                                                       // the merge's stream
     bool merged = false;
     uint64_t n_triplets = 0, n_ids = 0, colliding = 0;
     uint64_t bytes() const;

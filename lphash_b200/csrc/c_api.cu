@@ -1,6 +1,6 @@
-// C ABI of lphash_b200 (include/lphash_b200.h): handle management, host<->device staging and
-// kernel sequencing.  No CPU implementation of the path exists here: without a CUDA device every
-// computing entry point fails with LPHB_E_CUDA.
+// C ABI of lphash_b200 (include/lphash_b200.h), the lphb_mphf handle: loading, host<->device staging and kernel
+// sequencing of its queries, lookups and self-checks.  No CPU implementation of the path exists here: without a
+// CUDA device every computing entry point fails with LPHB_E_CUDA.  The handle-less build side is in scan_api.cu.
 #include <cuda_runtime.h>
 
 #include <cstdlib>
@@ -10,15 +10,12 @@
 #include <algorithm>
 #include <chrono>
 #include <memory>
-#include <mutex>
-#include <stdexcept>
 #include <string>
 #include <thread>
 #include <vector>
 
 #include "../../include/lphash_b200.h"
 #include "api_internal.h"
-#include "build_session.h"
 #include "check_kernels.cuh"
 #include "image_decode.cuh"
 #include "lph_image.h"
@@ -92,12 +89,49 @@ struct Workspace {
         CK(cudaEventRecord(ev_last, st));
         have_last = true;
     }
-    void ensure_pipeline() {
-        for (int i = 0; i < 2; ++i) {
-            cs[i].create();
-            ev_done[i].create(cudaEventDisableTiming);
+    // Stream of chunk j of a batch of n_chunks, called for j = 0, 1, ... in order: one chunk runs on s itself; several
+    // alternate between cs[0] and cs[1], which first wait for what s holds at chunk 0.  join_chunks then makes s wait
+    // for both.
+    cudaStream_t chunk_stream(cudaStream_t s, uint64_t j, uint64_t n_chunks) {
+        if (n_chunks < 2) return s;
+        if (j == 0) {
+            for (int i = 0; i < 2; ++i) {
+                cs[i].create();
+                ev_done[i].create(cudaEventDisableTiming);
+            }
+            ev_ready.create(cudaEventDisableTiming);
+            CK(cudaEventRecord(ev_ready, s));
         }
-        ev_ready.create(cudaEventDisableTiming);
+        if (j < 2) CK(cudaStreamWaitEvent(cs[j & 1], ev_ready, 0));
+        return cs[j & 1];
+    }
+    void join_chunks(cudaStream_t s, uint64_t n_chunks) {
+        if (n_chunks < 2) return;
+        for (int i = 0; i < 2; ++i) {
+            CK(cudaEventRecord(ev_done[i], cs[i]));
+            CK(cudaStreamWaitEvent(s, ev_done[i], 0));
+        }
+    }
+    // A call through the small block on s, ordered after the previous call: up(h) writes its input to [at, end) of
+    // the pinned mirror h, which goes up in one copy; kernels(d) enqueues its work on the device block d; [0, down)
+    // comes back in one copy to h, and the call returns after the device finished.  Returns false, doing nothing,
+    // when the block cannot hold `end` bytes or LPHB_NO_SMALL_PATH is set.
+    template <class Up, class Kernels>
+    bool small_round_trip(cudaStream_t s, uint64_t at, uint64_t end, uint64_t down, Up&& up, Kernels&& kernels) {
+        if (end > Small::kBytes || getenv("LPHB_NO_SMALL_PATH")) return false;
+        small.d.reserve(Small::kBytes);
+        small.h.reserve(Small::kBytes);
+        auto* h = small.h.as<unsigned char>();
+        auto* d = small.d.as<unsigned char>();
+        up(h);
+        order_after_previous(s);
+        CK(cudaMemcpyAsync(d + at, h + at, end - at, cudaMemcpyHostToDevice, s));
+        kernels(d);
+        mark_last(s);
+        CK(cudaMemcpyAsync(h, d, down, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        CK(cudaGetLastError());
+        return true;
     }
     // ring of event pairs bracketing the main kernel of the last kEvRing calls
     static constexpr int kEvRing = 128;
@@ -323,26 +357,6 @@ void check_chunk(lphb_mphf* f, DevBatch const& b, uint64_t j0, uint64_t j1, cons
     f->stats.kernel_launches += 1;
 }
 
-// Layout of a batch of contigs (host offsets): max(0, L-k+1) k-mers per contig and, with m, max(0, L-m+1) m-mers.
-// With code_offsets, writes where each contig's codes start (n_contigs + 1 entries).  Offsets that decrease are
-// an argument error (thrown; guarded() reports it as LPHB_E_ARG).
-struct ContigCounts {
-    uint64_t kmers = 0, mmers = 0;
-};
-ContigCounts contig_layout(const uint64_t* offsets, uint64_t n_contigs, uint32_t k, uint32_t m = 0,
-                           uint64_t* code_offsets = nullptr) {
-    ContigCounts n;
-    for (uint64_t c = 0; c < n_contigs; ++c) {
-        if (offsets[c + 1] < offsets[c]) throw std::invalid_argument("offsets must be non-decreasing");
-        const uint64_t len = offsets[c + 1] - offsets[c];
-        if (code_offsets) code_offsets[c] = n.kmers;
-        n.kmers += len >= k ? len - k + 1 : 0;
-        if (m) n.mmers += len >= m ? len - m + 1 : 0;
-    }
-    if (code_offsets) code_offsets[n_contigs] = n.kmers;
-    return n;
-}
-
 // ---- contigs with non-ACGT bytes (SURVEY.md Q1; quirk_kernels.cu) ----------------------------------------------
 // Their valid k-mers are ordinary work: the contigs are gathered into a compact batch, cut into maximal runs of
 // valid / invalid bytes, and the runs go through the same query kernel as contigs of their own.  Only the
@@ -551,47 +565,41 @@ struct HostQuery {
     // and flags arrive zeroed with it), the kernels, one copy down [codes | status].  Returns false when the batch
     // does not qualify, or when a contig holds a non-ACGT byte: the call then starts over on the general path.
     bool small_call() {
+        if (want_runs || sink.check || !codes || !total || total > codes_capacity) return false;
         const uint64_t codes_b = (total * 8 + 63) & ~uint64_t(63), dirty_b = (n_contigs + 8 + 63) & ~uint64_t(63);
         const uint64_t off_b = (n_contigs + 1) * 8;
-        const uint64_t in_b = 64 + dirty_b + 2 * off_b + span + 64, all_b = codes_b + in_b;
-        if (want_runs || sink.check || !codes || !total || total > codes_capacity || all_b > Workspace::Small::kBytes ||
-            getenv("LPHB_NO_SMALL_PATH"))
-            return false;
-        ws.small.d.reserve(Workspace::Small::kBytes);
-        ws.small.h.reserve(Workspace::Small::kBytes);
-        auto* h = ws.small.h.as<unsigned char>();
-        auto* d = ws.small.d.as<unsigned char>();
+        const uint64_t in_b = 64 + dirty_b + 2 * off_b + span + 64;
         const uint64_t at_status = codes_b, at_dirty = at_status + 64, at_off = at_dirty + dirty_b,
                        at_coff = at_off + off_b, at_bases = at_coff + off_b;
-        std::memset(h + at_status, 0, 64 + dirty_b);
-        std::memcpy(h + at_off, offsets, off_b);
-        std::memcpy(h + at_coff, code_offsets, off_b);
-        if (span) std::memcpy(h + at_bases, bases + first, span);
-        std::memset(h + at_bases + span, 'A', 64);
-        ws.order_after_previous(s);
-        CK(cudaMemcpyAsync(d + at_status, h + at_status, in_b, cudaMemcpyHostToDevice, s));
-        if (sink.non_streaming) launch_sanitize(reinterpret_cast<char*>(d + at_bases), span, s);
-        DevBatch b{};
-        b.bases = reinterpret_cast<const char*>(d + at_bases) - first;
-        b.offsets = reinterpret_cast<const uint64_t*>(d + at_off);
-        b.code_off = reinterpret_cast<const uint64_t*>(d + at_coff);
-        b.n_contigs = n_contigs;
-        b.first_base = first;
-        b.end_base = first + span;
-        b.codes = reinterpret_cast<uint64_t*>(d);
-        b.dirty = d + at_dirty;
-        b.status = reinterpret_cast<unsigned long long*>(d + at_status);
-        ws.tile.reserve(query_tiled_ws_bytes(span));
-        b.tile_ws = ws.tile.p;
-        b.tile_ws_bytes = ws.tile.cap;
-        run_kernels(f, b, s);
-        ws.mark_last(s);
-        CK(cudaMemcpyAsync(h, d, codes_b + 64, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        CK(cudaGetLastError());
+        auto up = [&](unsigned char* h) {
+            std::memset(h + at_status, 0, 64 + dirty_b);
+            std::memcpy(h + at_off, offsets, off_b);
+            std::memcpy(h + at_coff, code_offsets, off_b);
+            if (span) std::memcpy(h + at_bases, bases + first, span);
+            std::memset(h + at_bases + span, 'A', 64);
+        };
+        auto kernels = [&](unsigned char* d) {
+            if (sink.non_streaming) launch_sanitize(reinterpret_cast<char*>(d + at_bases), span, s);
+            DevBatch b{};
+            b.bases = reinterpret_cast<const char*>(d + at_bases) - first;
+            b.offsets = reinterpret_cast<const uint64_t*>(d + at_off);
+            b.code_off = reinterpret_cast<const uint64_t*>(d + at_coff);
+            b.n_contigs = n_contigs;
+            b.first_base = first;
+            b.end_base = first + span;
+            b.codes = reinterpret_cast<uint64_t*>(d);
+            b.dirty = d + at_dirty;
+            b.status = reinterpret_cast<unsigned long long*>(d + at_status);
+            ws.tile.reserve(query_tiled_ws_bytes(span));
+            b.tile_ws = ws.tile.p;
+            b.tile_ws_bytes = ws.tile.cap;
+            run_kernels(f, b, s);
+        };
+        if (!ws.small_round_trip(s, at_status, codes_b + in_b, codes_b + 64, up, kernels)) return false;
+        const auto* h = ws.small.h.as<unsigned char>();
         const auto* st = reinterpret_cast<const unsigned long long*>(h + at_status);
         f->last_dirty_n = n_contigs;
-        f->last_dirty = d + at_dirty;
+        f->last_dirty = ws.small.d.as<uint8_t>() + at_dirty;
         f->stats.h2d_bytes = in_b;
         f->stats.d2h_bytes = codes_b + 64;
         if (st[1] == 0) {
@@ -639,13 +647,8 @@ struct HostQuery {
         }
         ws.tile.reserve(tile_at[n_chunks]);
         if (want_runs) reserve_runs(max_codes + 16, copied_out ? 2 : 1, total, n_chunks);
-        if (copied_out) {
-            ws.ensure_pipeline();
-            CK(cudaEventRecord(ws.ev_ready, s));
-        }
         for (uint64_t j = 0; j < n_chunks; ++j) {
-            const cudaStream_t st = copied_out ? cudaStream_t(ws.cs[j & 1]) : s;
-            if (copied_out && j < 2) CK(cudaStreamWaitEvent(st, ws.ev_ready, 0));
+            const cudaStream_t st = ws.chunk_stream(s, j, n_chunks);
             const uint64_t c0 = cuts[j], c1 = cuts[j + 1];
             const uint64_t b0 = offsets[c0], b1 = offsets[c1];
             if (b1 > b0) {
@@ -675,13 +678,8 @@ struct HostQuery {
                 if (want_runs && j >= 1) fetch_runs(j - 1, code_offsets[cuts[j - 1]], ws.cs[(j - 1) & 1]);
             }
         }
-        if (copied_out) {
-            if (want_runs) fetch_runs(n_chunks - 1, code_offsets[cuts[n_chunks - 1]], ws.cs[(n_chunks - 1) & 1]);
-            for (int i = 0; i < 2; ++i) {
-                CK(cudaEventRecord(ws.ev_done[i], ws.cs[i]));
-                CK(cudaStreamWaitEvent(s, ws.ev_done[i], 0));
-            }
-        }
+        if (copied_out && want_runs) fetch_runs(n_chunks - 1, code_offsets[cuts[n_chunks - 1]], ws.cs[(n_chunks - 1) & 1]);
+        ws.join_chunks(s, n_chunks);
         auto* h_status = ws.h_status.as<unsigned long long>();
         CK(cudaMemcpyAsync(h_status, ws.status.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
@@ -779,99 +777,81 @@ int query_stream_host(lphb_mphf* f, const char* bases, const uint64_t* offsets, 
 
 // ---- batches in the caller's device buffers ------------------------------------------------------
 
-// lphb_query_stream_device and lphb_query_nonstreaming_device: the stateless codes of the batch, enqueued on s.
-// non_streaming: the kernels read a copy of the batch's bytes in the workspace with every non-ACGT byte made 'A',
-// so that every window has its code and the caller's bytes stay as they are.
-int device_query(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
-                 uint64_t n_contigs, uint64_t* d_codes, uint64_t codes_capacity, uint64_t* d_code_offsets,
-                 unsigned long long* st, cudaStream_t s, bool non_streaming) {
-    f->stats = lphb_stats{};
-    const uint32_t k = f->img.k;
-    const uint64_t total = contig_layout(h_offsets, n_contigs, k).kmers;
-    if (total > codes_capacity) return fail(LPHB_E_CAPACITY, "codes buffer too small");
-    if (total && (!d_bases || !d_codes)) return fail(LPHB_E_ARG, "null data pointer");
-    const uint64_t first = h_offsets[0], span = h_offsets[n_contigs] - first;
-    if (non_streaming && span && !d_bases) return fail(LPHB_E_ARG, "null data pointer");
+// What every call on a batch in the caller's device buffers runs first on s, ordered after the previous call: the
+// dirty flags cleared, the code offsets into code_off with status[0] = the k-mer total.  Reserves the workspace the
+// kernels use (with tile, the streaming pass's too) and returns the batch, its codes going to `codes`.
+// (growing a workspace buffer frees the old one: cudaFree waits for the device, so a previous call still running
+// never loses its buffer)
+DevBatch start_device_batch(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
+                            uint64_t n_contigs, uint64_t* code_off, uint64_t* codes, unsigned long long* status,
+                            bool tile, cudaStream_t s) {
     Workspace& ws = f->ws;
-    // (growing a workspace buffer frees the old one: cudaFree waits for the device, so a previous
-    // call still running never loses its buffer)
     ws.offsets_tmp.reserve(code_offsets_tmp_bytes(n_contigs));
     ws.dirty.reserve(n_contigs + 8);
-    ws.tile.reserve(query_tiled_ws_bytes(span));
-    if (non_streaming) ws.bases.reserve(span + 16 + kCopySanitizePad);
+    if (tile) ws.tile.reserve(query_tiled_ws_bytes(h_offsets[n_contigs] - h_offsets[0]));
     ws.order_after_previous(s);
     CK(cudaMemsetAsync(ws.dirty.p, 0, n_contigs + 8, s));
-    launch_code_offsets(d_offsets, n_contigs, k, d_code_offsets, st, ws.offsets_tmp.p, ws.offsets_tmp.cap, s);
+    launch_code_offsets(d_offsets, n_contigs, f->img.k, code_off, status, ws.offsets_tmp.p, ws.offsets_tmp.cap, s);
     f->stats.kernel_launches += 2;
-    const char* bases = d_bases;
-    if (non_streaming && span) {
-        launch_copy_sanitize(ws.bases.as<char>(), d_bases + first, span, s);
-        bases = ws.bases.as<char>() + copy_sanitize_at(d_bases + first) - first;  // indexed by the offsets
-        f->stats.kernel_launches += 1;
-    }
-    DevBatch b{};
-    b.bases = bases;
-    b.offsets = d_offsets;
-    b.code_off = d_code_offsets;
-    b.n_contigs = n_contigs;
-    b.first_base = first;
-    b.end_base = h_offsets[n_contigs];
-    b.codes = d_codes;
-    b.dirty = ws.dirty.as<uint8_t>();
-    b.status = st;
-    b.tile_ws = ws.tile.p;
-    b.tile_ws_bytes = ws.tile.cap;
-    if (n_contigs) run_kernels(f, b, s);
-    ws.mark_last(s);
     f->last_dirty_n = n_contigs;
     f->last_dirty = nullptr;
-    CK(cudaGetLastError());
-    return LPHB_OK;
-}
-
-// lphb_query_stream_exact_device: the clean pass of lphb_query_stream_device over the caller's batch, one read-back
-// of its status and, when a contig holds a non-ACGT byte, the repair lphb_query_stream runs.  The clean pass writes
-// straight into d_codes when the clean layout fits there, so a clean batch costs one device call more than the
-// stateless form: the status read.  A repair then assembles from a copy of those codes in the workspace, since the
-// assemble must not read the buffer it writes.
-int exact_device_query(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
-                       uint64_t n_contigs, uint64_t* d_codes, uint64_t codes_capacity, uint64_t* d_code_offsets,
-                       uint64_t* n_codes, cudaStream_t s) {
-    f->stats = lphb_stats{};
-    Workspace& ws = f->ws;
-    const uint32_t k = f->img.k;
-    std::vector<uint64_t> code_offsets(n_contigs + 1);
-    const uint64_t total = contig_layout(h_offsets, n_contigs, k, 0, code_offsets.data()).kmers;
-    *n_codes = total;
-    const uint64_t first = h_offsets[0], span = h_offsets[n_contigs] - first;
-    // (a contig shorter than k yields no code, spurious ones included: without a clean code there is none at all)
-    if ((span && !d_bases) || (total && !d_codes)) return fail(LPHB_E_ARG, "null data pointer");
-    const bool in_place = total <= codes_capacity;
-    ws.offsets_tmp.reserve(code_offsets_tmp_bytes(n_contigs));
-    ws.dirty.reserve(n_contigs + 8);
-    ws.tile.reserve(query_tiled_ws_bytes(span));
-    if (!in_place) ws.codes.reserve(total * 8 + 64);
-    ws.order_after_previous(s);
-    CK(cudaMemsetAsync(ws.dirty.p, 0, n_contigs + 8, s));
-    auto* st = ws.status.as<unsigned long long>();
-    launch_code_offsets(d_offsets, n_contigs, k, d_code_offsets, st, ws.offsets_tmp.p, ws.offsets_tmp.cap, s);
-    f->stats.kernel_launches += 2;
     DevBatch b{};
     b.bases = d_bases;
     b.offsets = d_offsets;
-    b.code_off = d_code_offsets;
+    b.code_off = code_off;
     b.n_contigs = n_contigs;
-    b.first_base = first;
+    b.first_base = h_offsets[0];
     b.end_base = h_offsets[n_contigs];
-    b.codes = in_place ? d_codes : ws.codes.as<uint64_t>();
+    b.codes = codes;
     b.dirty = ws.dirty.as<uint8_t>();
-    b.status = st;
+    b.status = status;
     b.tile_ws = ws.tile.p;
     b.tile_ws_bytes = ws.tile.cap;
+    return b;
+}
+
+// lphb_query_stream_device, lphb_query_nonstreaming_device and (n_codes not null) lphb_query_stream_exact_device.
+// The stateless forms enqueue the codes of the batch on s and count its dirty contigs into the caller's st.
+// non_streaming: the kernels read a copy of the batch's bytes in the workspace with every non-ACGT byte made 'A',
+// so that every window has its code and the caller's bytes stay as they are.
+// The exact form: the same clean pass, one read-back of its status and, when a contig holds a non-ACGT byte, the
+// repair lphb_query_stream runs.  The clean pass writes straight into d_codes when the clean layout fits there, so a
+// clean batch costs one device call more than the stateless form: the status read.  A repair then assembles from a
+// copy of those codes in the workspace, since the assemble must not read the buffer it writes.
+int device_query(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
+                 uint64_t n_contigs, uint64_t* d_codes, uint64_t codes_capacity, uint64_t* d_code_offsets,
+                 unsigned long long* st, uint64_t* n_codes, bool non_streaming, cudaStream_t s) {
+    f->stats = lphb_stats{};
+    Workspace& ws = f->ws;
+    const bool exact = n_codes != nullptr;
+    std::vector<uint64_t> code_offsets(exact ? n_contigs + 1 : 0);
+    // (one call per form, so that neither per-contig loop tests whether it writes code offsets)
+    const uint64_t total = exact ? contig_layout(h_offsets, n_contigs, f->img.k, 0, code_offsets.data()).kmers
+                                 : contig_layout(h_offsets, n_contigs, f->img.k).kmers;
+    const uint64_t first = h_offsets[0], span = h_offsets[n_contigs] - first;
+    if (exact) *n_codes = total;
+    else if (total > codes_capacity) return fail(LPHB_E_CAPACITY, "codes buffer too small");
+    // (a contig shorter than k yields no code, spurious ones included: without a clean code there is none at all;
+    // the stateless streaming form reads no byte of a batch without a k-mer)
+    if ((total && !d_codes) || (span && !d_bases && (total || exact || non_streaming)))
+        return fail(LPHB_E_ARG, "null data pointer");
+    const bool in_place = total <= codes_capacity;  // (only the exact form gets here with a clean layout too large)
+    if (non_streaming) ws.bases.reserve(span + 16 + kCopySanitizePad);
+    if (!in_place) ws.codes.reserve(total * 8 + 64);
+    if (exact) st = ws.status.as<unsigned long long>();
+    DevBatch b = start_device_batch(f, d_bases, d_offsets, h_offsets, n_contigs, d_code_offsets,
+                                    in_place ? d_codes : ws.codes.as<uint64_t>(), st, true, s);
+    if (non_streaming && span) {
+        launch_copy_sanitize(ws.bases.as<char>(), d_bases + first, span, s);
+        b.bases = ws.bases.as<char>() + copy_sanitize_at(d_bases + first) - first;  // indexed by the offsets
+        f->stats.kernel_launches += 1;
+    }
     if (n_contigs) run_kernels(f, b, s);
     ws.mark_last(s);
-    f->last_dirty_n = n_contigs;
-    f->last_dirty = nullptr;
+    if (!exact) {
+        CK(cudaGetLastError());
+        return LPHB_OK;
+    }
     auto* h_status = ws.h_status.as<unsigned long long>();
     CK(cudaMemcpyAsync(h_status, st, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
@@ -918,20 +898,10 @@ int lookup_host(lphb_mphf* f, const void* kmers, uint64_t n, uint64_t* codes) {
     f->stats.h2d_bytes = in_b;
     f->stats.d2h_bytes = out_b;
     const uint64_t codes_b = (out_b + 63) & ~uint64_t(63);  // [codes | k-mers]: the k-mers 16-byte aligned
-    if (codes_b + in_b <= Workspace::Small::kBytes && !getenv("LPHB_NO_SMALL_PATH")) {
-        ws.small.d.reserve(Workspace::Small::kBytes);
-        ws.small.h.reserve(Workspace::Small::kBytes);
-        auto* h = ws.small.h.as<unsigned char>();
-        auto* d = ws.small.d.as<unsigned char>();
-        std::memcpy(h + codes_b, kmers, in_b);
-        ws.order_after_previous(s);
-        CK(cudaMemcpyAsync(d + codes_b, h + codes_b, in_b, cudaMemcpyHostToDevice, s));
-        lookup_launch(f, d + codes_b, n, reinterpret_cast<uint64_t*>(d), s);
-        ws.mark_last(s);
-        CK(cudaMemcpyAsync(h, d, out_b, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        CK(cudaGetLastError());
-        std::memcpy(codes, h, out_b);
+    if (ws.small_round_trip(
+            s, codes_b, codes_b + in_b, out_b, [&](unsigned char* h) { std::memcpy(h + codes_b, kmers, in_b); },
+            [&](unsigned char* d) { lookup_launch(f, d + codes_b, n, reinterpret_cast<uint64_t*>(d), s); })) {
+        std::memcpy(codes, ws.small.h.p, out_b);
         return LPHB_OK;
     }
     const uint64_t per = std::max<uint64_t>(1, pipeline_chunk_bases() / kb);  // k-mers per chunk
@@ -939,15 +909,9 @@ int lookup_host(lphb_mphf* f, const void* kmers, uint64_t n, uint64_t* codes) {
     ws.bases.reserve(in_b + 64);
     ws.codes.reserve(out_b + 64);
     ws.order_after_previous(s);
-    const bool piped = n_chunks > 1;
-    if (piped) {
-        ws.ensure_pipeline();
-        CK(cudaEventRecord(ws.ev_ready, s));
-    }
     const auto* src = static_cast<const unsigned char*>(kmers);
     for (uint64_t j = 0; j < n_chunks; ++j) {
-        const cudaStream_t st = piped ? cudaStream_t(ws.cs[j & 1]) : s;
-        if (piped && j < 2) CK(cudaStreamWaitEvent(st, ws.ev_ready, 0));
+        const cudaStream_t st = ws.chunk_stream(s, j, n_chunks);
         const uint64_t i0 = j * per, c = std::min(per, n - i0);
         unsigned char* d_in = ws.bases.as<unsigned char>() + i0 * kb;
         uint64_t* d_out = ws.codes.as<uint64_t>() + i0;
@@ -955,12 +919,7 @@ int lookup_host(lphb_mphf* f, const void* kmers, uint64_t n, uint64_t* codes) {
         lookup_launch(f, d_in, c, d_out, st);
         CK(cudaMemcpyAsync(codes + i0, d_out, c * 8, cudaMemcpyDeviceToHost, st));
     }
-    if (piped) {
-        for (int i = 0; i < 2; ++i) {
-            CK(cudaEventRecord(ws.ev_done[i], ws.cs[i]));
-            CK(cudaStreamWaitEvent(s, ws.ev_done[i], 0));
-        }
-    }
+    ws.join_chunks(s, n_chunks);
     ws.mark_last(s);
     CK(cudaStreamSynchronize(s));
     CK(cudaGetLastError());
@@ -1011,35 +970,17 @@ int check_batch_device(lphb_mphf* f, const char* d_bases, const uint64_t* d_offs
     Workspace::Check& C = ws.check;
     f->stats = lphb_stats{};
     const uint64_t total = contig_layout(h_offsets, n_contigs, f->img.k).kmers;
-    const uint64_t first = h_offsets[0], span = h_offsets[n_contigs] - first;
+    const uint64_t span = h_offsets[n_contigs] - h_offsets[0];
     if (span && !d_bases) return fail(LPHB_E_ARG, "d_bases is null");
-    f->last_dirty_n = n_contigs;
-    f->last_dirty = nullptr;
-    if (n_contigs == 0) return LPHB_OK;
-    ws.offsets_tmp.reserve(code_offsets_tmp_bytes(n_contigs));
-    ws.code_off.reserve((n_contigs + 1) * 8);
-    ws.dirty.reserve(n_contigs + 8);
-    if (!d_stream_codes) {
-        ws.codes.reserve(total * 8 + 64);
-        ws.tile.reserve(query_tiled_ws_bytes(span));
+    if (n_contigs == 0) {
+        f->last_dirty_n = 0;
+        f->last_dirty = nullptr;
+        return LPHB_OK;
     }
-    ws.order_after_previous(s);
-    CK(cudaMemsetAsync(ws.dirty.p, 0, n_contigs + 8, s));
-    launch_code_offsets(d_offsets, n_contigs, f->img.k, ws.code_off.as<uint64_t>(), ws.status.as<unsigned long long>(),
-                        ws.offsets_tmp.p, ws.offsets_tmp.cap, s);
-    f->stats.kernel_launches += 2;
-    DevBatch b{};
-    b.bases = d_bases;
-    b.offsets = d_offsets;
-    b.code_off = ws.code_off.as<uint64_t>();
-    b.n_contigs = n_contigs;
-    b.first_base = first;
-    b.end_base = h_offsets[n_contigs];
-    b.codes = ws.codes.as<uint64_t>();
-    b.dirty = ws.dirty.as<uint8_t>();
-    b.status = ws.status.as<unsigned long long>();
-    b.tile_ws = ws.tile.p;
-    b.tile_ws_bytes = ws.tile.cap;
+    ws.code_off.reserve((n_contigs + 1) * 8);
+    if (!d_stream_codes) ws.codes.reserve(total * 8 + 64);
+    const DevBatch b = start_device_batch(f, d_bases, d_offsets, h_offsets, n_contigs, ws.code_off.as<uint64_t>(),
+                                          ws.codes.as<uint64_t>(), ws.status.as<unsigned long long>(), !d_stream_codes, s);
     check_chunk(f, b, 0, total, d_stream_codes, C.counters.as<unsigned long long>(), s);
     ws.mark_last(s);
     CK(cudaGetLastError());
@@ -1078,302 +1019,6 @@ int check_end(lphb_mphf* f, lphb_check_report* r) {
     r->min_duplicate_code = h[kCheckMinDuplicate];
     r->min_missing_code = h[kCheckMinMissing];
     r->ok = r->out_of_range == 0 && r->duplicates == 0 && r->missing == 0 && r->stream_mismatches == 0;
-    return LPHB_OK;
-}
-
-// ---- build-side scan ---------------------------------------------------------------------------
-
-// Device workspace of the build-side scan, kept per device between calls.
-struct ScanSession {
-    DevBuf bases, offsets, code_off, id_base, dirty, head, pos, rank, records, start_pos, tmp, status, tile_ws;
-    DevBuf r_starts, r_flag, r_voff, r_vstart, r_tmp, r_cnt, r_poff, r_pid;  // contigs with non-ACGT bytes: runs, pieces
-    Stream s;
-    ScanBatch b{};
-    uint64_t n_records = 0, n_kmers = 0, tmp_bytes = 0;
-    Event ev0, ev1;  // bracket the record-producing kernels of the last scan
-    double kernel_ms = 0;
-};
-
-// The scan entry points have no handle: their device workspace (a few bytes per base) is kept per
-// device between calls, so that a caller streaming batches does not pay cudaMalloc / cudaFree
-// (both synchronizing) on every batch.  One mutex PER DEVICE: scans on different GPUs driven from
-// different host threads run concurrently, scans on one GPU take turns; lphb_scan_release frees.
-struct ClassifySession;
-struct DeviceSessions {
-    std::mutex mu;
-    ScanSession* scan = nullptr;
-    ClassifySession* classify = nullptr;
-};
-DeviceSessions g_dev[64];
-DeviceSessions& device_sessions(int device) {
-    if (device < 0 || device >= 64) throw std::invalid_argument("device index out of range");
-    return g_dev[device];
-}
-ScanSession& scan_session(int device) {
-    DeviceSessions& d = device_sessions(device);
-    if (!d.scan) d.scan = new ScanSession();
-    return *d.scan;
-}
-
-// Checks a scan batch (host offsets) and counts its k-mers and m-mers; the session starts on it.
-ContigCounts begin_scan(ScanSession& S, uint32_t k, uint32_t m, const uint64_t* offsets, uint64_t n_contigs) {
-    if (m == 0 || m > 31 || k < m || k > 63) throw std::invalid_argument("need 1 <= m <= 31, m <= k <= 63");
-    const ContigCounts n = contig_layout(offsets, n_contigs, k, m);
-    if (n.kmers >= (1ull << 32) || (n_contigs && offsets[n_contigs] - offsets[0] >= (1ull << 32)))
-        throw std::invalid_argument("batch holds >= 2^32 k-mers or bases: split it");
-    S.n_kmers = n.kmers;
-    S.n_records = 0;
-    S.s.create();
-    return n;
-}
-
-// The scan of one batch whose bases and offsets are ALREADY on the device (d_bases indexed by the
-// offsets, i.e. d_bases + offsets[0] is the first base): leaves the records (scan order) and the
-// stream position of every record's first k-mer in the session, returns after the device finished.
-// Instantiated (k, m): one fused kernel (query_tiled.cu, kScan form); others: the generic passes.
-// One pass of the scan kernels over a partition of the stream into contigs.  d_bases is indexed by the offsets;
-// n_kmers = k-mers of the partition; d_id_base = m-mer ordinal of every contig's first m-mer, or null (then
-// mm_count_in + the m-mers of the contigs before it).  *n_dirty = contigs with non-ACGT bytes (their records are
-// meaningless; with `pieces` the partition was cut so that such contigs hold no k-mer at all).
-int scan_pass(ScanSession& S, uint32_t k, uint32_t m, uint64_t seed, const char* d_bases, const uint64_t* d_offsets,
-              uint64_t n_contigs, uint64_t first, uint64_t span, uint64_t n_kmers, uint64_t n_kmers_cap,
-              const uint64_t* d_id_base, uint64_t mm_count_in, bool pieces, uint64_t* n_dirty) {
-    cudaStream_t s = S.s;
-    S.code_off.reserve((n_contigs + 1) * 8);
-    S.id_base.reserve((n_contigs + 1) * 8);
-    S.dirty.reserve(n_contigs + 8);
-    S.status.reserve(64);
-    S.records.reserve(n_kmers_cap * 18 + 64);       // capacity: one record per k-mer (low-complexity worst case)
-    S.start_pos.reserve((n_kmers_cap + 2) * 4);
-    const bool tiled = scan_tiled_available(k, m);
-    uint64_t t1 = tiled ? 0 : head_ranks_tmp_bytes(n_kmers_cap > n_contigs ? n_kmers_cap : n_contigs);
-    uint64_t t2 = code_offsets_tmp_bytes(n_contigs);
-    uint64_t t3 = head_ranks_tmp_bytes(n_contigs);  // the m-mer ordinal scan over contigs
-    S.tmp_bytes = std::max(std::max(t1, t2), t3);
-    S.tmp.reserve(S.tmp_bytes);
-    if (!tiled) {
-        S.head.reserve(n_kmers_cap + 8);
-        S.pos.reserve(n_kmers_cap + 8);
-        S.rank.reserve((n_kmers_cap + 2) * 4);
-    }
-    S.tile_ws.reserve(query_tiled_ws_bytes(span));
-    S.ev0.create(cudaEventDefault);
-    S.ev1.create(cudaEventDefault);
-    CK(cudaMemsetAsync(S.dirty.p, 0, n_contigs + 8, s));
-    auto* st = S.status.as<unsigned long long>();
-    CK(cudaMemsetAsync(st, 0, 64, s));
-    launch_code_offsets(d_offsets, n_contigs, k, S.code_off.as<uint64_t>(), st, S.tmp.p, S.tmp_bytes, s);
-    if (!d_id_base) {
-        launch_id_base(d_offsets, n_contigs, m, mm_count_in, S.id_base.as<uint64_t>(), S.tmp.p, S.tmp_bytes, s);
-        d_id_base = S.id_base.as<uint64_t>();
-    }
-    if (pieces) {  // the partition's k-mer count is only known on the device
-        CK(cudaMemcpyAsync(&n_kmers, S.code_off.as<uint64_t>() + n_contigs, 8, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-    }
-    ScanBatch& b = S.b;
-    b.bases = d_bases;
-    b.offsets = d_offsets;
-    b.code_off = S.code_off.as<uint64_t>();
-    b.id_base = d_id_base;
-    b.n_contigs = n_contigs;
-    b.first_base = first;
-    b.end_base = first + span;
-    b.n_kmers = n_kmers;
-    b.k = k;
-    b.m = m;
-    b.seed = seed;
-    b.dirty = S.dirty.as<uint8_t>();
-    S.n_records = 0;
-    *n_dirty = 0;
-    // the generic kernels (and a batch without any k-mer) never see the bytes of contigs shorter than k: look at them here
-    if (!pieces && (!tiled || n_kmers == 0)) launch_flag_invalid_bytes(d_bases, first, span, d_offsets, n_contigs, b.dirty, s);
-    if (n_kmers == 0) {
-        if (!pieces) {
-            launch_count_dirty(b.dirty, n_contigs, st, s);
-            unsigned long long h_st[2] = {0, 0};
-            CK(cudaMemcpyAsync(h_st, st, sizeof(h_st), cudaMemcpyDeviceToHost, s));
-            CK(cudaStreamSynchronize(s));
-            *n_dirty = h_st[1];
-        }
-        return LPHB_OK;
-    }
-    CK(cudaEventRecord(S.ev0, s));
-    unsigned long long h_nrec = 0;
-    if (tiled) {
-        DevBatch qb{};
-        qb.bases = b.bases;
-        qb.offsets = b.offsets;
-        qb.code_off = b.code_off;
-        qb.n_contigs = n_contigs;
-        qb.first_base = b.first_base;
-        qb.end_base = b.end_base;
-        qb.dirty = b.dirty;
-        qb.status = st;
-        qb.tile_ws = S.tile_ws.p;
-        qb.tile_ws_bytes = S.tile_ws.cap;
-        if (!launch_scan_records_tiled(k, m, seed, qb, b.id_base, S.records.as<uint8_t>(), S.start_pos.as<uint32_t>(),
-                                       st + 2, s))
-            return fail(LPHB_E_ARG, "scan: batch too large for one launch");
-        CK(cudaEventRecord(S.ev1, s));
-        launch_count_dirty(b.dirty, n_contigs, st, s);
-    } else {
-        CK(cudaMemsetAsync(S.head.p, 0, n_kmers + 8, s));
-        launch_scan_heads(b, S.head.as<uint8_t>(), S.pos.as<uint8_t>(), s);
-        launch_count_dirty(b.dirty, n_contigs, st, s);
-        launch_head_ranks(S.head.as<uint8_t>(), n_kmers, S.rank.as<uint32_t>(), S.tmp.p, S.tmp_bytes, s);
-    }
-    unsigned long long h_st[3] = {0, 0, 0};
-    uint32_t n_rec32 = 0;
-    CK(cudaMemcpyAsync(h_st, st, sizeof(h_st), cudaMemcpyDeviceToHost, s));
-    if (!tiled) CK(cudaMemcpyAsync(&n_rec32, S.rank.as<uint32_t>() + n_kmers, 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    CK(cudaGetLastError());
-    *n_dirty = h_st[1];
-    if (h_st[1] != 0 && !pieces) return LPHB_OK;  // the caller cuts the batch at the invalid bytes and comes back
-    h_nrec = tiled ? h_st[2] : n_rec32;
-    S.n_records = h_nrec;
-    if (!tiled) {
-        launch_scan_emit(b, S.head.as<uint8_t>(), S.pos.as<uint8_t>(), S.rank.as<uint32_t>(),
-                         S.records.as<uint8_t>(), S.start_pos.as<uint32_t>(), s);
-        CK(cudaEventRecord(S.ev1, s));
-        CK(cudaStreamSynchronize(s));
-        CK(cudaGetLastError());
-    }
-    float ms = 0;
-    if (cudaEventElapsedTime(&ms, S.ev0, S.ev1) == cudaSuccess) S.kernel_ms = ms; else cudaGetLastError();
-    return LPHB_OK;
-}
-
-int run_scan_device(ScanSession& S, uint32_t k, uint32_t m, uint64_t seed, const char* d_bases,
-                    const uint64_t* d_offsets, const uint64_t* offsets, uint64_t n_contigs, uint64_t mm_count_in,
-                    uint64_t* mm_count_out) {
-    cudaStream_t s = S.s;
-    const uint64_t first = offsets[0], span = offsets[n_contigs] - first;
-    const uint64_t n_kmers = S.n_kmers;
-    uint64_t n_dirty = 0;
-    int rc = scan_pass(S, k, m, seed, d_bases, d_offsets, n_contigs, first, span, n_kmers, n_kmers, nullptr, mm_count_in,
-                       false, &n_dirty);
-    if (rc != LPHB_OK || n_dirty == 0) return rc;
-    // Contigs with non-ACGT bytes (include/minimizer.hpp:138-151): every maximal valid run is scanned as a contig
-    // of its own (quirk_kernels.cu, build side); k-mer and m-mer totals come from the runs.
-    if (k < 2) return fail(LPHB_E_ARG, "build input with non-ACGT bytes needs k >= 2");
-    const char* rel = d_bases + first;  // positions below are relative to the batch
-    S.r_starts.reserve((n_contigs + 2) * 8);
-    S.r_flag.reserve(span + 8);
-    S.r_voff.reserve((span + 2) * 8);
-    S.r_vstart.reserve((n_contigs + 2) * 4);
-    const uint64_t qt = quirk_tmp_bytes(span + 2);
-    S.r_tmp.reserve(qt);
-    auto* st = S.status.as<unsigned long long>();
-    launch_shift_starts(d_offsets, n_contigs, first, S.r_starts.as<uint64_t>(), s);
-    launch_find_runs(rel, span, S.r_starts.as<uint64_t>(), n_contigs, S.r_flag.as<uint8_t>(), S.r_voff.as<uint64_t>(), st + 4,
-                     S.r_vstart.as<uint32_t>(), S.r_tmp.p, qt, s);
-    unsigned long long n_v = 0;
-    CK(cudaMemcpyAsync(&n_v, st + 4, 8, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    S.r_cnt.reserve(3 * (n_v + 1) * 8);
-    uint64_t *d_pieces = S.r_cnt.as<uint64_t>(), *d_ids = d_pieces + (n_v + 1), *d_kmers = d_ids + (n_v + 1);
-    launch_build_run_counts(rel, S.r_voff.as<uint64_t>(), st + 4, S.r_vstart.as<uint32_t>(), n_contigs, n_v, k, m, d_pieces,
-                            d_ids, d_kmers, S.r_tmp.p, qt, s);
-    uint64_t totals[3] = {0, 0, 0};
-    CK(cudaMemcpyAsync(&totals[0], d_pieces + n_v, 8, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(&totals[1], d_ids + n_v, 8, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(&totals[2], d_kmers + n_v, 8, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    const uint64_t n_pieces = totals[0];
-    S.r_poff.reserve((n_pieces + 2) * 8);
-    S.r_pid.reserve((n_pieces + 2) * 8);
-    launch_build_pieces(S.r_voff.as<uint64_t>(), st + 4, n_v, k, d_pieces, d_ids, mm_count_in, span, S.r_poff.as<uint64_t>(),
-                        S.r_pid.as<uint64_t>(), s);
-    *mm_count_out = mm_count_in + totals[1];
-    rc = scan_pass(S, k, m, seed, rel, S.r_poff.as<uint64_t>(), n_pieces, 0, span, 0, n_kmers, S.r_pid.as<uint64_t>(),
-                   mm_count_in, true, &n_dirty);
-    S.n_kmers = totals[2];  // what from_string returns: the swallowed k-mers of exactly-k runs included
-    return rc;
-}
-
-// Validates a host batch, moves it to the device and scans it.
-int run_scan(ScanSession& S, uint32_t k, uint32_t m, uint64_t seed, const char* bases,
-             const uint64_t* offsets, uint64_t n_contigs, uint64_t mm_count_in,
-             uint64_t* mm_count_out) {
-    const ContigCounts n = begin_scan(S, k, m, offsets, n_contigs);
-    *mm_count_out = mm_count_in + n.mmers;
-    if (n_contigs == 0 || n.mmers == 0) return LPHB_OK;  // (without a k-mer there is no record, but an invalid byte
-    if (!bases) return fail(LPHB_E_ARG, "bases is null");  //  still changes the m-mer ordinals: the device decides)
-    cudaStream_t s = S.s;
-    const uint64_t first = offsets[0], span = offsets[n_contigs] - first;
-    S.bases.reserve(span + 64);
-    S.offsets.reserve((n_contigs + 1) * 8);
-    CK(cudaMemcpyAsync(S.bases.p, bases + first, span, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(S.offsets.p, offsets, (n_contigs + 1) * 8, cudaMemcpyHostToDevice, s));
-    return run_scan_device(S, k, m, seed, S.bases.as<char>() - first, S.offsets.as<uint64_t>(), offsets, n_contigs,
-                           mm_count_in, mm_count_out);
-}
-
-struct ClassifySession {
-    DevBuf rec, key, key2, idx, idx2, flags, gslot, cslot, counts, tmp, trip, idu, ids_s;
-};
-ClassifySession& classify_session(int device) {
-    DeviceSessions& d = device_sessions(device);
-    if (!d.classify) d.classify = new ClassifySession();
-    return *d.classify;
-}
-
-// Sort by minimizer + classify of n records that are already on the device (stream s); results to host.
-int classify_device(const uint8_t* d_rec, uint64_t n, void* triplets, uint64_t triplets_capacity,
-                    uint64_t* n_triplets, uint64_t* ids, uint64_t ids_capacity, uint64_t* n_ids,
-                    int key_bits, cudaStream_t s) {
-    // workspace kept per device between calls (freed by lphb_scan_release); callers hold the device's mutex
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    ClassifySession& cs = classify_session(dev);
-    DevBuf &key = cs.key, &key2 = cs.key2, &idx = cs.idx, &idx2 = cs.idx2, &flags = cs.flags, &gslot = cs.gslot,
-           &cslot = cs.cslot, &counts = cs.counts, &tmp = cs.tmp, &trip = cs.trip, &idu = cs.idu, &ids_s = cs.ids_s;
-    key.reserve(n * 8);
-    key2.reserve(n * 8);
-    idx.reserve(n * 4);
-    idx2.reserve(n * 4);
-    flags.reserve(n + 8);
-    gslot.reserve(n * 4);
-    cslot.reserve(n * 4);
-    counts.reserve(64);
-    const uint64_t tb = classify_tmp_bytes(n);
-    tmp.reserve(tb);
-    launch_classify_groups(d_rec, n, key.as<uint64_t>(), key2.as<uint64_t>(), idx.as<uint32_t>(),
-                           idx2.as<uint32_t>(), flags.as<uint8_t>(), gslot.as<uint32_t>(), cslot.as<uint32_t>(),
-                           counts.as<unsigned long long>(), tmp.p, tb, key_bits, s);
-    unsigned long long h_counts[2] = {0, 0};
-    CK(cudaMemcpyAsync(h_counts, counts.p, sizeof(h_counts), cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    CK(cudaGetLastError());
-    *n_triplets = h_counts[0];
-    *n_ids = h_counts[1];
-    if (h_counts[0] > triplets_capacity) return fail(LPHB_E_CAPACITY, "triplets buffer too small");
-    if (h_counts[1] > ids_capacity) return fail(LPHB_E_CAPACITY, "ids buffer too small");
-    if (!triplets || (h_counts[1] && !ids)) return fail(LPHB_E_ARG, "null output buffer");
-    trip.reserve(h_counts[0] * 10 + 64);
-    idu.reserve(h_counts[1] * 8 + 64);
-    ids_s.reserve(h_counts[1] * 8 + 64);
-    launch_classify_emit(d_rec, key2.as<uint64_t>(), idx2.as<uint32_t>(), flags.as<uint8_t>(),
-                         gslot.as<uint32_t>(), cslot.as<uint32_t>(), n, trip.as<uint8_t>(), idu.as<uint64_t>(),
-                         ids_s.as<uint64_t>(), h_counts[1], tmp.p, tb, s);
-    CK(cudaMemcpyAsync(triplets, trip.p, h_counts[0] * 10, cudaMemcpyDeviceToHost, s));
-    if (h_counts[1]) CK(cudaMemcpyAsync(ids, ids_s.p, h_counts[1] * 8, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    CK(cudaGetLastError());
-    return LPHB_OK;
-}
-
-// Adds the batch the scan session holds (records still on the device) to a build session.
-int build_take_scan(lphb_build* b, ScanSession& S, uint64_t n_contigs, uint64_t mm_out) {
-    build_add_batch(b, S.records.as<uint8_t>(), S.n_records, S.s);
-    lphb_build_report& t = b->totals;
-    t.batches += 1;
-    t.contigs += n_contigs;
-    t.kmers += S.n_kmers;
-    t.records += S.n_records;
-    t.mm_count = mm_out;
     return LPHB_OK;
 }
 
@@ -1513,7 +1158,7 @@ int lphb_query_stream_device(lphb_mphf* f, const char* d_bases, const uint64_t* 
     return guarded([&]() -> int {
         DeviceGuard g(f->device);
         return device_query(f, d_bases, d_offsets, h_offsets, n_contigs, d_codes, codes_capacity, d_code_offsets,
-                            reinterpret_cast<unsigned long long*>(d_status), static_cast<cudaStream_t>(stream), false);
+                            reinterpret_cast<unsigned long long*>(d_status), nullptr, false, static_cast<cudaStream_t>(stream));
     });
 }
 
@@ -1526,7 +1171,7 @@ int lphb_query_nonstreaming_device(lphb_mphf* f, const char* d_bases, const uint
     return guarded([&]() -> int {
         DeviceGuard g(f->device);
         return device_query(f, d_bases, d_offsets, h_offsets, n_contigs, d_codes, codes_capacity, d_code_offsets,
-                            reinterpret_cast<unsigned long long*>(d_status), static_cast<cudaStream_t>(stream), true);
+                            reinterpret_cast<unsigned long long*>(d_status), nullptr, true, static_cast<cudaStream_t>(stream));
     });
 }
 
@@ -1538,8 +1183,8 @@ int lphb_query_stream_exact_device(lphb_mphf* f, const char* d_bases, const uint
         return fail(LPHB_E_ARG, "null argument");
     return guarded([&]() -> int {
         DeviceGuard g(f->device);
-        return exact_device_query(f, d_bases, d_offsets, h_offsets, n_contigs, d_codes, codes_capacity, d_code_offsets,
-                                  n_codes, static_cast<cudaStream_t>(stream));
+        return device_query(f, d_bases, d_offsets, h_offsets, n_contigs, d_codes, codes_capacity, d_code_offsets,
+                            nullptr, n_codes, false, static_cast<cudaStream_t>(stream));
     });
 }
 
@@ -1694,208 +1339,6 @@ int lphb_expand_runs(const void* runs, uint64_t n_runs, uint64_t* codes, uint64_
             for (int t = 0; t < threads; ++t) pool.emplace_back(work, t);
             for (auto& th : pool) th.join();
         }
-        return LPHB_OK;
-    });
-}
-
-int lphb_scan_superkmers(int device, uint32_t k, uint32_t m, uint64_t seed, const char* bases,
-                         const uint64_t* offsets, uint64_t n_contigs, uint64_t* mm_count,
-                         void* records, uint64_t records_capacity, uint64_t* n_records,
-                         uint64_t* n_kmers) {
-    if (!offsets || !mm_count || !n_records || !n_kmers) return fail(LPHB_E_ARG, "null argument");
-    return guarded([&]() -> int {
-        DeviceGuard g(device);
-        std::lock_guard<std::mutex> lock(device_sessions(device).mu);
-        ScanSession& S = scan_session(device);
-        uint64_t mm_out = *mm_count;
-        int rc = run_scan(S, k, m, seed, bases, offsets, n_contigs, *mm_count, &mm_out);
-        if (rc != LPHB_OK) return rc;
-        *n_kmers = S.n_kmers;
-        *n_records = S.n_records;
-        if (S.n_records > records_capacity) return fail(LPHB_E_CAPACITY, "records buffer too small");
-        if (S.n_records) {
-            if (!records) return fail(LPHB_E_ARG, "records is null");
-            CK(cudaMemcpyAsync(records, S.records.p, S.n_records * 18, cudaMemcpyDeviceToHost, S.s));
-        }
-        CK(cudaStreamSynchronize(S.s));
-        *mm_count = mm_out;
-        return LPHB_OK;
-    });
-}
-
-int lphb_scan_superkmers_device(int device, uint32_t k, uint32_t m, uint64_t seed, const char* d_bases,
-                                const uint64_t* d_offsets, const uint64_t* h_offsets, uint64_t n_contigs,
-                                uint64_t* mm_count, const void** d_records, uint64_t* n_records, uint64_t* n_kmers,
-                                double* kernel_ms) {
-    if (!h_offsets || !d_offsets || !mm_count || !d_records || !n_records || !n_kmers)
-        return fail(LPHB_E_ARG, "null argument");
-    return guarded([&]() -> int {
-        DeviceGuard g(device);
-        std::lock_guard<std::mutex> lock(device_sessions(device).mu);
-        ScanSession& S = scan_session(device);
-        const ContigCounts n = begin_scan(S, k, m, h_offsets, n_contigs);
-        *n_kmers = n.kmers;
-        *n_records = 0;
-        *d_records = nullptr;
-        if (kernel_ms) *kernel_ms = 0;
-        uint64_t mm_out = *mm_count + n.mmers;
-        if (n_contigs && n.mmers) {
-            if (!d_bases) return fail(LPHB_E_ARG, "d_bases is null");
-            CK(cudaDeviceSynchronize());  // the caller's buffers may still be written on other streams
-            int rc = run_scan_device(S, k, m, seed, d_bases, d_offsets, h_offsets, n_contigs, *mm_count, &mm_out);
-            if (rc != LPHB_OK) return rc;
-            *d_records = S.records.p;
-            *n_records = S.n_records;
-            *n_kmers = S.n_kmers;  // (differs from the count above when contigs hold non-ACGT bytes)
-            if (kernel_ms) *kernel_ms = S.kernel_ms;
-        }
-        *mm_count = mm_out;
-        return LPHB_OK;
-    });
-}
-
-int lphb_scan_release(int device) {
-    return guarded([&]() -> int {
-        if (device < 0 || device >= 64) return LPHB_OK;
-        DeviceSessions& d = device_sessions(device);
-        std::lock_guard<std::mutex> lock(d.mu);
-        if (!d.scan && !d.classify) return LPHB_OK;
-        DeviceGuard g(device);
-        delete d.scan;
-        d.scan = nullptr;
-        delete d.classify;
-        d.classify = nullptr;
-        return LPHB_OK;
-    });
-}
-
-int lphb_classify(int device, const void* records, uint64_t n_records, void* triplets,
-                  uint64_t triplets_capacity, uint64_t* n_triplets, uint64_t* ids, uint64_t ids_capacity,
-                  uint64_t* n_ids) {
-    if (!n_triplets || !n_ids || (n_records && !records)) return fail(LPHB_E_ARG, "null argument");
-    if (n_records >= (1ull << 32)) return fail(LPHB_E_ARG, "batch holds >= 2^32 records: split it");
-    return guarded([&]() -> int {
-        DeviceGuard g(device);
-        *n_triplets = 0;
-        *n_ids = 0;
-        if (n_records == 0) return LPHB_OK;
-        std::lock_guard<std::mutex> lock(device_sessions(device).mu);
-        DevBuf& rec = classify_session(device).rec;
-        Stream s;
-        s.create();
-        rec.reserve(n_records * 18 + 64);
-        CK(cudaMemcpyAsync(rec.p, records, n_records * 18, cudaMemcpyHostToDevice, s));
-        return classify_device(rec.as<uint8_t>(), n_records, triplets, triplets_capacity, n_triplets, ids,
-                               ids_capacity, n_ids, 64, s);  // m unknown here: all key bits
-    });
-}
-
-int lphb_scan_classify(int device, uint32_t k, uint32_t m, uint64_t seed, const char* bases,
-                       const uint64_t* offsets, uint64_t n_contigs, uint64_t* mm_count, void* triplets,
-                       uint64_t triplets_capacity, uint64_t* n_triplets, uint64_t* ids,
-                       uint64_t ids_capacity, uint64_t* n_ids, uint64_t* n_kmers) {
-    if (!offsets || !mm_count || !n_triplets || !n_ids || !n_kmers) return fail(LPHB_E_ARG, "null argument");
-    return guarded([&]() -> int {
-        DeviceGuard g(device);
-        std::lock_guard<std::mutex> lock(device_sessions(device).mu);
-        ScanSession& S = scan_session(device);
-        uint64_t mm_out = *mm_count;
-        int rc = run_scan(S, k, m, seed, bases, offsets, n_contigs, *mm_count, &mm_out);
-        if (rc != LPHB_OK) return rc;
-        *n_kmers = S.n_kmers;
-        *n_triplets = 0;
-        *n_ids = 0;
-        if (S.n_records) {  // the records never leave the device
-            rc = classify_device(S.records.as<uint8_t>(), S.n_records, triplets, triplets_capacity, n_triplets,
-                                 ids, ids_capacity, n_ids, int(2 * m), S.s);  // a minimizer is 2m bits
-            if (rc != LPHB_OK) return rc;
-        }
-        *mm_count = mm_out;
-        return LPHB_OK;
-    });
-}
-
-int lphb_build_batch(lphb_build* b, const char* bases, const uint64_t* offsets, uint64_t n_contigs) {
-    if (!b || !offsets) return fail(LPHB_E_ARG, "null argument");
-    if (!b->dev) return fail(LPHB_E_ARG, "the build session has ended");
-    return guarded_nomem([&]() -> int {
-        DeviceGuard g(b->device);
-        std::lock_guard<std::mutex> lock(device_sessions(b->device).mu);
-        ScanSession& S = scan_session(b->device);
-        uint64_t mm_out = b->totals.mm_count;
-        int rc = run_scan(S, b->k, b->m, b->seed, bases, offsets, n_contigs, b->totals.mm_count, &mm_out);
-        if (rc != LPHB_OK) return rc;
-        return build_take_scan(b, S, n_contigs, mm_out);
-    });
-}
-
-int lphb_build_batch_device(lphb_build* b, const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
-                            uint64_t n_contigs, void* stream) {
-    if (!b || !d_offsets || !h_offsets) return fail(LPHB_E_ARG, "null argument");
-    if (!b->dev) return fail(LPHB_E_ARG, "the build session has ended");
-    return guarded_nomem([&]() -> int {
-        DeviceGuard g(b->device);
-        std::lock_guard<std::mutex> lock(device_sessions(b->device).mu);
-        ScanSession& S = scan_session(b->device);
-        const ContigCounts n = begin_scan(S, b->k, b->m, h_offsets, n_contigs);
-        uint64_t mm_out = b->totals.mm_count + n.mmers;
-        if (n_contigs && n.mmers) {
-            if (!d_bases) return fail(LPHB_E_ARG, "d_bases is null");
-            CK(cudaStreamSynchronize(static_cast<cudaStream_t>(stream)));  // the caller wrote its buffers on `stream`
-            int rc = run_scan_device(S, b->k, b->m, b->seed, d_bases, d_offsets, h_offsets, n_contigs, b->totals.mm_count,
-                                     &mm_out);
-            if (rc != LPHB_OK) return rc;
-        }
-        return build_take_scan(b, S, n_contigs, mm_out);
-    });
-}
-
-int lphb_colliding_kmers(int device, uint32_t k, uint32_t m, uint64_t seed, const char* bases,
-                         const uint64_t* offsets, uint64_t n_contigs, uint64_t* mm_count,
-                         const uint64_t* ids, uint64_t n_ids, int kmer_bits, void* kmers,
-                         uint64_t kmers_capacity, uint64_t* n_kmers) {
-    if (!offsets || !mm_count || !n_kmers || (n_ids && !ids)) return fail(LPHB_E_ARG, "null argument");
-    if (kmer_bits != 64 && kmer_bits != 128) return fail(LPHB_E_ARG, "kmer_bits must be 64 or 128");
-    if (k > uint32_t(kmer_bits / 2 - 1)) return fail(LPHB_E_ARG, "k too large for this kmer_t");
-    return guarded([&]() -> int {
-        DeviceGuard g(device);
-        std::lock_guard<std::mutex> lock(device_sessions(device).mu);
-        ScanSession& S = scan_session(device);
-        uint64_t mm_out = *mm_count;
-        int rc = run_scan(S, k, m, seed, bases, offsets, n_contigs, *mm_count, &mm_out);
-        if (rc != LPHB_OK) return rc;
-        *n_kmers = 0;
-        if (S.n_records == 0 || n_ids == 0) {
-            *mm_count = mm_out;
-            return LPHB_OK;
-        }
-        DevBuf d_ids, take, out_off, out;
-        cudaStream_t s = S.s;
-        d_ids.reserve(n_ids * 8);
-        take.reserve((S.n_records + 1) * 4);
-        out_off.reserve((S.n_records + 1) * 8);
-        CK(cudaMemcpyAsync(d_ids.p, ids, n_ids * 8, cudaMemcpyHostToDevice, s));
-        launch_colliding_mark(S.records.as<uint8_t>(), S.n_records, d_ids.as<uint64_t>(), n_ids,
-                              take.as<uint32_t>(), s);
-        uint64_t tb = exclusive_u32_tmp_bytes(S.n_records);
-        S.tmp.reserve(tb);
-        launch_exclusive_u32(take.as<uint32_t>(), S.n_records, out_off.as<uint64_t>(), S.tmp.p, tb, s);
-        uint64_t total = 0;
-        CK(cudaMemcpyAsync(&total, out_off.as<uint64_t>() + S.n_records, 8, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        *n_kmers = total;
-        if (total > kmers_capacity) return fail(LPHB_E_CAPACITY, "kmers buffer too small");
-        if (total) {
-            if (!kmers) return fail(LPHB_E_ARG, "kmers is null");
-            const uint64_t bytes = total * uint64_t(kmer_bits / 8);
-            out.reserve(bytes + 64);
-            launch_colliding_emit(S.b, S.n_records, S.start_pos.as<uint32_t>(), take.as<uint32_t>(),
-                                  out_off.as<uint64_t>(), kmer_bits, out.as<uint8_t>(), s);
-            CK(cudaMemcpyAsync(kmers, out.p, bytes, cudaMemcpyDeviceToHost, s));
-            CK(cudaStreamSynchronize(s));
-            CK(cudaGetLastError());
-        }
-        *mm_count = mm_out;
         return LPHB_OK;
     });
 }

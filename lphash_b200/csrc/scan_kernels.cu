@@ -108,46 +108,6 @@ __global__ void __launch_bounds__(256) k_scan_heads(const __grid_constant__ Scan
     }
 }
 
-// b(i) = i + pos(i) is the absolute position of k-mer i's minimizer: a record starts where
-// b(i) != b(i-1), i.e. pos(i) + 1 != pos(i-1), and at every contig's first k-mer.
-__global__ void k_heads_from_pos(const uint8_t* pos, uint64_t n, uint8_t* head) {
-    // 16 k-mers per thread: one 16-byte load of the offsets, one 16-byte store of the flags
-    const uint64_t n16 = (n + 15) / 16;
-    for (uint64_t t = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; t < n16; t += uint64_t(gridDim.x) * blockDim.x) {
-        const uint64_t d0 = t * 16;
-        uint32_t prev = d0 ? pos[d0 - 1] : 0x1FFu;  // no predecessor: never equal to pos + 1
-        if (d0 + 16 <= n) {
-            const uint4 v = *reinterpret_cast<const uint4*>(pos + d0);
-            const uint32_t w[4] = {v.x, v.y, v.z, v.w};
-            uint32_t o[4];
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                uint32_t f = 0;
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const uint32_t p = (w[q] >> (8 * j)) & 0xFFu;
-                    f |= (p + 1u != prev ? 1u : 0u) << (8 * j);
-                    prev = p;
-                }
-                o[q] = f;
-            }
-            *reinterpret_cast<uint4*>(head + d0) = make_uint4(o[0], o[1], o[2], o[3]);
-        } else {
-            for (uint64_t d = d0; d < n; ++d) {
-                const uint32_t p = pos[d];
-                head[d] = p + 1u != prev ? 1 : 0;
-                prev = p;
-            }
-        }
-    }
-}
-__global__ void k_heads_contig_first(const uint64_t* code_off, uint64_t n_contigs, uint8_t* head) {
-    for (uint64_t c = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; c < n_contigs; c += uint64_t(gridDim.x) * blockDim.x) {
-        const uint64_t a = code_off[c];
-        if (code_off[c + 1] > a) head[a] = 1;
-    }
-}
-
 struct U8ToU32 {
     __host__ __device__ uint32_t operator()(uint8_t v) const { return v; }
 };
@@ -306,12 +266,6 @@ void launch_scan_heads(ScanBatch const& b, uint8_t* head, uint8_t* pos, cudaStre
     uint64_t span = b.end_base - b.first_base;
     if (!span) return;
     k_scan_heads<<<grid_for(span), 256, 0, stream>>>(b, head, pos);
-}
-
-void launch_heads_from_pos(ScanBatch const& b, const uint8_t* pos, uint8_t* head, cudaStream_t stream) {
-    if (!b.n_kmers) return;
-    k_heads_from_pos<<<grid_for((b.n_kmers + 15) / 16), 256, 0, stream>>>(pos, b.n_kmers, head);
-    k_heads_contig_first<<<grid_for(b.n_contigs), 256, 0, stream>>>(b.code_off, b.n_contigs, head);
 }
 
 uint64_t head_ranks_tmp_bytes(uint64_t n_kmers) {

@@ -25,9 +25,6 @@ void launch_id_base(const uint64_t* d_offsets, uint64_t n_contigs, uint32_t m, u
 // Pass 1: head[d] = 1 where k-mer d starts a super-k-mer, pos[d] = offset of its minimizer.
 void launch_scan_heads(ScanBatch const& b, uint8_t* head, uint8_t* pos, cudaStream_t stream);
 
-// Pass 1 when pos[] came from the tiled kernel (launch_scan_pos_tiled): head flags from pos alone.
-void launch_heads_from_pos(ScanBatch const& b, const uint8_t* pos, uint8_t* head, cudaStream_t stream);
-
 // rank[d] = number of heads before d (exclusive); rank[n_kmers] = number of records.
 void launch_head_ranks(const uint8_t* head, uint64_t n_kmers, uint32_t* rank, void* d_tmp,
                        uint64_t tmp_bytes, cudaStream_t stream);
