@@ -93,7 +93,11 @@ int lphb_mphf_info(const lphb_mphf* f, lphb_info* info);
  *                 code_offsets[c+1] - code_offsets[c] codes: L-k+1 for an ACGT-only contig of
  *                 length L >= k, 0 if L < k; contigs with other bytes follow the reference's
  *                 streaming behaviour exactly (its spurious entries included, SURVEY.md Q1)
- *   n_codes       total number of codes (also set when returning LPHB_E_CAPACITY)              */
+ *   n_codes       total number of codes (also set when returning LPHB_E_CAPACITY)
+ * Workspace: beyond the staging of the batch, a batch with a contig holding a non-ACGT byte grows the handle's
+ * repair scratch (the device repair of lphb_query_stream_exact_device_async) to 68 bytes per contig + 9.03 bytes
+ * per base of the whole batch + 12 KB, plus 8 bytes per code of the result; it is kept for the next call.  The same
+ * holds for lphb_query_stream_runs.                                                                               */
 int lphb_query_stream(lphb_mphf* f, const char* bases, const uint64_t* offsets,
                       uint64_t n_contigs, uint64_t* codes, uint64_t codes_capacity,
                       uint64_t* code_offsets, uint64_t* n_codes);
@@ -134,8 +138,9 @@ int lphb_expand_runs(const void* runs, uint64_t n_runs, uint64_t* codes, uint64_
  * ACGT bases, SURVEY.md S1); d_status[0] = number of codes laid out (sum of max(0, L-k+1)),
  * d_status[1] = number of contigs containing a non-ACGT byte.  For such a contig the code slot of
  * every k-mer window that contains a non-ACGT byte is UNSPECIFIED (the slots of its other k-mers hold
- * their codes); lphb_mphf_dirty_flags names those contigs, and lphb_query_stream and
- * lphb_query_stream_exact_device apply the reference's exact streaming behaviour to them - this call does not.
+ * their codes); lphb_mphf_dirty_flags names those contigs, and lphb_query_stream,
+ * lphb_query_stream_exact_device and lphb_query_stream_exact_device_async apply the reference's exact streaming
+ * behaviour to them - this call does not.
  * Ordering: a handle owns one device workspace, so consecutive calls on one handle are ordered on
  * the device (each call makes its stream wait for the previous call's kernels), on whatever
  * streams they are issued; they never overlap each other.  Overlap comes from several handles or
@@ -148,10 +153,12 @@ int lphb_query_stream_device(lphb_mphf* f, const char* d_bases, const uint64_t* 
 /* Exact streaming branch on device buffers (include/partitioned_mphf.hpp:73-184, src/query.cpp:52): d_codes and
  * d_code_offsets receive what lphb_query_stream gives for the same batch, the reference's spurious codes of contigs
  * with non-ACGT bytes included (SURVEY.md Q1).  Arguments as in lphb_query_stream_device; n_codes receives the total.
- * SYNCHRONOUS: returns once d_codes / d_code_offsets hold the result (the layout of a contig with non-ACGT bytes is
- * known only after its repair).  The work runs on `stream` and is ordered against the handle's other calls as in
- * lphb_query_stream_device; every copy, the status read-back included, goes on `stream`.  A clean batch costs the
- * stateless form plus one read-back of its 32-byte status.
+ * SYNCHRONOUS: returns once d_codes / d_code_offsets hold the result.  The work runs on `stream` and is ordered
+ * against the handle's other calls as in lphb_query_stream_device; every copy goes on `stream`.  A clean batch costs
+ * the stateless form plus one read-back of its 32-byte status; a batch with non-ACGT bytes adds the repair of
+ * lphb_query_stream_exact_device_async on the device and one 8-byte read-back of the final total between its layout
+ * and its assemble (the capacity check).  lphb_query_stream_exact_device_async is the same without any of these
+ * host synchronisations.
  * Capacity: sum of max(0, L-m+1) over the contigs always suffices.  With less than the result needs, the call
  * returns LPHB_E_CAPACITY with *n_codes set; it then writes nothing at or past d_codes + codes_capacity, and the
  * contents of d_codes / d_code_offsets are unspecified.                                                            */
@@ -159,6 +166,26 @@ int lphb_query_stream_exact_device(lphb_mphf* f, const char* d_bases, const uint
                                    const uint64_t* h_offsets, uint64_t n_contigs, uint64_t* d_codes,
                                    uint64_t codes_capacity, uint64_t* d_code_offsets,
                                    uint64_t* n_codes, void* stream);
+
+/* The exact streaming branch, ASYNCHRONOUS: d_codes and d_code_offsets receive what lphb_query_stream gives for the
+ * batch (spurious codes included, as lphb_query_stream_exact_device), d_status[0] the number of codes and
+ * d_status[1] the number of contigs holding a non-ACGT byte (4 words; [2] and [3] are not written).  Arguments as in
+ * lphb_query_stream_device.  The call returns once the work is enqueued on `stream`: it makes no host
+ * synchronisation, no read-back and no pageable copy, and every kernel whose work depends on a count produced on the
+ * device reads that count there.  Ordered against the handle's other calls as lphb_query_stream_device; afterwards
+ * lphb_mphf_dirty_flags names the batch's dirty contigs and lphb_mphf_stats reports the launches and the main
+ * kernel's time, but its dirty_contigs is 0: the count is in d_status[1].
+ * Capacity: codes_capacity must be at least sum of max(0, L-m+1) over the contigs, else LPHB_E_CAPACITY (the bound in
+ * the message) before anything is enqueued.  The device never writes at or past d_codes + codes_capacity.
+ * Workspace: the repair's scratch grows to 68 bytes per contig + 9.03 bytes per base of the batch + 8 bytes per
+ * clean code (those it moves) + 12 KB, sized from h_offsets alone; a call that grows it waits for the
+ * device while it frees the old buffer (cudaFree), so a pipeline reaches full asynchrony from its second call on
+ * batches no larger than the first.  The repair's work grows with the dirty contigs: a clean batch costs the
+ * stateless form plus 8 launches and a 48-byte memset that find nothing to do.                                    */
+int lphb_query_stream_exact_device_async(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets,
+                                         const uint64_t* h_offsets, uint64_t n_contigs, uint64_t* d_codes,
+                                         uint64_t codes_capacity, uint64_t* d_code_offsets,
+                                         uint64_t* d_status, void* stream);
 
 /* Non-streaming branch on device buffers, hf(seq, len, false) (include/partitioned_mphf.hpp:185-195; a non-ACGT
  * byte counts as 'A', include/mphf_utils.hpp:108): every window of k bytes has its code, max(0, L-k+1) per contig,

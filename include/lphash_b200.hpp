@@ -190,6 +190,17 @@ public:
         if (rc != LPHB_OK) detail::raise("lphash_b200::mphf::query_batch_device", rc);
         return n;
     }
+    // The same as query_batch_device, asynchronous on `stream` (lphb_query_stream_exact_device_async): d_status (4
+    // words) receives the number of codes and of contigs with non-ACGT bytes; codes_capacity must be at least
+    // sum of max(0, L-m+1).
+    void query_batch_device_async(const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
+                                  uint64_t n_contigs, uint64_t* d_codes, uint64_t codes_capacity,
+                                  uint64_t* d_code_offsets, uint64_t* d_status, void* stream = nullptr) const {
+        if (!h_) throw std::runtime_error("lphash_b200::mphf: no index loaded");
+        int rc = lphb_query_stream_exact_device_async(h_, d_bases, d_offsets, h_offsets, n_contigs, d_codes,
+                                                      codes_capacity, d_code_offsets, d_status, stream);
+        if (rc != LPHB_OK) detail::raise("lphash_b200::mphf::query_batch_device_async", rc);
+    }
     // hf(contig, len, false) for every contig (lphb_query_nonstreaming_device): max(0, L-k+1) codes per contig,
     // asynchronous on `stream`; d_status (4 words) as lphb_query_stream_device fills it.
     void query_batch_device_nonstreaming(const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,

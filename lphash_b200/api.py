@@ -98,7 +98,8 @@ EXPORTS = ["lphb_last_error", "lphb_version", "lphb_device_count", "lphb_mphf_lo
            "lphb_mphf_alt_load_file", "lphb_mphf_alt_load_memory", "lphb_inverted_index_bound",
            "lphb_build_inverted_index", "lphb_lph_assemble", "lphb_lph_sections", "lphb_build_inverted_index_alt",
            "lphb_lph_assemble_alt", "lphb_mphf_device_image", "lphb_lookup_kmers", "lphb_lookup_kmers_device",
-           "lphb_query_stream_exact_device", "lphb_query_nonstreaming_device", "lphb_check_begin", "lphb_check_batch",
+           "lphb_query_stream_exact_device", "lphb_query_stream_exact_device_async", "lphb_query_nonstreaming_device",
+           "lphb_check_begin", "lphb_check_batch",
            "lphb_check_batch_device", "lphb_check_end", "lphb_build_begin", "lphb_build_batch",
            "lphb_build_batch_device", "lphb_build_end", "lphb_build_free"]
 
@@ -129,6 +130,7 @@ def lib() -> C.CDLL:
     L.lphb_query_nonstreaming.argtypes = [p, p, p, u64, p, u64, p, C.POINTER(u64)]
     L.lphb_query_stream_device.argtypes = [p, p, p, p, u64, p, u64, p, p, p]
     L.lphb_query_stream_exact_device.argtypes = [p, p, p, p, u64, p, u64, p, C.POINTER(u64), p]
+    L.lphb_query_stream_exact_device_async.argtypes = [p, p, p, p, u64, p, u64, p, p, p]
     L.lphb_query_nonstreaming_device.argtypes = [p, p, p, p, u64, p, u64, p, p, p]
     L.lphb_lookup_kmers.argtypes = [p, p, u64, p]
     L.lphb_lookup_kmers_device.argtypes = [p, p, u64, p, p]
@@ -335,6 +337,20 @@ class Mphf:
             raise CapacityError(rc, lib().lphb_last_error().decode(), n.value)
         _check(rc)
         return n.value
+
+    def query_device_exact_async(self, d_bases: int, d_offsets: int, h_offsets: np.ndarray, d_codes: int,
+                                 capacity: int, d_code_offsets: int, d_status: int, stream: int = 0) -> None:
+        """lphb_query_stream_exact_device_async: the codes of query_device_exact, enqueued on the stream with no host
+        synchronisation; d_status (4 int64 words) receives the number of codes and of contigs with non-ACGT bytes.
+        capacity must be at least sum(max(0, L-m+1)), else CapacityError (n_codes = that bound) before anything runs."""
+        h_offsets = np.ascontiguousarray(h_offsets, dtype=np.uint64)
+        rc = lib().lphb_query_stream_exact_device_async(self._h, d_bases, d_offsets, h_offsets.ctypes.data,
+                                                        len(h_offsets) - 1, d_codes, capacity, d_code_offsets,
+                                                        d_status, stream)
+        if rc == E_CAPACITY:
+            lens = np.diff(h_offsets.astype(np.int64))
+            raise CapacityError(rc, lib().lphb_last_error().decode(), int(np.maximum(lens - self.m + 1, 0).sum()))
+        _check(rc)
 
     def query_device_nonstreaming(self, d_bases: int, d_offsets: int, h_offsets: np.ndarray, d_codes: int,
                                   capacity: int, d_code_offsets: int, d_status: int, stream: int = 0) -> None:

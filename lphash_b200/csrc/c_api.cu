@@ -52,16 +52,9 @@ struct Workspace {
         HostBuf h_count;              // runs per chunk
         std::vector<Event> ev_count;  // per chunk: its run count has reached h_count
     } runs;
-    // repair of contigs with non-ACGT bytes
+    // repair of contigs with non-ACGT bytes (quirk_kernels.cu): its scratch, and the host forms' final codes
     struct Repair {
-        DevBuf contigs, starts;                          // the contigs, where each starts in `bases`
-        DevBuf bases, flag, run_off, run_first, status;  // their bytes gathered, cut into maximal runs
-        DevBuf tmp;                                      // scan scratch
-        DevBuf run_code_off, run_dirty, run_codes, tile;  // the runs through the query kernel
-        DevBuf spur, spur_count, out_off, out;           // the runs' final codes
-        DevBuf out_at, counts;                           // per contig: where its codes are in `out`, how many
-        DevBuf src_off, assembled;                       // the batch's codes in their final layout
-        std::vector<uint64_t> h_src_off;                 // src_off as the host computes it
+        DevBuf scratch, out;
     } repair;
     // chunk pipeline of lphb_query_stream: two extra streams so that the H2D copy of chunk j+1,
     // the kernels of chunk j and the D2H copy of chunk j-1 overlap (PCIe is full duplex)
@@ -358,138 +351,31 @@ void check_chunk(lphb_mphf* f, DevBatch const& b, uint64_t j0, uint64_t j1, cons
 }
 
 // ---- contigs with non-ACGT bytes (SURVEY.md Q1; quirk_kernels.cu) ----------------------------------------------
-// Their valid k-mers are ordinary work: the contigs are gathered into a compact batch, cut into maximal runs of
-// valid / invalid bytes, and the runs go through the same query kernel as contigs of their own.  Only the
-// reference's spurious codes (pushed while a run is shorter than k) need the sequential state machine, one thread
-// per episode of a few dozen bases.  Two stages: repair_layout (the dirty contigs' codes and the final layout),
-// then, once the caller has checked its capacity, repair_assemble (the batch's codes in that layout).
+// Every form runs the same two device stages after its clean pass: launch_repair_layout (the dirty contigs listed,
+// their spurious codes replayed, the final layout into the code offsets and its total into a status word), then
+// launch_repair_assemble (the codes in that layout).  Nothing between them needs the host; the synchronous forms
+// read the total back there for their capacity check.
 
-// A batch after its clean pass, as the repair reads it.  Device pointers, but h_offsets.
-struct DirtyBatch {
-    const char* bases;            // indexed by the offsets
-    const uint64_t* offsets;      // n_contigs + 1
-    const uint64_t* h_offsets;    // the same offsets on the host
-    uint64_t n_contigs;
-    const uint8_t* dirty;         // per contig: holds a non-ACGT byte
-    const uint64_t* clean_codes;  // the clean pass's codes, clean layout (L-k+1 per contig)
-};
-
-// Leaves the dirty contigs' final codes in the handle's repair scratch and where each contig's codes come from in
-// ws.repair.h_src_off; writes the final layout to code_offsets (host, n_contigs + 1) and returns its total.
-// *d2h_bytes = what it copied to the host.  Every copy runs on s.
-uint64_t repair_layout(lphb_mphf* f, DirtyBatch const& b, uint64_t* code_offsets, cudaStream_t s, uint64_t* d2h_bytes) {
-    Workspace::Repair& R = f->ws.repair;
-    const uint32_t k = f->img.k, w_cap = f->img.w;
-    const uint64_t n_contigs = b.n_contigs;
-    const uint64_t* offsets = b.h_offsets;
-    std::vector<uint8_t> dirty(n_contigs);
-    CK(cudaMemcpyAsync(dirty.data(), b.dirty, n_contigs, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    std::vector<uint64_t> list, starts;
-    uint64_t q_bytes = 0;
-    for (uint64_t c = 0; c < n_contigs; ++c)
-        if (dirty[c]) {
-            list.push_back(c);
-            starts.push_back(q_bytes);
-            q_bytes += offsets[c + 1] - offsets[c];
-        }
-    starts.push_back(q_bytes);
-    const uint64_t n_list = list.size();
-    R.contigs.reserve(n_list * 8);
-    R.starts.reserve((n_list + 1) * 8);
-    R.out_at.reserve(n_list * 8);
-    R.counts.reserve(n_list * 8);
-    R.bases.reserve(q_bytes + 64);
-    R.flag.reserve(q_bytes + 8);
-    R.run_off.reserve((q_bytes + 2) * 8);
-    R.run_first.reserve((n_list + 2) * 4);
-    R.status.reserve(64);
-    R.tmp.reserve(std::max<uint64_t>(quirk_tmp_bytes(q_bytes + 1), code_offsets_tmp_bytes(q_bytes + 1)));
-    CK(cudaMemcpyAsync(R.contigs.p, list.data(), n_list * 8, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(R.starts.p, starts.data(), (n_list + 1) * 8, cudaMemcpyHostToDevice, s));
-    CK(cudaMemsetAsync(R.bases.as<char>() + q_bytes, 'A', 64, s));  // read-ahead of the last tile
-    launch_gather_contigs(b.bases, b.offsets, R.contigs.as<uint64_t>(), R.starts.as<uint64_t>(), n_list, q_bytes,
-                          R.bases.as<char>(), s);
-    auto* qst = R.status.as<unsigned long long>();
-    launch_find_runs(R.bases.as<char>(), q_bytes, R.starts.as<uint64_t>(), n_list, R.flag.as<uint8_t>(),
-                     R.run_off.as<uint64_t>(), qst + 4, R.run_first.as<uint32_t>(), R.tmp.p, R.tmp.cap, s);
-    unsigned long long n_v = 0;
-    CK(cudaMemcpyAsync(&n_v, qst + 4, 8, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    CK(cudaGetLastError());
-    f->stats.kernel_launches += 7;
-    // the runs as a batch of their own: valid k-mers of every run, clean layout per run
-    R.run_code_off.reserve((n_v + 2) * 8);
-    R.run_dirty.reserve(n_v + 8);
-    R.run_codes.reserve(q_bytes * 8 + 64);
-    R.tile.reserve(query_tiled_ws_bytes(q_bytes));
-    CK(cudaMemsetAsync(R.run_dirty.p, 0, n_v + 8, s));
-    launch_code_offsets(R.run_off.as<uint64_t>(), n_v, k, R.run_code_off.as<uint64_t>(), qst, R.tmp.p, R.tmp.cap, s);
-    DevBatch bq{};
-    bq.bases = R.bases.as<char>();
-    bq.offsets = R.run_off.as<uint64_t>();
-    bq.code_off = R.run_code_off.as<uint64_t>();
-    bq.n_contigs = n_v;
-    bq.first_base = 0;
-    bq.end_base = q_bytes;
-    bq.codes = R.run_codes.as<uint64_t>();
-    bq.dirty = R.run_dirty.as<uint8_t>();
-    bq.status = qst;
-    bq.tile_ws = R.tile.p;
-    bq.tile_ws_bytes = R.tile.cap;
-    if (!launch_query_tiled(f->img, bq, s)) launch_query_generic(f->img, bq, s);
-    f->stats.kernel_launches += 3;
-    R.spur.reserve((n_v + 1) * uint64_t(w_cap) * 8);
-    R.spur_count.reserve((n_v + 2) * 4);
-    R.out_off.reserve((n_v + 2) * 8);
-    R.out.reserve((q_bytes + n_v * uint64_t(w_cap)) * 8 + 64);
-    launch_quirk_finish(f->img, R.bases.as<char>(), R.run_off.as<uint64_t>(), n_v, qst + 4, R.run_first.as<uint32_t>(),
-                        n_list, R.run_code_off.as<uint64_t>(), R.run_codes.as<uint64_t>(), R.spur.as<uint64_t>(),
-                        R.spur_count.as<uint32_t>(), w_cap, R.out_off.as<uint64_t>(), R.out.as<uint64_t>(),
-                        R.out_at.as<uint64_t>(), R.counts.as<uint64_t>(), R.tmp.p, R.tmp.cap, s);
-    launch_quirk_emit(R.run_code_off.as<uint64_t>(), R.run_codes.as<uint64_t>(), R.spur.as<uint64_t>(),
-                      R.spur_count.as<uint32_t>(), w_cap, n_v, qst + 4, R.out_off.as<uint64_t>(), q_bytes,
-                      R.out.as<uint64_t>(), s);
-    f->stats.kernel_launches += 6;
-    std::vector<uint64_t> counts(n_list), out_at(n_list);
-    CK(cudaMemcpyAsync(out_at.data(), R.out_at.p, n_list * 8, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(counts.data(), R.counts.p, n_list * 8, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    CK(cudaGetLastError());
-    // final layout + where each contig's codes come from (clean layout or the repaired runs)
-    std::vector<uint64_t>& src_off = R.h_src_off;
-    src_off.resize(n_contigs);
-    uint64_t new_total = 0, clean_run = 0;
-    for (uint64_t c = 0, j = 0; c < n_contigs; ++c) {
-        uint64_t len = offsets[c + 1] - offsets[c];
-        uint64_t clean_cnt = len >= k ? len - k + 1 : 0;
-        uint64_t cnt = clean_cnt;
-        if (dirty[c]) {
-            src_off[c] = out_at[j];
-            cnt = counts[j++];
-        } else {
-            src_off[c] = clean_run;
-        }
-        clean_run += clean_cnt;
-        code_offsets[c] = new_total;
-        new_total += cnt;
-    }
-    code_offsets[n_contigs] = new_total;
-    *d2h_bytes = n_contigs + n_list * 8;
-    return new_total;
+// The repair scratch of a batch (n_contigs contigs over `span` bases with clean_total clean codes), sized from the
+// host offsets alone, over the batch's bytes (indexed by the offsets) and the clean pass's dirty flags.
+RepairWs reserve_repair(lphb_mphf* f, const char* bases, const uint64_t* d_offsets, const uint8_t* dirty,
+                        uint64_t n_contigs, uint64_t span, uint64_t clean_total, bool in_place) {
+    RepairWs w{};
+    w.bases = bases;
+    w.offsets = d_offsets;
+    w.n_contigs = n_contigs;
+    w.dirty = dirty;
+    DevBuf& buf = f->ws.repair.scratch;
+    buf.reserve(repair_scratch(n_contigs, span, clean_total, in_place, nullptr, nullptr));
+    repair_scratch(n_contigs, span, clean_total, in_place, buf.as<char>(), &w);
+    return w;
 }
 
-// The batch's codes in the final layout of repair_layout (code_offsets, total new_total) into dst, which must not be
-// b.clean_codes; d_code_off receives that layout.
-void repair_assemble(lphb_mphf* f, DirtyBatch const& b, const uint64_t* code_offsets, uint64_t new_total,
-                     uint64_t* d_code_off, uint64_t* dst, cudaStream_t s) {
-    Workspace::Repair& R = f->ws.repair;
-    R.src_off.reserve((b.n_contigs + 1) * 8);
-    CK(cudaMemcpyAsync(R.src_off.p, R.h_src_off.data(), b.n_contigs * 8, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(d_code_off, code_offsets, (b.n_contigs + 1) * 8, cudaMemcpyHostToDevice, s));
-    launch_assemble(dst, d_code_off, b.clean_codes, R.out.as<uint64_t>(), R.src_off.as<uint64_t>(), b.dirty, b.n_contigs,
-                    new_total, s);
-    f->stats.kernel_launches += 1;
+// the layout stage on s, its counters cleared first
+void repair_layout(lphb_mphf* f, RepairWs const& w, uint64_t* d_code_off, const uint64_t* codes, uint64_t clean_total,
+                   bool in_place, unsigned long long* d_total, cudaStream_t s) {
+    CK(cudaMemsetAsync(w.ctr, 0, sizeof(RepairCounters), s));
+    f->stats.kernel_launches += launch_repair_layout(f->img, w, d_code_off, codes, clean_total, in_place, d_total, s);
 }
 
 // What the caller wants back: the codes themselves (8 B per k-mer) or their run-length form (12-byte
@@ -507,7 +393,8 @@ struct RunSink {
 
 // One call of lphb_query_stream, lphb_query_nonstreaming or lphb_query_stream_runs with its batch on the host.
 // Stages: the layout (run), then either the small-batch block (small_call) or the clean pass (clean_pass); when
-// a contig holds a non-ACGT byte, the repair of such contigs (repair_layout, repair_assemble); the output (output).
+// a contig holds a non-ACGT byte, the repair of such contigs (launch_repair_layout, launch_repair_assemble); the
+// output (output).
 struct HostQuery {
     lphb_mphf* f;
     const char* bases;
@@ -547,17 +434,22 @@ struct HostQuery {
             return LPHB_OK;
         }
         if (n_dirty == 0) return copied_out ? finish(total, n_chunks, 0) : output(ws.codes.as<uint64_t>(), total, 0);
-        const DirtyBatch db{ws.bases.as<char>() - first, ws.offsets.as<uint64_t>(), offsets, n_contigs,
-                            ws.dirty.as<uint8_t>(), ws.codes.as<uint64_t>()};
-        uint64_t d2h_repair = 0;
-        const uint64_t new_total = repair_layout(f, db, code_offsets, s, &d2h_repair);
+        const RepairWs w = reserve_repair(f, ws.bases.as<char>() - first, ws.offsets.as<uint64_t>(), ws.dirty.as<uint8_t>(),
+                                          n_contigs, span, total, false);
+        repair_layout(f, w, ws.code_off.as<uint64_t>(), ws.codes.as<uint64_t>(), total, false,
+                      ws.status.as<unsigned long long>(), s);
+        CK(cudaMemcpyAsync(code_offsets, ws.code_off.p, (n_contigs + 1) * 8, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        CK(cudaGetLastError());
+        const uint64_t new_total = code_offsets[n_contigs];
         *n_codes = new_total;
         if (!want_runs && new_total > codes_capacity) return fail(LPHB_E_CAPACITY, "codes buffer too small");
         if (want_runs && new_total >= (1ull << 31)) return fail(LPHB_E_ARG, "batch holds >= 2^31 codes: split it");
-        ws.repair.assembled.reserve(new_total * 8 + 64);
-        repair_assemble(f, db, code_offsets, new_total, ws.code_off.as<uint64_t>(), ws.repair.assembled.as<uint64_t>(), s);
+        ws.repair.out.reserve(new_total * 8 + 64);
+        f->stats.kernel_launches += launch_repair_assemble(f->img, w, ws.code_off.as<uint64_t>(), ws.codes.as<uint64_t>(),
+                                                           false, ws.repair.out.as<uint64_t>(), new_total, s);
         if (want_runs) reserve_runs(new_total + 16, 1, new_total, 1);
-        return output(ws.repair.assembled.as<uint64_t>(), new_total, d2h_repair);
+        return output(ws.repair.out.as<uint64_t>(), new_total, (n_contigs + 1) * 8);
     }
 
     // ---- small batch (the reference's own loop hands over one record per call, src/query.cpp:48-56): one device
@@ -815,19 +707,16 @@ DevBatch start_device_batch(lphb_mphf* f, const char* d_bases, const uint64_t* d
 // non_streaming: the kernels read a copy of the batch's bytes in the workspace with every non-ACGT byte made 'A',
 // so that every window has its code and the caller's bytes stay as they are.
 // The exact form: the same clean pass, one read-back of its status and, when a contig holds a non-ACGT byte, the
-// repair lphb_query_stream runs.  The clean pass writes straight into d_codes when the clean layout fits there, so a
-// clean batch costs one device call more than the stateless form: the status read.  A repair then assembles from a
-// copy of those codes in the workspace, since the assemble must not read the buffer it writes.
+// repair's layout stage, one read-back of the final total (the capacity check), the assemble stage.  The clean pass
+// writes straight into d_codes when the clean layout fits there, so a clean batch costs one device call more than
+// the stateless form: the status read.  The layout stage then saves the clean codes the assemble overwrites.
 int device_query(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
                  uint64_t n_contigs, uint64_t* d_codes, uint64_t codes_capacity, uint64_t* d_code_offsets,
                  unsigned long long* st, uint64_t* n_codes, bool non_streaming, cudaStream_t s) {
     f->stats = lphb_stats{};
     Workspace& ws = f->ws;
     const bool exact = n_codes != nullptr;
-    std::vector<uint64_t> code_offsets(exact ? n_contigs + 1 : 0);
-    // (one call per form, so that neither per-contig loop tests whether it writes code offsets)
-    const uint64_t total = exact ? contig_layout(h_offsets, n_contigs, f->img.k, 0, code_offsets.data()).kmers
-                                 : contig_layout(h_offsets, n_contigs, f->img.k).kmers;
+    const uint64_t total = contig_layout(h_offsets, n_contigs, f->img.k).kmers;
     const uint64_t first = h_offsets[0], span = h_offsets[n_contigs] - first;
     if (exact) *n_codes = total;
     else if (total > codes_capacity) return fail(LPHB_E_CAPACITY, "codes buffer too small");
@@ -859,19 +748,44 @@ int device_query(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets, c
     f->stats.d2h_bytes = 4 * sizeof(unsigned long long);
     f->stats.dirty_contigs = h_status[1];
     if (h_status[1] == 0) return in_place ? LPHB_OK : fail(LPHB_E_CAPACITY, "codes buffer too small");
-    if (in_place) {
-        ws.codes.reserve(total * 8 + 64);
-        CK(cudaMemcpyAsync(ws.codes.p, d_codes, total * 8, cudaMemcpyDeviceToDevice, s));
-    }
-    const DirtyBatch db{d_bases, d_offsets, h_offsets, n_contigs, ws.dirty.as<uint8_t>(), ws.codes.as<uint64_t>()};
-    uint64_t d2h_repair = 0;
-    const uint64_t new_total = repair_layout(f, db, code_offsets.data(), s, &d2h_repair);
+    uint64_t* clean = in_place ? d_codes : ws.codes.as<uint64_t>();
+    const RepairWs w = reserve_repair(f, d_bases, d_offsets, b.dirty, n_contigs, span, total, in_place);
+    repair_layout(f, w, d_code_offsets, clean, total, in_place, st, s);
+    CK(cudaMemcpyAsync(h_status, st, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    CK(cudaGetLastError());
+    const uint64_t new_total = h_status[0];
     *n_codes = new_total;
-    f->stats.d2h_bytes += d2h_repair;
+    f->stats.d2h_bytes += sizeof(unsigned long long);
     if (new_total > codes_capacity) return fail(LPHB_E_CAPACITY, "codes buffer too small");
-    repair_assemble(f, db, code_offsets.data(), new_total, d_code_offsets, d_codes, s);
+    f->stats.kernel_launches += launch_repair_assemble(f->img, w, d_code_offsets, clean, in_place, d_codes, new_total, s);
     ws.mark_last(s);
     CK(cudaStreamSynchronize(s));
+    CK(cudaGetLastError());
+    return LPHB_OK;
+}
+
+// lphb_query_stream_exact_device_async: the exact form with nothing on the host between the stages.  The capacity
+// is checked against the bound, Σ max(0, L-m+1), before anything is enqueued, so the clean pass always writes in
+// place and the assemble never needs the total on the host; the scratch is sized from h_offsets alone.
+int device_query_exact_async(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets, const uint64_t* h_offsets,
+                             uint64_t n_contigs, uint64_t* d_codes, uint64_t codes_capacity, uint64_t* d_code_offsets,
+                             unsigned long long* st, cudaStream_t s) {
+    f->stats = lphb_stats{};
+    const ContigCounts n = contig_layout(h_offsets, n_contigs, f->img.k, f->img.m);
+    const uint64_t span = h_offsets[n_contigs] - h_offsets[0];
+    if (n.mmers > codes_capacity)
+        return fail(LPHB_E_CAPACITY, "codes_capacity = " + std::to_string(codes_capacity) +
+                                         " is below the bound sum of max(0, L-m+1) = " + std::to_string(n.mmers));
+    if ((n.kmers && !d_codes) || (span && !d_bases)) return fail(LPHB_E_ARG, "null data pointer");
+    const DevBatch b = start_device_batch(f, d_bases, d_offsets, h_offsets, n_contigs, d_code_offsets, d_codes, st, true, s);
+    if (n_contigs) {
+        const RepairWs w = reserve_repair(f, d_bases, d_offsets, b.dirty, n_contigs, span, n.kmers, true);
+        run_kernels(f, b, s);
+        repair_layout(f, w, d_code_offsets, d_codes, n.kmers, true, st, s);
+        f->stats.kernel_launches += launch_repair_assemble(f->img, w, d_code_offsets, d_codes, true, d_codes, n.mmers, s);
+    }
+    f->ws.mark_last(s);
     CK(cudaGetLastError());
     return LPHB_OK;
 }
@@ -1185,6 +1099,20 @@ int lphb_query_stream_exact_device(lphb_mphf* f, const char* d_bases, const uint
         DeviceGuard g(f->device);
         return device_query(f, d_bases, d_offsets, h_offsets, n_contigs, d_codes, codes_capacity, d_code_offsets,
                             nullptr, n_codes, false, static_cast<cudaStream_t>(stream));
+    });
+}
+
+int lphb_query_stream_exact_device_async(lphb_mphf* f, const char* d_bases, const uint64_t* d_offsets,
+                                         const uint64_t* h_offsets, uint64_t n_contigs, uint64_t* d_codes,
+                                         uint64_t codes_capacity, uint64_t* d_code_offsets, uint64_t* d_status,
+                                         void* stream) {
+    if (!f || !d_offsets || !h_offsets || !d_code_offsets || !d_status)
+        return fail(LPHB_E_ARG, "null argument");
+    return guarded([&]() -> int {
+        DeviceGuard g(f->device);
+        return device_query_exact_async(f, d_bases, d_offsets, h_offsets, n_contigs, d_codes, codes_capacity,
+                                        d_code_offsets, reinterpret_cast<unsigned long long*>(d_status),
+                                        static_cast<cudaStream_t>(stream));
     });
 }
 

@@ -52,21 +52,61 @@ bool launch_scan_records_tiled(uint32_t k, uint32_t m, uint64_t seed, DevBatch c
                                cudaStream_t stream);
 bool scan_tiled_available(uint32_t k, uint32_t m);
 
-// Contigs with non-ACGT bytes, run-parallel (quirk_kernels.cu).  All asynchronous on `stream`.
-void launch_gather_contigs(const char* bases, const uint64_t* offsets, const uint64_t* list, const uint64_t* dst_off,
-                           uint64_t n_list, uint64_t total_bytes, char* dst, cudaStream_t stream);
+// Contigs with non-ACGT bytes (quirk_kernels.cu): the build side's run finder, and the query side's repair.
 uint64_t quirk_tmp_bytes(uint64_t n);
 void launch_find_runs(const char* d_bases, uint64_t n, const uint64_t* d_starts, uint64_t n_list, uint8_t* d_flag,
                       uint64_t* d_voff, unsigned long long* d_n_v, uint32_t* d_vstart, void* d_tmp, uint64_t tmp_bytes,
                       cudaStream_t stream);
-void launch_quirk_finish(DevImage const& img, const char* d_bases, const uint64_t* d_voff, uint64_t n_v_host,
-                         const unsigned long long* d_n_v, const uint32_t* d_vstart, uint64_t n_list,
-                         const uint64_t* d_vcode_off, const uint64_t* d_vcodes, uint64_t* d_spur, uint32_t* d_spur_cnt,
-                         uint32_t w_cap, uint64_t* d_out_off, uint64_t* d_out, uint64_t* d_q_off, uint64_t* d_counts,
-                         void* d_tmp, uint64_t tmp_bytes, cudaStream_t stream);
-void launch_quirk_emit(const uint64_t* d_vcode_off, const uint64_t* d_vcodes, const uint64_t* d_spur,
-                       const uint32_t* d_spur_cnt, uint32_t w_cap, uint64_t n_v_host, const unsigned long long* d_n_v,
-                       const uint64_t* d_out_off, uint64_t total_hint, uint64_t* d_out, cudaStream_t stream);
+
+// The repair of a batch after its clean pass (the stateless codes in the clean layout, L-k+1 slots per contig, and
+// the dirty flags), all on the device and asynchronous: every count it depends on stays in device memory, and every
+// kernel reads it there and exits early when there is nothing to do (a clean batch).  A dirty contig is cut into
+// chunks of kRepairChunk bytes; each chunk is one block's work.  Scratch, sized from the host offsets alone
+// (repair_scratch): 68 bytes per contig, 9.03 bytes per base (a flag and a code slot per byte of a dirty contig,
+// 28 bytes per chunk), 8 bytes per clean code when the clean pass wrote in place, and 12 KB.
+constexpr uint32_t kRepairChunk = 1024;
+constexpr uint32_t kRepairScanBlocks = 1024;
+struct RepairCounters {
+    unsigned long long n_list;    // dirty contigs listed
+    unsigned long long bytes;     // their bytes (the scratch slots handed out)
+    unsigned long long n_chunks;  // their chunks
+    unsigned long long fd_rev;    // n_contigs - (first dirty contig); 0: none
+    unsigned long long scan_done[2];  // up-sweep blocks finished (the chunks' scan, the contigs')
+};
+struct RepairWs {
+    const char* bases;            // indexed by the offsets
+    const uint64_t* offsets;      // n_contigs + 1 (device)
+    uint64_t n_contigs;
+    const uint8_t* dirty;         // per contig (the clean pass's flags)
+    RepairCounters* ctr;          // zeroed by the caller before launch_repair_layout
+    uint64_t* list;               // 3 words per listed contig: contig, first scratch slot, first chunk
+    uint64_t* slot;               // per contig: its list entry (dirty contigs only)
+    uint64_t* chunk_tab;          // per chunk: its list entry
+    uint16_t* chunk_first;        // per chunk: offset of its first ACGT byte, 0xFFFF if none
+    uint16_t* chunk_last_inv;     // per chunk: offset of its last non-ACGT byte, 0xFFFF if none
+    uint64_t* chunk_cnt;          // per chunk: codes it yields
+    uint64_t* chunk_out;          // exclusive sums of chunk_cnt (n_chunks + 1)
+    uint8_t* spur_flag;           // per scratch slot: a spurious code is pushed at this byte
+    uint64_t* spur_code;          // ... and this is it
+    uint64_t* tail_off;           // clean code offsets of the contigs from the first dirty one on
+    uint64_t* tail_codes;         // in place: the clean codes from the first dirty contig on
+    uint64_t* part;               // scan spine (kRepairScanBlocks + 1)
+};
+// Bytes of scratch for a batch (offsets of the fields above in one allocation, 256-byte aligned): fills `w`'s pointers
+// relative to `base` when base is not null.
+uint64_t repair_scratch(uint64_t n_contigs, uint64_t span, uint64_t clean_total, bool in_place, char* base, RepairWs* w);
+// Layout stage (the caller zeroes w.ctr first, on the same stream): lists the dirty contigs, replays their
+// episodes, counts every chunk's codes and writes the final layout to d_code_off (n_contigs + 1, the clean layout on
+// entry; rewritten from the first dirty contig on) and its total to *d_total.  `codes` holds the clean pass's
+// clean_total codes; when in_place they are saved from the first dirty contig on (the assemble then overwrites
+// them).  Returns the launches.
+int launch_repair_layout(DevImage const& img, RepairWs const& w, uint64_t* d_code_off, const uint64_t* codes,
+                         uint64_t clean_total, bool in_place, unsigned long long* d_total, cudaStream_t stream);
+// Assemble stage: the final codes into dst in the layout of d_code_off.  in_place: dst is the clean pass's buffer and
+// only codes from the first dirty contig on are written; otherwise src holds the clean codes and every code is
+// written.  max_total bounds the final total (grid size).  Returns the launches.
+int launch_repair_assemble(DevImage const& img, RepairWs const& w, const uint64_t* d_code_off, const uint64_t* src,
+                           bool in_place, uint64_t* dst, uint64_t max_total, cudaStream_t stream);
 
 // Build side (minimizer::from_string over contigs with non-ACGT bytes): launch_find_runs over the whole batch
 // (d_starts = contig starts relative to the batch, launch_shift_starts), then per run r the number of pieces the
@@ -82,11 +122,6 @@ void launch_build_run_counts(const char* d_bases, const uint64_t* d_voff, const 
 void launch_build_pieces(const uint64_t* d_voff, const unsigned long long* d_n_v, uint64_t n_v_host, uint32_t k,
                          const uint64_t* d_pieces, const uint64_t* d_ids, uint64_t mm_count_in, uint64_t n, uint64_t* d_poff,
                          uint64_t* d_pid, cudaStream_t stream);
-
-// dst[dst_off[c] .. dst_off[c+1]) = src_c[src_off[c] ..) where src_c = from_b[c] ? src_b : src_a (`total` = dst_off[n_contigs])
-void launch_assemble(uint64_t* dst, const uint64_t* dst_off, const uint64_t* src_a,
-                     const uint64_t* src_b, const uint64_t* src_off, const uint8_t* from_b,
-                     uint64_t n_contigs, uint64_t total, cudaStream_t stream);
 
 // Run-length form of a code stream on the device (runs_kernels.cu): codes[0..n), n < 2^31 -> 12-byte
 // records {u64 first, i32 n} (n > 0 ascending, n < 0 descending), never across a contig start.
